@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W                (our arm; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W   (the reference's CPU path)
+    python bench.py ... --dump-outputs DIR                        (also writes the last timed step's flows, see dump_outputs)
 
 A "step" is one pass of the hot path over one batch: every rank refines `--pairs` consecutive
 synthetic frame pairs at 2560x1440 with the reference's default two-frame parameters (5 outer x 1 inner
@@ -54,7 +55,13 @@ def parse():
     ap.add_argument("--no-secondary", action="store_true", help="skip the multi-frame (config 3 / 4) secondary measurement")
     ap.add_argument("--sor-fuse", type=int, default=0)
     ap.add_argument("--sor-variant", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm only: write the refined flows of the last timed step (rank 0) as DIR/flow_x.npy and "
+                         "DIR/flow_y.npy, see dump_outputs")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no flows (it times the CPU path on a sample)")
+    return a
 
 
 # ----------------------------------------------------------------------------------------- helpers
@@ -472,6 +479,34 @@ def run_epic_secondary(ctx, with_cpu, reps=3):
 
 
 # ----------------------------------------------------------------------------------------- our arm
+DUMP_SAMPLES = 1 << 21  # per flow component when the whole output exceeds DUMP_LIMIT_BYTES: 32 MB in all with the index
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, d_wx, d_wy, W, H, S):
+    """What a caller of sfgpu_variational_dev receives from one step: the refined flow of every pair, cropped from the row stride
+    S to the image width, as float32 flow_x.npy / flow_y.npy of shape (pairs, H, W).  When the two exceed DUMP_LIMIT_BYTES, the
+    same fixed, seeded sample of (pair, row, column) positions is taken from both instead (1-D arrays), and the positions'
+    indices into the (pairs, H, W) array go to sample_index.npy (float64, exact below 2**53).  The inputs depend only on the
+    arguments, so two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    import torch
+    B = len(d_wx)
+    n = B * H * W
+    fx = torch.stack(d_wx).view(B, H, S)[:, :, :W]
+    fy = torch.stack(d_wy).view(B, H, S)[:, :, :W]
+    if 2 * 4 * n <= DUMP_LIMIT_BYTES:
+        out = {"flow_x": fx.cpu().numpy(), "flow_y": fy.cpu().numpy()}
+    else:
+        idx = np.unique(np.random.default_rng(20170721).integers(0, n, size=DUMP_SAMPLES))
+        ti = torch.from_numpy(idx).to(fx.device)
+        out = {"flow_x": fx.reshape(-1)[ti].cpu().numpy(), "flow_y": fy.reshape(-1)[ti].cpu().numpy(),
+               "sample_index": idx.astype(np.float64)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def _profile_counts():
     """Per-launch counters of the kernels from the committed ncu --set full capture (profiles/kernel_counts.json):
     evidence of the build that was profiled, reported under `from_profile`, never presented as measured in this run."""
@@ -643,6 +678,8 @@ def run_ours(args):
     ms = max_over_ranks(ms_plain)
     total_fields = sum_over_ranks(B * args.steps)
     value = total_fields / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_wx, d_wy, W, H, S)
     # ---- timed region 2 (kernel attribution): the same K steps with CUDA events around every sor_coupled call and
     # every data-term launch.  Kept out of region 1 because an event record between two launches breaks their
     # programmatic-dependent-launch chaining (sf_internal.cuh: pdl_enter), i.e. it perturbs what it measures.

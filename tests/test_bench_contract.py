@@ -61,3 +61,35 @@ def test_driver_secondary_never_takes_the_bench_line_down(built):
             assert leg["jets_per_sec"] > 0 and abs(leg["windows_per_sec"] - 2 * leg["jets_per_sec"]) < 1e-9
         else:
             assert "no CUDA device" in leg["error"]
+
+
+def test_dump_outputs_crops_the_stride_and_samples_large_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: the flows as the caller holds them, (pairs, H, W) float32; above the size limit a seeded sample of both
+    components at the same positions, with those positions in sample_index.npy."""
+    torch = pytest.importorskip("torch")
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    W, H, S, B = 61, 45, 64, 3
+    wx = [torch.arange(S * H, dtype=torch.float32) + 1e4 * j for j in range(B)]
+    wy = [-x for x in wx]
+    ref = np.stack([x.numpy().reshape(H, S)[:, :W] for x in wx])
+    bench.dump_outputs(str(tmp_path / "whole"), wx, wy, W, H, S)
+    fx, fy = np.load(tmp_path / "whole" / "flow_x.npy"), np.load(tmp_path / "whole" / "flow_y.npy")
+    assert fx.dtype == np.float32 and np.array_equal(fx, ref) and np.array_equal(fy, -ref)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["flow_x.npy", "flow_y.npy"]
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1024)
+    monkeypatch.setattr(bench, "DUMP_SAMPLES", 100)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), wx, wy, W, H, S)
+    ix = np.load(tmp_path / "s1" / "sample_index.npy")
+    assert ix.dtype == np.float64 and 0 < len(ix) <= 100 and np.array_equal(ix, np.load(tmp_path / "s2" / "sample_index.npy"))
+    k = ix.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "s1" / "flow_x.npy"), ref.reshape(-1)[k])
+    assert np.array_equal(np.load(tmp_path / "s1" / "flow_y.npy"), -ref.reshape(-1)[k])
+
+
+def test_reference_arm_rejects_dump_outputs(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "d")],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and not (tmp_path / "d").exists()

@@ -11,6 +11,8 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import epic_helpers as eh
+from epic_helpers import epic_inputs, nnfield_inputs
 from slowflow_b200 import ColorImage, Image, synth
 from slowflow_b200.api import EpicParams, epic_params_default
 from slowflow_b200.image import color_image_t, image_t
@@ -28,12 +30,6 @@ def ref_lib(reference):
     return L
 
 
-def unique_seeds(w, h, n, seed):
-    r = np.random.RandomState(seed)
-    p = r.permutation(w * h)[:n]
-    return np.stack([p % w, p // w], axis=1).astype(np.int32)
-
-
 @pytest.mark.parametrize("w,h,ns,nn,kind", [
     (97, 61, 40, 10, "texture"), (200, 150, 300, 26, "texture"), (64, 64, 64, 26, "flat"), (333, 211, 900, 100, "texture"),
     (1024, 436, 5000, 100, "texture"), (130, 33, 50, 50, "ridges"),
@@ -45,16 +41,7 @@ def test_nnfield_labels_and_neighbours_equal_reference(ctx, reference, w, h, ns,
     """dist_trf_nnfield_subset (epic_aux.cpp:350-401): the sweeps are reproduced operation for operation, so the label map
     is identical; the neighbour lists are identical including the order among equal distances (same heap discipline)."""
     L = ref_lib(reference)
-    _, _, cost = synth.epic_case(w, h, 10)
-    if kind == "flat":
-        cost = np.full((h, w), 0.25, np.float32)  # constant cost: ties everywhere
-    elif kind == "ridges":
-        cost = cost + (np.arange(w)[None, :] % 17 == 0) * 5.0  # expensive ridges: many sweeps until nothing changes
-        cost = cost.astype(np.float32)
-    cost = np.ascontiguousarray(cost + np.float32(0.001))
-    if kind == "zero":
-        cost = np.zeros((h, w), np.float32)
-    seeds = unique_seeds(w, h, ns, w * 7 + ns)
+    seeds, cost = nnfield_inputs(w, h, ns, kind)
     rb, rd, rl = np.zeros((ns, nn), np.int32), np.zeros((ns, nn), np.float32), np.zeros((h, w), np.int32)
     c2 = cost.copy()
     L.sf_ref_dist_trf_nnfield(rb.ctypes.data, rd.ctypes.data, rl.ctypes.data, seeds.ctypes.data, ns, nn, c2.ctypes.data, w, h)
@@ -120,3 +107,30 @@ def test_epic_then_variational_pipeline(ctx):
     # (the synthetic ground truth is only approximate at the motion discontinuity, SURVEY 8d: no strict improvement is
     # guaranteed there; the refinement must keep the interpolated field's quality and stay finite)
     assert np.isfinite(wx.array).all() and after < 1.25 * before and after < 0.5
+
+
+
+# Regression vectors (tests/golden/make_golden_epic.py): the GPU path's own outputs on the cases above, recorded when they
+# were added.  They are NOT the reference's outputs and do not replace the comparisons above; they make a change of the EPIC
+# kernels' results visible where the reference build is absent.  Discrete parts must stay equal; the dense flow may move by a tenth of the reference gate
+# (mean 0.001 px, max 0.01 px), so that the recorded vectors cannot take up more than that of the reference tolerance.
+@pytest.mark.parametrize("w,h,ns,nn,kind", eh.REGRESSION_NNFIELD)
+def test_nnfield_unchanged_since_recorded(ctx, w, h, ns, nn, kind):
+    g, t = np.load(eh.REGRESSION_FILE), eh.tag(w, h, ns, nn, kind)
+    seeds, cost = nnfield_inputs(w, h, ns, kind)
+    gl, gb, gd, _ = ctx.epic_nnfield(seeds, nn, cost)
+    for name, a in (("labels_", gl), ("best_", gb), ("dist_", gd)):
+        now, then = eh.stored(a), g[name + t]
+        assert np.array_equal(now, then), "%s differs in %d of %d stored entries" % (name[:-1], int((now != then).sum()), then.size)
+
+
+@pytest.mark.parametrize("w,h,n,method,filters", eh.REGRESSION_EPIC)
+def test_epic_unchanged_since_recorded(ctx, w, h, n, method, filters):
+    g, t = np.load(eh.REGRESSION_FILE), eh.tag(w, h, n, method, filters)
+    ci, m, edges, p = epic_inputs(w, h, n, method, filters)
+    gx, gy = Image(w, h), Image(w, h)
+    st = ctx.epic(gx, gy, ci, m, edges, p)
+    assert [st.matches_in, st.matches_after_saliency, st.matches_after_consistency] == g["counts_" + t].tolist()
+    assert np.array_equal(eh.stored(edges, eh.FLOW_SAMPLE), g["edges_" + t])
+    d = np.hypot(eh.stored(gx.array, eh.FLOW_SAMPLE) - g["fx_" + t], eh.stored(gy.array, eh.FLOW_SAMPLE) - g["fy_" + t])
+    assert d.mean() <= 0.001 and d.max() <= 0.01, (d.mean(), d.max())
