@@ -157,32 +157,49 @@ int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d
     launch_dpsis_weight(st, g, d_im1, c->dpsis, 5.0f, avg0, std1, 255.0f); // variational.c:34
     c->prof_acc.kernel_launches++;
 
-    const bool fused_prep = c->data_variant == 0; // 1: separate warp kernel + tile-based data-term kernel (A/B reference)
+    // 0: marching data pass (k_prep_fused / k_prep_two_frame), 1: separate warp kernel + tile-based data-term kernel,
+    // 2: as 0 but the default loop keeps the smoothness pass separate (k_flow_smooth + k_prep_two_frame); 1 and 2 are the
+    // A/B references of the tests and benchmarks
+    const bool fused_prep = c->data_variant == 0 || c->data_variant == 2;
     if (fused_prep && params->niter_inner == 1 && params->niter_solver > 0) {
         // Default shape of the loop (one inner iteration): per outer iteration the flow update of the previous
-        // iteration (variational.c:60-69 collapsed to w += du) is folded into the smoothness pass, so an outer
-        // iteration is {update+smoothness, warp+derivatives+data term+Laplacian+block inverse, SOR launches}.
+        // iteration (variational.c:60-69 collapsed to w += du) and the smoothness pass are folded into the data pass,
+        // so an outer iteration is {update+smoothness+warp+derivatives+data term+Laplacian+block inverse, SOR launches}.
         // The flow ping-pongs between the caller's planes and (uu, vv); the last update lands in the caller's.
+        const bool fused_psi = c->data_variant == 0;
         float *fx = d_wx, *fy = d_wy, *ax = c->uu, *ay = c->vv;
         const float *pdu = nullptr, *pdv = nullptr;
         for (int outer = 0; outer < params->niter_outer; outer++) {
-            if (outer == 0) {
-                launch_smoothness(st, g, fx, fy, c->dpsis, half_alpha, two_frame_reg, 1, A + SP_PH * P, A + SP_PV * P);
-            } else {
-                launch_update_smoothness(st, g, fx, fy, pdu, pdv, c->dpsis, half_alpha, two_frame_reg, 1, ax, ay,
-                                         A + SP_PH * P, A + SP_PV * P);
-                std::swap(fx, ax);
-                std::swap(fy, ay);
-            }
             cudaEvent_t ev;
-            c->prof_begin(PROF_DATA, ev);
-            launch_prep_two_frame(st, g, c->num_sms, d_im1, d_im2, fx, fy, nullptr, nullptr, A + SP_PH * P, A + SP_PV * P,
-                                  half_delta_over3, half_gamma_over3, A + SP_A11 * P, A + SP_A12 * P, A + SP_A22 * P,
-                                  A + SP_B1 * P, A + SP_B2 * P);
-            c->prof_end(PROF_DATA, ev);
+            if (fused_psi) {
+                c->prof_begin(PROF_DATA, ev);
+                launch_prep_fused(st, g, c->num_sms, d_im1, d_im2, fx, fy, pdu, pdv, c->dpsis, half_alpha, half_delta_over3,
+                                  half_gamma_over3, ax, ay, A + SP_PH * P, A + SP_PV * P, A + SP_A11 * P, A + SP_A12 * P,
+                                  A + SP_A22 * P, A + SP_B1 * P, A + SP_B2 * P);
+                c->prof_end(PROF_DATA, ev);
+                if (outer > 0) {
+                    std::swap(fx, ax);
+                    std::swap(fy, ay);
+                }
+                c->prof_acc.kernel_launches += 1;
+            } else {
+                if (outer == 0) {
+                    launch_smoothness(st, g, fx, fy, c->dpsis, half_alpha, two_frame_reg, 1, A + SP_PH * P, A + SP_PV * P);
+                } else {
+                    launch_update_smoothness(st, g, fx, fy, pdu, pdv, c->dpsis, half_alpha, two_frame_reg, 1, ax, ay,
+                                             A + SP_PH * P, A + SP_PV * P);
+                    std::swap(fx, ax);
+                    std::swap(fy, ay);
+                }
+                c->prof_begin(PROF_DATA, ev);
+                launch_prep_two_frame(st, g, c->num_sms, d_im1, d_im2, fx, fy, nullptr, nullptr, A + SP_PH * P, A + SP_PV * P,
+                                      half_delta_over3, half_gamma_over3, A + SP_A11 * P, A + SP_A12 * P, A + SP_A22 * P,
+                                      A + SP_B1 * P, A + SP_B2 * P);
+                c->prof_end(PROF_DATA, ev);
+                c->prof_acc.kernel_launches += 2;
+            }
             c->prof_acc.data_launches++;
             c->prof_acc.data_pixels += (long long)g.W * g.H;
-            c->prof_acc.kernel_launches += 2;
             int cur = 0;
             rc = run_sor(c, params->niter_solver, params->sor_omega, &cur, true); // variational.c:57
             if (rc != SFGPU_OK) return rc;

@@ -27,7 +27,7 @@ struct sfgpu_ctx {
     int num_sms = 148;
 
     int sor_variant = 0; // 0 tiled, 1 per-half-sweep launches
-    int data_variant = 0; // 0 fused marching warp+data-term kernel, 1 separate warp + tile kernel (env SLOWFLOW_GPU_DATA_VARIANT)
+    int data_variant = 0; // 0 fused marching data pass, 1 separate warp + tile kernel, 2 as 0 with a separate smoothness pass (env SLOWFLOW_GPU_DATA_VARIANT)
     int sor_fuse = 0;    // 0 = auto
     int mt_warp_variant = 0; // 0: fused warp + per-frame derivatives (sf_wderivs.cu), 1: k_warp + k_data_term<DK_DERIVS> (env SLOWFLOW_GPU_MT_WARP_VARIANT)
     bool mt_terms_scalar = false; // env SLOWFLOW_GPU_MT_TERMS_SCALAR: one column per thread in the all-terms pass (A/B switch)

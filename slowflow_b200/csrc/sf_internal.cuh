@@ -157,6 +157,14 @@ void launch_mt_terms(cudaStream_t st, Geom g, const MtTermsArgs &ta, const DataC
 void launch_prep_two_frame(cudaStream_t st, Geom g, int num_sms, const float *im1, const float *im2, const float *wx, const float *wy, const float *du, const float *dv, const float *ph, const float *pv,
                            float half_delta_over3, float half_gamma_over3, float *a11, float *a12, float *a22, float *b1,
                            float *b2);
+// One outer iteration of the two-frame loop with niter_inner == 1 in one pass (sf_prep.cu): launch_update_smoothness
+// (du != nullptr: the flow is wx + du, stored to wx_out / wy_out) or launch_smoothness (du == nullptr) with the two-frame
+// penalty and mode 1, followed by launch_prep_two_frame on that flow and its diffusivities (also stored to ph / pv) at
+// a zero increment.  The same planes as the two launches, bit for bit.
+void launch_prep_fused(cudaStream_t st, Geom g, int num_sms, const float *im1, const float *im2, const float *wx, const float *wy,
+                       const float *du, const float *dv, const float *dpsis, float half_alpha, float half_delta_over3,
+                       float half_gamma_over3, float *wx_out, float *wy_out, float *ph, float *pv, float *a11, float *a12,
+                       float *a22, float *b1, float *b2);
 // convolve_horiz / convolve_vert over `planes` planes (operator twins; order 1 = 3 taps, 2 = 5 taps)
 void launch_convolve(cudaStream_t st, Geom g, const float *src, float *dst, bool vertical, int order, const float *coeffs,
                      int planes);

@@ -9,6 +9,9 @@
 //     block inverse of sor_coupled's first sweep              solver.c:101-106
 // HBM traffic: read wx,wy (8 B/px) + im1 (12) + im2 through L1/L2 gathers (12) + psi_h,psi_v (8); write the five
 // system planes (20).  SURVEY 8(d) counts 52 B/px for this step.
+// k_prep_fused (the default loop, niter_inner == 1) also does the smoothness pass that precedes it (k_flow_smooth):
+// it reads dpsis (4 B/px) and, after the first outer iteration, du,dv (8) instead of psi_h,psi_v, and writes
+// psi_h,psi_v (8) and the updated flow (8): 64 B/px in the first outer iteration, 80 after it.
 //
 // Work decomposition (no CTA barrier):
 //   * one WARP owns a strip of 64 columns (lane l = columns 2l, 2l+1) and marches down a segment of rows;
@@ -27,6 +30,7 @@
 // reproduces the replicate border of the first derivative stage; the second stage (d/dx of Ix, d/dy of Iy)
 // replicates the first-stage VALUE, which is patched explicitly in edge strips / segments.
 #include <atomic>
+#include <type_traits>
 
 #include "sf_internal.cuh"
 #include "sf_pack.cuh"
@@ -40,24 +44,46 @@ constexpr int PR_WARPS = 2;                             // warps per CTA (indepe
 #define SF_PREP_MINB 6 // resident CTAs per SM the register allocation aims at (6 x 2 warps, 6 x 30 KB of windows)
 #endif
 constexpr int PR_RING = 60 * 32;                        // packed values of one warp's windows
+constexpr int PR_RING_PSI = 68 * 32;                    // ... plus 4 rows of the flow (u, v) when the kernel forms psi
 
+
+// 1/sqrt of both halves of a pair whose values are >= 1e-6 (or NaN): MUFU.RSQ as rsqrtf issues it, without the
+// rescaling of denormal inputs that rsqrtf wraps around it (it never triggers above FLT_MIN), so the result is
+// bit-identical to rsqrtf's for these inputs
+__device__ __forceinline__ p64 rsqrt2_normal(p64 s) {
+    float a, b;
+    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(a) : "f"(lo_of(s)));
+    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(b) : "f"(hi_of(s)));
+    return pk(a, b);
+}
 
 struct PrepArgs {
     Geom g;
     const float *im1, *im2; // 3 planes each
     const float *wx, *wy;   // flow: warps im2 and is the argument of the Laplacian
-    const float *du, *dv;   // current increment (nullable: 0)
-    const float *ph, *pv;   // smoothness diffusivities
+    const float *du, *dv;   // INC: current increment (nullable: 0); UPDATE: the flow is (wx + du, wy + dv)
+    const float *ph, *pv;   // smoothness diffusivities (read unless the kernel forms them: PSI)
     float *a11, *a12, *a22, *b1, *b2;
     float hd, hg;           // 0.5*delta/3, 0.5*gamma/3
     int strips, seg_rows, nwork;
+    // PSI only: the diffusivities are formed from the flow and the weight map dpsis and stored to (ph_out, pv_out);
+    // UPDATE also stores the updated flow to (wx_out, wy_out)
+    const float *dpsis;
+    float half_alpha;
+    float *ph_out, *pv_out, *wx_out, *wy_out;
 };
 
 // One warp marches down its (strip, segment).  EDGE: the strip touches the left or right image border.
 // INC: the data term is linearised around a non-zero increment (du,dv); the default two-frame path (niter_inner == 1)
-// evaluates it at du = dv = 0, where the residuals are Iz / Ixz / Iyz themselves
-template <bool COLOR, bool EDGE, bool INC>
+// evaluates it at du = dv = 0, where the residuals are Iz / Ixz / Iyz themselves.
+// PSI: the smoothness diffusivities psi_h / psi_v of the output row are computed here (what k_flow_smooth<UPDATE, 1>
+// computes, with the same rounding) instead of being read; UPDATE (PSI only): the flow is w + du, formed on the fly.
+// The flow rows r-3 .. r then live in the warp's ring: a row is loaded once, for the warp, and read back three steps
+// later for the Laplacian and psi of the output row, whose Laplacian window (rows o-1, o, o+1) is exactly what psi_h(o)
+// and psi_v(o) are made of.
+template <bool COLOR, bool EDGE, bool INC, bool PSI = false, bool UPDATE = false>
 __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, const int seg, const int lane, p64 *ring_sm) {
+    static_assert(!(PSI && INC) && (PSI || !UPDATE), "PSI is the niter_inner == 1 form (data term at du = 0)");
     const Geom g = a.g;
     const int W = g.W, H = g.H, H1 = H - 1, S = g.S;
     const int P = (int)g.plane();
@@ -90,19 +116,63 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
     auto rd = [&](int arr, int c, int s) -> p64 { return sm[((arr * 3 + c) * 4 + s) * 32]; };
     auto wr = [&](int arr, int c, int s, p64 v) { sm[((arr * 3 + c) * 4 + s) * 32] = v; };
 #pragma unroll
-    for (int k = 0; k < 60; k++) sm[k * 32] = zero2;
+    for (int k = 0; k < (PSI ? 68 : 60); k++) sm[k * 32] = zero2;
+    // PSI: flow ring, slot s of u / v (the slot of row r is the same as in the derivative windows)
+    enum { RG_FU = 60, RG_FV = 64 };
+    auto frd = [&](int arr, int s) -> p64 { return sm[(arr + s) * 32]; };
+    auto fwr = [&](int arr, int s, p64 v) { sm[(arr + s) * 32] = v; };
 
     // software pipeline: im1 and the flow of the NEXT row to be warped are loaded one step ahead
-    p64 An[3], fx, fy;
+    p64 An[3], fx, fy, fdx = zero2, fdy = zero2;
     {
         const int ro = clampi(Rbase, 0, H1) * S;
 #pragma unroll
         for (int c = 0; c < 3; c++) An[c] = load_pair<EDGE>(a.im1 + c * P, ro, L);
         fx = load_pair<EDGE>(a.wx, ro, L);
         fy = load_pair<EDGE>(a.wy, ro, L);
+        if (UPDATE) {
+            fdx = load_pair<EDGE>(a.du, ro, L);
+            fdy = load_pair<EDGE>(a.dv, ro, L);
+        }
     }
     p64 lu_m = zero2, lu_0 = zero2, lv_m = zero2, lv_0 = zero2; // Laplacian window: flow of rows o-1, o
     p64 vt = zero2;                                            // psi_v of row o-1
+    // PSI: dpsis of row o; the neighbouring lanes' edge columns of the flow: left and right of row o, right of row o-1
+    p64 dw0 = zero2;
+    float u0l = 0.0f, u0r = 0.0f, v0l = 0.0f, v0r = 0.0f, umr = 0.0f, vmr = 0.0f;
+    const p64 ha2 = splat2(a.half_alpha), q2 = splat2(0.25f), eps_s2 = splat2(0.001f * 0.001f);
+
+    // PSI, start of step r: the (updated) flow of row r enters the ring; row o+1 = r-3 comes back out of it with its
+    // edge columns from the neighbouring lanes, and dpsis of row o+1 is loaded
+    auto psi_rows = [&](const int U, const int U1, const int on, p64 &lu_p, p64 &lv_p, p64 &dw_p, float &upl, float &upr,
+                        float &vpl, float &vpr) {
+        if (UPDATE) { // variational.c:60-61 for niter_inner == 1: w + du (k_flow_smooth<1, 1> forms the same sum)
+            fx = add2(fx, fdx);
+            fy = add2(fy, fdy);
+        }
+        fwr(RG_FU, U, fx);
+        fwr(RG_FV, U, fy);
+        lu_p = frd(RG_FU, U1);
+        lv_p = frd(RG_FV, U1);
+        dw_p = load_pair<EDGE>(a.dpsis, on, L);
+        upl = __shfl_up_sync(0xffffffffu, hi_of(lu_p), 1);
+        upr = __shfl_down_sync(0xffffffffu, lo_of(lu_p), 1);
+        vpl = __shfl_up_sync(0xffffffffu, hi_of(lv_p), 1);
+        vpr = __shfl_down_sync(0xffffffffu, lo_of(lv_p), 1);
+    };
+    // psi_v of row o (variational_aux.c:127-142 with the arithmetic of k_flow_smooth: the cross term is
+    // 0.25 * ((w(x+1) - w(x-1)) + (w'(x+1) - w'(x-1))), its square is added by FFMA to dy^2, the two flow components are
+    // summed, and (w + w') * half_alpha is multiplied by MUFU.RSQ of that plus 1e-6); 0 in the last row and beyond W-1
+    auto psi_v = [&](const int o, const p64 wl_u, const p64 wr_u, const p64 wl_v, const p64 wr_v, const p64 lu_p,
+                     const p64 lv_p, const p64 dw_p, float upl, float upr, float vpl, float vpr) -> p64 {
+        const p64 tu = mul2(q2, add2(sub2(wr_u, wl_u), sub2(pk(hi_of(lu_p), upr), pk(upl, lo_of(lu_p)))));
+        const p64 tv = mul2(q2, add2(sub2(wr_v, wl_v), sub2(pk(hi_of(lv_p), vpr), pk(vpl, lo_of(lv_p)))));
+        const p64 uy = sub2(lu_p, lu_0), vy = sub2(lv_p, lv_0);
+        const p64 s = add2(add2(fma2(uy, uy, mul2(tu, tu)), fma2(vy, vy, mul2(tv, tv))), eps_s2);
+        const p64 r = mul2(mul2(add2(dw0, dw_p), ha2), rsqrt2_normal(s)); // s >= 1e-6
+        const bool rowok = o < H1;
+        return pk((rowok && L.x0 < W) ? lo_of(r) : 0.0f, (rowok && L.x0 + 1 < W) ? hi_of(r) : 0.0f);
+    };
 
     // one marching step; U = (r - Rbase) & 3 is the ring slot of row r.  Everything is computed unconditionally
     // (rows are clamped); only the stores are predicated, so every shuffle sits in straight-line code.
@@ -111,6 +181,10 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
         const int rr = clampi(r, 0, H1);
         const int o = r - 4, oc = clampi(o, 0, H1);
         const bool out_row = (o >= Y0) && (o < Yend); // warp-uniform
+        const int oo = oc * S, on = clampi(o + 1, 0, H1) * S;
+        p64 lu_p, lv_p, dw_p = zero2; // flow of row o+1; PSI: dpsis of row o+1
+        float upl = 0.0f, upr = 0.0f, vpl = 0.0f, vpr = 0.0f;
+        if (PSI) psi_rows(U, U1, on, lu_p, lv_p, dw_p, upl, upr, vpl, vpr);
 
         // ---- issue the gathers of row r (flow prefetched one step ago) and the loads of the next row
         const Taps t0 = warp_taps(g, fxc0 + lo_of(fx), (float)rr + lo_of(fy));
@@ -127,10 +201,32 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
             for (int c = 0; c < 3; c++) An[c] = load_pair<EDGE>(a.im1 + c * P, rn, L);
             fx = load_pair<EDGE>(a.wx, rn, L);
             fy = load_pair<EDGE>(a.wy, rn, L);
+            if (UPDATE) {
+                fdx = load_pair<EDGE>(a.du, rn, L);
+                fdy = load_pair<EDGE>(a.dv, rn, L);
+            }
         }
-        const int oo = oc * S, on = clampi(o + 1, 0, H1) * S;
-        const p64 lu_p = load_pair<EDGE>(a.wx, on, L), lv_p = load_pair<EDGE>(a.wy, on, L); // flow of row o+1
-        const p64 hr = load_pair<EDGE>(a.ph, oo, L), vb = load_pair<EDGE>(a.pv, oo, L);
+        p64 hr, vb; // psi_h, psi_v of row o
+        if (!PSI) {
+            lu_p = load_pair<EDGE>(a.wx, on, L);
+            lv_p = load_pair<EDGE>(a.wy, on, L);
+            hr = load_pair<EDGE>(a.ph, oo, L);
+            vb = load_pair<EDGE>(a.pv, oo, L);
+        }
+        if (PSI) {
+            // psi_h of row o (variational_aux.c:112-126, arithmetic of k_flow_smooth as in psi_v); 0 from column W-1 on
+            const p64 wl_u = pk(u0l, lo_of(lu_0)), wr_u = pk(hi_of(lu_0), u0r); // columns x-1 / x+1 of row o
+            const p64 wl_v = pk(v0l, lo_of(lv_0)), wr_v = pk(hi_of(lv_0), v0r);
+            const float dwr = __shfl_down_sync(0xffffffffu, lo_of(dw0), 1);
+            const p64 du_ = sub2(lu_p, lu_m), dv_ = sub2(lv_p, lv_m);
+            const p64 tu = mul2(q2, add2(du_, pk(hi_of(du_), upr - umr)));
+            const p64 tv = mul2(q2, add2(dv_, pk(hi_of(dv_), vpr - vmr)));
+            const p64 ux = sub2(wr_u, lu_0), vx = sub2(wr_v, lv_0);
+            const p64 s = add2(add2(fma2(ux, ux, mul2(tu, tu)), fma2(vx, vx, mul2(tv, tv))), eps_s2);
+            const p64 h = mul2(mul2(add2(dw0, pk(hi_of(dw0), dwr)), ha2), rsqrt2_normal(s));
+            hr = pk(L.x0 < W - 1 ? lo_of(h) : 0.0f, L.x0 + 1 < W - 1 ? hi_of(h) : 0.0f);
+            vb = psi_v(o, wl_u, wr_u, wl_v, wr_v, lu_p, lv_p, dw_p, upl, upr, vpl, vpr);
+        }
         p64 u = zero2, v = zero2;
         if (INC) {
             u = load_pair<EDGE>(a.du, oo, L);
@@ -153,8 +249,13 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
         const float hl_lane = __shfl_up_sync(0xffffffffu, hi_of(hr), 1);
         const p64 hl = pk(L.x0 > 0 ? hl_lane : 0.0f, lo_of(hr));
         const p64 vtt = (o > 0) ? vt : zero2;
-        const float ul = __shfl_up_sync(0xffffffffu, hi_of(lu_0), 1), ur = __shfl_down_sync(0xffffffffu, lo_of(lu_0), 1);
-        const float vl = __shfl_up_sync(0xffffffffu, hi_of(lv_0), 1), vr = __shfl_down_sync(0xffffffffu, lo_of(lv_0), 1);
+        float ul, ur, vl, vr;
+        if (PSI) { // carried from the step that brought row o out of the ring
+            ul = u0l; ur = u0r; vl = v0l; vr = v0r;
+        } else {
+            ul = __shfl_up_sync(0xffffffffu, hi_of(lu_0), 1), ur = __shfl_down_sync(0xffffffffu, lo_of(lu_0), 1);
+            vl = __shfl_up_sync(0xffffffffu, hi_of(lv_0), 1), vr = __shfl_down_sync(0xffffffffu, lo_of(lv_0), 1);
+        }
         float mk0, mk1;
         {
             const float xx0 = fxc0 + lo_of(lu_0), yy0 = (float)o + lo_of(lv_0);
@@ -253,21 +354,52 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
             *reinterpret_cast<float2 *>(a.a22 + off) = make_float2(v0 ? lo_of(i22) : 0.0f, v1 ? hi_of(i22) : 0.0f);
             *reinterpret_cast<float2 *>(a.b1 + off) = make_float2(v0 ? lo_of(b1) : 0.0f, v1 ? hi_of(b1) : 0.0f);
             *reinterpret_cast<float2 *>(a.b2 + off) = make_float2(v0 ? lo_of(b2) : 0.0f, v1 ? hi_of(b2) : 0.0f);
+            if (PSI) { // (already 0 in the padding columns)
+                *reinterpret_cast<p64 *>(a.ph_out + off) = hr;
+                *reinterpret_cast<p64 *>(a.pv_out + off) = vb;
+            }
+            if (UPDATE) {
+                // the updated flow goes to the other buffer (neighbouring rows are read by other warps).  The ring holds
+                // clamped columns; padding columns get the unclamped sum, as k_flow_smooth<1, 1> stores it
+                p64 su = lu_0, sv = lv_0;
+                if (EDGE && L.x0 + 1 >= W) {
+                    float u0 = lo_of(su), v0f = lo_of(sv);
+                    if (L.x0 >= W) {
+                        u0 = a.wx[off] + a.du[off];
+                        v0f = a.wy[off] + a.dv[off];
+                    }
+                    su = pk(u0, a.wx[off + 1] + a.du[off + 1]);
+                    sv = pk(v0f, a.wy[off + 1] + a.dv[off + 1]);
+                }
+                *reinterpret_cast<p64 *>(a.wx_out + off) = su;
+                *reinterpret_cast<p64 *>(a.wy_out + off) = sv;
+            }
         }
 
         // ---- rotate the row windows of the Laplacian
         vt = vb;
         lu_m = lu_0; lu_0 = lu_p;
         lv_m = lv_0; lv_0 = lv_p;
+        if (PSI) {
+            umr = u0r; u0l = upl; u0r = upr;
+            vmr = v0r; v0l = vpl; v0r = vpr;
+            dw0 = dw_p;
+        }
     };
 
     // The first 8 steps of a segment only fill the windows (their output rows lie above the segment): the lean step
     // loads / warps row r and rotates the windows exactly like step(), but skips the second-stage derivatives, the data
     // term, the Laplacian and the block inverse -- about 60 % of a step's instructions.
-    auto lean_step = [&](const int U, const int r) {
+    // LAST (a std::bool_constant): the last warm-up step, the only one whose psi_v is used (PSI); a compile-time switch,
+    // since a run-time test in the rolled loop costs registers
+    auto lean_step = [&](const int U, const int r, auto LAST) {
         const int U1 = (U + 1) & 3, U2 = (U + 2) & 3, U3 = (U + 3) & 3;
         const int rr = clampi(r, 0, H1);
         const int o = r - 4;
+        const int oo = clampi(o, 0, H1) * S, on = clampi(o + 1, 0, H1) * S;
+        p64 lu_p, lv_p, dw_p = zero2;
+        float upl = 0.0f, upr = 0.0f, vpl = 0.0f, vpr = 0.0f;
+        if (PSI) psi_rows(U, U1, on, lu_p, lv_p, dw_p, upl, upr, vpl, vpr);
         const Taps t0 = warp_taps(g, fxc0 + lo_of(fx), (float)rr + lo_of(fy));
         const Taps t1 = warp_taps(g, fxc1 + hi_of(fx), (float)rr + hi_of(fy));
         p64 A[3], B[3];
@@ -282,10 +414,22 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
             for (int c = 0; c < 3; c++) An[c] = load_pair<EDGE>(a.im1 + c * P, rn, L);
             fx = load_pair<EDGE>(a.wx, rn, L);
             fy = load_pair<EDGE>(a.wy, rn, L);
+            if (UPDATE) {
+                fdx = load_pair<EDGE>(a.du, rn, L);
+                fdy = load_pair<EDGE>(a.dv, rn, L);
+            }
         }
-        const int oo = clampi(o, 0, H1) * S, on = clampi(o + 1, 0, H1) * S;
-        const p64 lu_p = load_pair<EDGE>(a.wx, on, L), lv_p = load_pair<EDGE>(a.wy, on, L);
-        const p64 vb = load_pair<EDGE>(a.pv, oo, L);
+        p64 vb = zero2;
+        if (PSI) {
+            // only psi_v of the last warm-up row is used (as psi_v of the row above the first output row)
+            if (decltype(LAST)::value)
+                vb = psi_v(o, pk(u0l, lo_of(lu_0)), pk(hi_of(lu_0), u0r), pk(v0l, lo_of(lv_0)), pk(hi_of(lv_0), v0r), lu_p,
+                           lv_p, dw_p, upl, upr, vpl, vpr);
+        } else {
+            lu_p = load_pair<EDGE>(a.wx, on, L);
+            lv_p = load_pair<EDGE>(a.wy, on, L);
+            vb = load_pair<EDGE>(a.pv, oo, L);
+        }
 #pragma unroll
         for (int c = 0; c < 3; c++) {
             p64 ix_new = hconv_pair(rd(RG_M, c, U2));
@@ -304,6 +448,11 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
         vt = vb;
         lu_m = lu_0; lu_0 = lu_p;
         lv_m = lv_0; lv_0 = lv_p;
+        if (PSI) {
+            umr = u0r; u0l = upl; u0r = upr;
+            vmr = v0r; v0l = vpl; v0r = vpr;
+            dw0 = dw_p;
+        }
     };
 
     const int Rend = Yend + 4; // last loaded row is Yend + 3
@@ -313,7 +462,8 @@ __device__ __forceinline__ void prep_march(const PrepArgs &a, const int strip, c
 #if SF_PREP_LEAN
     // output row o = r - 4 reaches the segment at r = Y0 + 4: steps Rbase .. Y0 + 3 are warm-up
 #pragma unroll 1
-    for (int r = Rbase; r < Y0 + 4; r++) lean_step((r - Rbase) & 3, r);
+    for (int r = Rbase; r < Y0 + 3; r++) lean_step((r - Rbase) & 3, r, std::false_type());
+    lean_step((Y0 + 3 - Rbase) & 3, Y0 + 3, std::true_type());
 #pragma unroll 1
     for (int r = Y0 + 4; r < Rend; r++) step((r - Rbase) & 3, r);
 #else
@@ -336,6 +486,22 @@ __global__ void __launch_bounds__(PR_WARPS * 32, SF_PREP_MINB) k_prep_two_frame(
     else prep_march<COLOR, false, INC>(a, strip, seg, lane, ring_sm);
 }
 
+// One outer iteration of the default two-frame loop (niter_inner == 1) in one pass: k_flow_smooth<UPDATE, 1> (flow
+// update w += du, psi_h / psi_v) followed by k_prep_two_frame<COLOR, 0>, with the same results bit for bit
+template <bool COLOR, bool UPDATE>
+__global__ void __launch_bounds__(PR_WARPS * 32, SF_PREP_MINB) k_prep_fused(PrepArgs a) {
+    pdl_enter();
+    __shared__ p64 ring[PR_WARPS * PR_RING_PSI];
+    const int lane = threadIdx.x & 31;
+    const int work = blockIdx.x * PR_WARPS + (threadIdx.x >> 5);
+    if (work >= a.nwork) return; // whole warp
+    const int strip = work % a.strips, seg = work / a.strips;
+    const int X0 = strip * PR_OUT_W - 2 * PR_OUT_LO;
+    p64 *ring_sm = ring + (threadIdx.x >> 5) * PR_RING_PSI;
+    if ((X0 < 0) || (X0 + 63 > a.g.W - 1)) prep_march<COLOR, true, false, true, UPDATE>(a, strip, seg, lane, ring_sm);
+    else prep_march<COLOR, false, false, true, UPDATE>(a, strip, seg, lane, ring_sm);
+}
+
 // rows per segment: the largest number of (strip, segment) work items that is still ONE wave of resident warps
 // (a second, mostly empty wave would double the kernel time), but at least 16 rows (8 warm-up rows per segment)
 static int prep_seg_rows(Geom g, int num_sms, int resident_warps_per_sm) {
@@ -347,15 +513,15 @@ static int prep_seg_rows(Geom g, int num_sms, int resident_warps_per_sm) {
     return (rows + 3) & ~3;
 }
 
-template <bool COLOR, bool INC>
-static void launch_prep_variant(cudaStream_t st, Geom g, int num_sms, PrepArgs &a) {
+template <void (*KERNEL)(PrepArgs)>
+static void launch_march(cudaStream_t st, Geom g, int num_sms, PrepArgs &a) {
     // resident warps per SM (the same on every device of the box: all are sm_100a; relaxed atomics because one host
     // thread per device may get here at the same time)
     static std::atomic<int> resident{0};
     int res = resident.load(std::memory_order_relaxed);
     if (!res) {
         int blocks_per_sm = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, k_prep_two_frame<COLOR, INC>, PR_WARPS * 32, 0);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, KERNEL, PR_WARPS * 32, 0);
         res = (blocks_per_sm > 0 ? blocks_per_sm : 1) * PR_WARPS;
         resident.store(res, std::memory_order_relaxed);
     }
@@ -363,7 +529,33 @@ static void launch_prep_variant(cudaStream_t st, Geom g, int num_sms, PrepArgs &
     const int segs = (g.H + a.seg_rows - 1) / a.seg_rows;
     a.nwork = a.strips * segs;
     const int blocks = (a.nwork + PR_WARPS - 1) / PR_WARPS;
-    launch_pdl(k_prep_two_frame<COLOR, INC>, dim3(blocks), dim3(PR_WARPS * 32), 0, st, a);
+    launch_pdl(KERNEL, dim3(blocks), dim3(PR_WARPS * 32), 0, st, a);
+}
+template <bool COLOR, bool INC>
+static void launch_prep_variant(cudaStream_t st, Geom g, int num_sms, PrepArgs &a) {
+    launch_march<k_prep_two_frame<COLOR, INC>>(st, g, num_sms, a);
+}
+
+void launch_prep_fused(cudaStream_t st, Geom g, int num_sms, const float *im1, const float *im2, const float *wx, const float *wy,
+                       const float *du, const float *dv, const float *dpsis, float half_alpha, float half_delta_over3,
+                       float half_gamma_over3, float *wx_out, float *wy_out, float *ph, float *pv, float *a11, float *a12,
+                       float *a22, float *b1, float *b2) {
+    PrepArgs a;
+    a.g = g;
+    a.im1 = im1; a.im2 = im2; a.wx = wx; a.wy = wy; a.du = du; a.dv = dv; a.ph = nullptr; a.pv = nullptr;
+    a.a11 = a11; a.a12 = a12; a.a22 = a22; a.b1 = b1; a.b2 = b2;
+    a.hd = half_delta_over3; a.hg = half_gamma_over3;
+    a.strips = (g.S + PR_OUT_W - 1) / PR_OUT_W;
+    a.dpsis = dpsis; a.half_alpha = half_alpha;
+    a.ph_out = ph; a.pv_out = pv; a.wx_out = wx_out; a.wy_out = wy_out;
+    const bool update = du != nullptr;
+    if (half_delta_over3 != 0.0f) {
+        if (update) launch_march<k_prep_fused<true, true>>(st, g, num_sms, a);
+        else launch_march<k_prep_fused<true, false>>(st, g, num_sms, a);
+    } else {
+        if (update) launch_march<k_prep_fused<false, true>>(st, g, num_sms, a);
+        else launch_march<k_prep_fused<false, false>>(st, g, num_sms, a);
+    }
 }
 
 void launch_prep_two_frame(cudaStream_t st, Geom g, int num_sms, const float *im1, const float *im2, const float *wx, const float *wy, const float *du, const float *dv, const float *ph, const float *pv,

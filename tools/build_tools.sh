@@ -14,4 +14,5 @@ done
 wait
 [ -n "$SOR_ONLY" ] && exit 0
 $NV -o bin/ffma_bench ffma_bench.cu
+$NV -o bin/prep_bench prep_bench.cu
 $NV -o bin/tma_bw tma_bw.cu -lcuda
