@@ -330,6 +330,16 @@ typedef struct sfgpu_epic_stats_s {
  * params->euc is ADDED TO THE CALLER'S ARRAY.  stats may be NULL.  The reference's n_thread argument has no meaning here. */
 int sfgpu_epic(sfgpu_ctx *ctx, image_t *flowx, image_t *flowy, const color_image_t *im, const float_image *input_matches,
                float_image *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats);
+/* epic() on n images of ONE geometry in one call: item k is exactly sfgpu_epic(ctx, flowx[k], flowy[k], im[k],
+ * input_matches[k], edges[k], params, &stats[k]).  params is shared; match counts may differ per item.  euc is added to
+ * every caller's edges[k] once, like sfgpu_epic (so the edges[k] must be distinct arrays).  stats: n entries or NULL.
+ * The items' distance transforms, neighbour searches and fits run side by side on the device, which is what makes a batch
+ * faster than n calls.  On error nothing is written to any flow plane and the message names the first failing item;
+ * SFGPU_ERR_ARG for n < 1, a null pointer, items of different width / height / stride, any check sfgpu_epic makes, and an
+ * item with no match left after the filters. */
+int sfgpu_epic_batch(sfgpu_ctx *ctx, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                     const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params,
+                     sfgpu_epic_stats_t *stats);
 /* operator twin of dist_trf_nnfield_subset (epic_aux.cpp:350-401) with the seeds as the query points: the label map
  * (w*h), and per seed the nn nearest seeds over the geodesic neighbourhood graph with their distances */
 int sfgpu_epic_nnfield(sfgpu_ctx *ctx, int *best, float *dist, int *labels, const int *seeds, int ns, int nn,

@@ -64,7 +64,7 @@ ABI_SYMBOLS = [
     "sfgpu_host_unregister", "sfgpu_variational_mt", "sfgpu_mt_frame_cache", "sfgpu_normalize", "sfgpu_get_mt_stats", "sfgpu_profile_enable",
     "sfgpu_profile_reset", "sfgpu_profile_get", "sfgpu_image_warp", "sfgpu_warp_frame_derivs", "sfgpu_compute_dpsis_weight",
     "sfgpu_compute_smoothness", "sfgpu_compute_data_and_match", "sfgpu_prep_two_frame", "sfgpu_sub_laplacian", "sfgpu_sor_coupled",
-    "sfgpu_epic", "sfgpu_epic_nnfield", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
+    "sfgpu_epic", "sfgpu_epic_batch", "sfgpu_epic_nnfield", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
     "sfgpu_write_flo", "sfgpu_read_flo_size", "sfgpu_read_flo", "sfgpu_write_occlusion_pbm", "sfgpu_set_device", "sfgpu_get_device",
     "sfgpu_convolve_horiz", "sfgpu_convolve_vert", "sfgpu_color_image_convolve_hv", "sfgpu_get_derivatives",
 ]
@@ -137,6 +137,8 @@ def load_library(path=None):
     lib.epic_params_default.restype = None
     lib.sfgpu_epic.argtypes = [C.c_void_p, IP, IP, CP, C.POINTER(FloatImage), C.POINTER(FloatImage), C.POINTER(EpicParams),
                                C.POINTER(EpicStats)]
+    lib.sfgpu_epic_batch.argtypes = [C.c_void_p, C.c_int, C.POINTER(IP), C.POINTER(IP), C.POINTER(CP), C.POINTER(C.POINTER(FloatImage)),
+                                     C.POINTER(C.POINTER(FloatImage)), C.POINTER(EpicParams), C.POINTER(EpicStats)]
     lib.sfgpu_epic_nnfield.argtypes = [C.c_void_p, C.POINTER(C.c_int), FP, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int, C.c_int, FP,
                                        C.c_int, C.c_int, C.POINTER(C.c_int)]
     lib.sfgpu_grid_mincut.argtypes = [C.c_int, C.c_int, FP, FP, C.c_float, C.c_int, C.POINTER(C.c_int)]
@@ -269,6 +271,28 @@ class Context:
         _check(self.lib, self.lib.sfgpu_epic(self.h, flowx.ptr(), flowy.ptr(), im.ptr(), C.byref(m), C.byref(e), C.byref(params),
                                              C.byref(st)), "sfgpu_epic")
         return st
+
+    def epic_batch(self, flowsx, flowsy, ims, matches, edges, params=None):
+        """epic() on n images of one geometry in one call (sfgpu_epic_batch): item k gets exactly what
+        ``epic(flowsx[k], flowsy[k], ims[k], matches[k], edges[k], params)`` gives it.  Same input checks as ``epic``;
+        params.euc is added IN PLACE to every edges[k].  Returns the list of the items' EpicStats."""
+        import numpy as np
+        n = len(flowsx)
+        assert len(flowsy) == n and len(ims) == n and len(matches) == n and len(edges) == n
+        for im, m, e in zip(ims, matches, edges):
+            assert m.dtype == np.float32 and m.flags.c_contiguous and m.ndim == 2
+            assert e.dtype == np.float32 and e.flags.c_contiguous and e.shape == (im.height, im.width)
+        if params is None:
+            params = epic_params_default()
+        FP, IP, CP, FIP = C.POINTER(C.c_float), C.POINTER(image_t), C.POINTER(color_image_t), C.POINTER(FloatImage)
+        ms = [FloatImage(m.ctypes.data_as(FP), m.shape[1], m.shape[0]) for m in matches]
+        es = [FloatImage(e.ctypes.data_as(FP), e.shape[1], e.shape[0]) for e in edges]
+        st = (EpicStats * max(n, 1))()
+        _check(self.lib, self.lib.sfgpu_epic_batch(self.h, n, (IP * n)(*[C.pointer(f.c) for f in flowsx]),
+                                                   (IP * n)(*[C.pointer(f.c) for f in flowsy]), (CP * n)(*[C.pointer(i.c) for i in ims]),
+                                                   (FIP * n)(*[C.pointer(m) for m in ms]), (FIP * n)(*[C.pointer(e) for e in es]),
+                                                   C.byref(params), st), "sfgpu_epic_batch")
+        return list(st[:n])
 
     def epic_nnfield(self, seeds, nn, cost):
         """seeds: int32 (ns, 2) x y; cost: float32 (H, W).  -> (labels (H, W), best (ns, nn), dist (ns, nn), sweeps)."""

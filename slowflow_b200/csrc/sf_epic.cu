@@ -45,11 +45,15 @@ constexpr unsigned EPIC_UNSEEN = 0x7F7F7F7Fu; // memset(…, 0x7F, …) pattern 
 
 // ------------------------------------------------------------------------------------------ saliency (image.c:728-790)
 struct ConvTaps { int order; float c[17]; }; // c[order + k] = weight of src[i + k]
+// The image-sized kernels of a call cover all its items at once: blockIdx.z is the item, and the item's planes lie zs floats
+// after those of the item before it.
 __global__ void __launch_bounds__(256) k_conv_any(Geom g, const float *__restrict__ src, float *__restrict__ dst, ConvTaps t, int vertical,
-                                                  int planes) {
+                                                  int planes, size_t zs) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
     if (i >= g.W || j >= g.H) return;
     const size_t P = g.plane();
+    src += blockIdx.z * zs;
+    dst += blockIdx.z * zs;
     for (int c = 0; c < planes; c++) {
         const float *s = src + c * P;
         float sum = 0.0f;
@@ -61,20 +65,20 @@ __global__ void __launch_bounds__(256) k_conv_any(Geom g, const float *__restric
     }
 }
 __global__ void __launch_bounds__(256) k_autocorr(Geom g, const float *__restrict__ ix, const float *__restrict__ iy, float *__restrict__ xx,
-                                                  float *__restrict__ xy, float *__restrict__ yy) {
+                                                  float *__restrict__ xy, float *__restrict__ yy, size_t zs) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
     if (i >= g.W || j >= g.H) return;
-    const size_t P = g.plane(), o = (size_t)j * g.S + i;
+    const size_t P = g.plane(), o = (size_t)j * g.S + i + blockIdx.z * zs;
     const float a0 = ix[o], a1 = ix[o + P], a2 = ix[o + 2 * P], b0 = iy[o], b1 = iy[o + P], b2 = iy[o + 2 * P];
     xx[o] = a0 * a0 + a1 * a1 + a2 * a2;
     xy[o] = a0 * b0 + a1 * b1 + a2 * b2;
     yy[o] = b0 * b0 + b1 * b1 + b2 * b2;
 }
 __global__ void __launch_bounds__(256) k_min_eig(Geom g, const float *__restrict__ xx, const float *__restrict__ xy, const float *__restrict__ yy,
-                                                 float *__restrict__ out) {
+                                                 float *__restrict__ out, size_t zs) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
     if (i >= g.W || j >= g.H) return;
-    const size_t o = (size_t)j * g.S + i;
+    const size_t o = (size_t)j * g.S + i + blockIdx.z * zs;
     const float t = 0.5f * (xx[o] + yy[o]);
     out[o] = sqrtf(fmaxf(0.0f, t - sqrtf(fmaxf(0.0f, t * t + xy[o] * xy[o] - xx[o] * yy[o]))));
 }
@@ -96,43 +100,57 @@ static ConvTaps gaussian_taps(float sigma) { // gaussian_filter + convolution_ne
 }
 
 // ------------------------------------------------------------------------------------------ small per-match kernels
-__global__ void k_gather_plane(int n, const int *__restrict__ seeds, Geom g, const float *__restrict__ plane, float *__restrict__ out) {
+// pos: (x, y, item) per match; the item's plane lies item * zs floats after `plane`
+__global__ void k_gather_plane(int n, const int *__restrict__ pos, Geom g, const float *__restrict__ plane, size_t zs, float *__restrict__ out) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < n) out[k] = plane[(size_t)seeds[2 * k + 1] * g.S + seeds[2 * k]];
+    if (k < n) out[k] = plane[(size_t)pos[3 * k + 2] * zs + (size_t)pos[3 * k + 1] * g.S + pos[3 * k]];
 }
 __global__ void k_fill_u32(size_t n, unsigned *__restrict__ dst, unsigned v) {
     for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (size_t)gridDim.x * blockDim.x) dst[k] = v;
 }
-// seeds onto the distance / label maps: dmap[p] = cost[p]; of several seeds on one pixel the LAST one wins (the reference
-// writes them in order, epic_aux.cpp:319-323)
-__global__ void k_dt_seed_labels(int ns, const int *__restrict__ seeds, int W, int *__restrict__ labels) {
+// The seeds of the n items of a call carry global ids: item k owns off[k] .. off[k+1]-1, in its own order, and label maps
+// hold global ids.  So the keys of the border list sort by item, one CSR covers all seeds and no graph edge crosses items.
+struct SeedItems {
+    const int *item; // per seed: its item
+    const int *off;  // per item: its first seed
+    const int *nns;  // per item: neighbours searched (min(nn, its seeds))
+};
+// seeds onto the distance / label maps (W x H = N pixels per item): dmap[p] = cost[p]; of several seeds on one pixel the
+// LAST one wins (the reference writes them in order, epic_aux.cpp:319-323; ids of one item keep its order)
+__global__ void k_dt_seed_labels(int ns, const int *__restrict__ seeds, const int *__restrict__ item, int W, size_t N, int *__restrict__ labels) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < ns) atomicMax(labels + (size_t)seeds[2 * k + 1] * W + seeds[2 * k], k);
+    if (k < ns) atomicMax(labels + item[k] * N + (size_t)seeds[2 * k + 1] * W + seeds[2 * k], k);
 }
-__global__ void k_dt_seed_dist(int ns, const int *__restrict__ seeds, int W, const float *__restrict__ cost, float *__restrict__ dmap) {
+__global__ void k_dt_seed_dist(int ns, const int *__restrict__ seeds, const int *__restrict__ item, int W, size_t N, const float *__restrict__ cost,
+                               float *__restrict__ dmap) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k < ns) {
-        const size_t p = (size_t)seeds[2 * k + 1] * W + seeds[2 * k];
+        const size_t p = item[k] * N + (size_t)seeds[2 * k + 1] * W + seeds[2 * k];
         dmap[p] = cost[p];
     }
 }
 
 // ------------------------------------------------------------------------------------------ distance transform sweeps
-struct DtCtrl {
+struct DtCtrl { // one per item
     int end_iter;                   // sweeps with index > end_iter are skipped (epic_aux.cpp:170-178)
     int sweeps_run;
     unsigned maxdiff[DT_MAX_SWEEPS + 1]; // float bits of the largest decrease of sweep k (non-negative: ordered like ints)
+};
+struct DtGroup { // one per group of items whose transforms run side by side
+    int end_iter;                   // the largest end_iter of the group's items
     int ticket[DT_MAX_SWEEPS + 1];
 };
 struct DtSweepArgs {
     int W, H, NS, NB; // image, strips of 32 rows, blocks of 32 columns
+    int n;            // items of the group: their planes follow each other (W x H each)
     const float *cost;
     float *A;
     int *L;
     int sx, sy;       // sweep direction (+1 / -1)
     int k;            // sweep index, 1-based
-    DtCtrl *ctrl;
-    int *prog;        // per strip (in sweep order): k * 65536 + column blocks finished and stored in sweep k
+    DtCtrl *ctrl;     // per item
+    DtGroup *grp;
+    int *prog;        // per item and strip (in sweep order): k * 65536 + column blocks finished and stored in sweep k
 };
 
 __device__ __forceinline__ int ld_acquire_gpu(const int *p) {
@@ -222,8 +240,11 @@ __device__ __forceinline__ void dt_wait_smem(const volatile int *cnt, int need) 
 // step and wraps once per 96 steps.  Row pitch 98 floats: lane l reads column (s - l) of row l at step s -> bank
 // (2 l + s - l) % 32 = (l + s) % 32, conflict-free; the mover's row-wise accesses are conflict-free anyway.
 constexpr int DT_COLS = DT_RING * DT_TILE, DT_ROWP = DT_COLS + 2, DT_ARR = DT_TILE * DT_ROWP;
+// A group of items runs its sweeps in the same launches.  The strips of all its items share one ticket sequence in sweep
+// order (ticket t = strip t / n of item t % n), so every strip still only waits for the strip above it in its own image,
+// which holds a smaller ticket.  An item past its own end_iter returns at once, as a single transform does.
 __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
-    if (a.k > *reinterpret_cast<volatile int *>(&a.ctrl->end_iter)) return;
+    if (a.k > *reinterpret_cast<volatile int *>(&a.grp->end_iter)) return;
     // [A | L | cost] arrays, then the halo row (t, label) of the strip above in the same circular column index
     __shared__ __align__(16) float smem[3 * DT_ARR + 2 * DT_COLS];
     __shared__ int s_strip;
@@ -238,15 +259,23 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
     const bool mover = threadIdx.x >= 32;
     const float INF = __int_as_float(0x7f800000);
     if (threadIdx.x == 0) {
-        s_strip = atomicAdd(&a.ctrl->ticket[a.k], 1);
+        s_strip = atomicAdd(&a.grp->ticket[a.k], 1);
         s_full = 0;
         s_done = 0;
     }
     __syncthreads();
-    const int strip = s_strip;
-    if (strip >= a.NS) return;
+    const int ticket = s_strip;
+    if (ticket >= a.NS * a.n) return;
+    const int item = ticket % a.n, strip = ticket / a.n;
+    DtCtrl *const ctrl = a.ctrl + item;
+    if (a.k > *reinterpret_cast<volatile int *>(&ctrl->end_iter)) return;
     const int W = a.W, H = a.H, q0 = strip * DT_TILE, rows = min(DT_TILE, H - q0);
     const int NB = a.NB;
+    const size_t item_off = (size_t)item * W * H;
+    const float *const cost = a.cost + item_off;
+    float *const gA = a.A + item_off;
+    int *const gL = a.L + item_off;
+    int *const prog = a.prog + item * a.NS;
 
     if (mover) {
         const int jtop = (a.sy > 0) ? q0 - 1 : H - q0; // image row of sweep row q0 - 1 (the last row of the strip above)
@@ -260,9 +289,9 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
                 for (int r = 0; r < rows; r++) {
                     const size_t o = (size_t)(a.sy > 0 ? q0 + r : H - 1 - (q0 + r)) * W + i;
                     const int e = r * DT_ROWP + e0;
-                    cp_async4(&sA[e], a.A + o);
-                    cp_async4(&sL[e], a.L + o);
-                    cp_async4(&sC[e], a.cost + o);
+                    cp_async4(&sA[e], gA + o);
+                    cp_async4(&sL[e], gL + o);
+                    cp_async4(&sC[e], cost + o);
                 }
             }
             asm volatile("cp.async.commit_group;" ::: "memory");
@@ -277,8 +306,8 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
                 for (int r = r0; r < r1; r++) {
                     const size_t o = (size_t)(a.sy > 0 ? q0 + r : H - 1 - (q0 + r)) * W + i;
                     const int e = r * DT_ROWP + e0;
-                    a.A[o] = sA[e];
-                    a.L[o] = sL[e];
+                    gA[o] = sA[e];
+                    gL[o] = sL[e];
                 }
             }
         };
@@ -289,12 +318,12 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
                 float t = INF;
                 int l = -1;
                 if (strip > 0) {
-                    if (lane == 0) dt_wait(a.prog + strip - 1, base + m + 1);
+                    if (lane == 0) dt_wait(prog + strip - 1, base + m + 1);
                     __syncwarp();
                     if (p < W) {
                         const int ii = a.sx > 0 ? p : W - 1 - p;
-                        t = __ldcg(a.A + (size_t)jtop * W + ii);
-                        l = __ldcg(a.L + (size_t)jtop * W + ii);
+                        t = __ldcg(gA + (size_t)jtop * W + ii);
+                        l = __ldcg(gL + (size_t)jtop * W + ii);
                     }
                 }
                 hT[(m % DT_RING) * DT_TILE + lane] = t;
@@ -314,7 +343,7 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
                 // visible with lane 0's release: __syncwarp orders them before it, the release is cumulative.
                 store_rows(i - 3, rows - 1, rows);
                 __syncwarp();
-                if (lane == 0) st_release_gpu(a.prog + strip, base + i - 2);
+                if (lane == 0) st_release_gpu(prog + strip, base + i - 2);
                 store_rows(i - 3, 0, rows - 1);
             }
             if (i < NB) load_block(i); // C (after the store: the slot is the one block i-3 was read out of just now)
@@ -369,18 +398,24 @@ __global__ void __launch_bounds__(64) k_dt_sweep(DtSweepArgs a) {
     __threadfence_block();
     if (lane == 0) s_done = NB; // every block may be stored now
     for (int off = 16; off > 0; off >>= 1) maxdiff = fmaxf(maxdiff, __shfl_xor_sync(0xffffffffu, maxdiff, off));
-    if (lane == 0 && maxdiff > 0.0f) atomicMax(&a.ctrl->maxdiff[a.k], __float_as_uint(maxdiff));
+    if (lane == 0 && maxdiff > 0.0f) atomicMax(&ctrl->maxdiff[a.k], __float_as_uint(maxdiff));
 }
-// the loop control of weighted_distance_transform (epic_aux.cpp:170-178) after sweep k
-__global__ void k_dt_control(DtCtrl *c, int k, float min_change, int max_iter) {
+// the loop control of weighted_distance_transform (epic_aux.cpp:170-178) after sweep k; one thread per item of the group
+__global__ void k_dt_control(DtCtrl *ctrl, DtGroup *grp, int n, int k, float min_change, int max_iter) {
+    if ((int)threadIdx.x >= n) return;
+    DtCtrl *c = ctrl + threadIdx.x;
     if (k > c->end_iter) return;
     c->sweeps_run = k;
-    if (__uint_as_float(c->maxdiff[k]) > min_change) c->end_iter = min(max_iter, k + 3);
+    if (__uint_as_float(c->maxdiff[k]) > min_change) {
+        c->end_iter = min(max_iter, k + 3);
+        atomicMax(&grp->end_iter, c->end_iter);
+    }
 }
 
 // ------------------------------------------------------------------------------------------ neighbourhood graph of the seeds
 // (ngh_labels_to_spmat, epic_aux.cpp:226-288): for every pixel with i >= 1 and j >= 1 whose left / upper neighbour carries
-// another label, the edge (l0, l1) with cost dis[p] + dis[q]; emitted in both directions with key = (row << 32) | col
+// another label, the edge (l0, l1) with cost dis[p] + dis[q]; emitted in both directions with key = (row << 32) | col.
+// blockIdx.z is the item (maps of W x H each); the labels are global seed ids, so one list serves all items.
 __global__ void __launch_bounds__(256) k_border_emit(int W, int H, const int *__restrict__ lab, const float *__restrict__ dis,
                                                      unsigned long long *__restrict__ keys, float *__restrict__ vals, int *__restrict__ count, int cap) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
@@ -388,7 +423,7 @@ __global__ void __launch_bounds__(256) k_border_emit(int W, int H, const int *__
     unsigned long long k0 = 0, k1 = 0;
     float d0 = 0.f, d1 = 0.f;
     if (i >= 1 && j >= 1 && i < W && j < H) {
-        const size_t o = (size_t)j * W + i;
+        const size_t o = (size_t)j * W + i + (size_t)blockIdx.z * W * H;
         const int l0 = lab[o], l1 = lab[o - 1], l2 = lab[o - W];
         if (l0 != l1 && l0 >= 0 && l1 >= 0) { k0 = ((unsigned long long)(unsigned)l0 << 32) | (unsigned)l1; d0 = dis[o] + dis[o - 1]; n = 1; }
         if (l0 != l2 && l0 >= 0 && l2 >= 0) { k1 = ((unsigned long long)(unsigned)l0 << 32) | (unsigned)l2; d1 = dis[o] + dis[o - W]; n |= 2; }
@@ -472,28 +507,33 @@ __device__ HeapItem heap_pop(HeapItem *h, int &len) { // pop_heap + pop_back
     h[hole] = v;
     return top;
 }
-// one warp per seed (lane 0 runs the search, the warp restores the tentative-distance array afterwards)
-__global__ void __launch_bounds__(256) k_knn_graph(int ns, int nn, const int *__restrict__ indptr, const int *__restrict__ indices,
+// one warp per seed (lane 0 runs the search, the warp restores the tentative-distance array afterwards).  Rows of nnf / dis
+// are `ld` entries apart, and a seed fills the first nns of its item.  A search never leaves its seed's item, so the
+// per-warp tentative distances are indexed by the node's index within the item: done_all holds `nsmax` (the largest item's
+// seed count) entries per warp.
+__global__ void __launch_bounds__(256) k_knn_graph(int ns, int ld, int nsmax, SeedItems si, const int *__restrict__ indptr, const int *__restrict__ indices,
                                                    const float *__restrict__ data, unsigned *__restrict__ done_all, int *__restrict__ touched_all,
                                                    int *__restrict__ nnf, float *__restrict__ dis, int *__restrict__ overflow, int heap_cap) {
     extern __shared__ HeapItem heaps[];
     const int warp_in_block = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int gwarp = blockIdx.x * (blockDim.x >> 5) + warp_in_block, nwarps = gridDim.x * (blockDim.x >> 5);
     HeapItem *h = heaps + warp_in_block * heap_cap; // heap_cap <= KNN_HEAP entries of shared memory per warp
-    unsigned *done = done_all + (size_t)gwarp * ns; // float bits; EPIC_UNSEEN = not reached (memset 0x7F in the reference)
-    int *touched = touched_all + (size_t)gwarp * KNN_HEAP * 2;
+    unsigned *const done_w = done_all + (size_t)gwarp * nsmax; // float bits; EPIC_UNSEEN = not reached (memset 0x7F in the reference)
+    int *touched = touched_all + (size_t)gwarp * KNN_HEAP * 2;   // (indices within the item)
     for (int seed = gwarp; seed < ns; seed += nwarps) {
         int ntouched = 0, n = 0;
         if (lane == 0) {
+            const int it = si.item[seed], nn = si.nns[it];
+            unsigned *const done = done_w - si.off[it]; // done[node] for the global ids of this item
             int len = 0;
             heap_push(h, len, HeapItem{seed, 0.0f});
             done[seed] = __float_as_uint(0.0f);
-            touched[ntouched++] = seed;
+            touched[ntouched++] = seed - si.off[it];
             while (len > 0) {
                 const HeapItem cur = heap_pop(h, len);
                 if (cur.dis > __uint_as_float(done[cur.node])) continue;
-                nnf[(size_t)seed * nn + n] = cur.node;
-                dis[(size_t)seed * nn + n] = cur.dis;
+                nnf[(size_t)seed * ld + n] = cur.node;
+                dis[(size_t)seed * ld + n] = cur.dis;
                 n++;
                 if (n >= nn) break;
                 for (int e = indptr[cur.node]; e < indptr[cur.node + 1]; e++) {
@@ -502,18 +542,18 @@ __global__ void __launch_bounds__(256) k_knn_graph(int ns, int nn, const int *__
                     if (nd >= __uint_as_float(done[ngh])) continue;
                     if (len >= heap_cap || ntouched >= 2 * KNN_HEAP) { atomicExch(overflow, 1); continue; }
                     heap_push(h, len, HeapItem{ngh, nd});
-                    if (done[ngh] == EPIC_UNSEEN) touched[ntouched++] = ngh;
+                    if (done[ngh] == EPIC_UNSEEN) touched[ntouched++] = ngh - si.off[it];
                     done[ngh] = __float_as_uint(nd);
                 }
             }
             for (int k = n; k < nn; k++) { // not enough results: 0xFF / 0x7F patterns like the reference's memsets
-                nnf[(size_t)seed * nn + k] = -1;
-                dis[(size_t)seed * nn + k] = __uint_as_float(EPIC_UNSEEN);
+                nnf[(size_t)seed * ld + k] = -1;
+                dis[(size_t)seed * ld + k] = __uint_as_float(EPIC_UNSEEN);
             }
         }
         ntouched = __shfl_sync(0xffffffffu, ntouched, 0);
         __syncwarp();
-        for (int k = lane; k < ntouched; k += 32) done[touched[k]] = EPIC_UNSEEN;
+        for (int k = lane; k < ntouched; k += 32) done_w[touched[k]] = EPIC_UNSEEN;
         __syncwarp();
     }
 }
@@ -521,27 +561,32 @@ __global__ void __launch_bounds__(256) k_knn_graph(int ns, int nn, const int *__
 // ------------------------------------------------------------------------------------------ per-seed fits, per-pixel apply
 // query point = seed i: neighbours of the seed that owns its pixel, distances + the pixel's own distance, then the kernel
 // exp(-coef d) + 1e-08 (dist_trf_nnfield_subset :385-394, epic.cpp:96-98, 203-205)
-__global__ void k_query_weights(int ns, int nn, const int *__restrict__ seeds, int W, const int *__restrict__ labels, const float *__restrict__ dmap,
-                                const int *__restrict__ nnf, const float *__restrict__ dis, float coef, int *__restrict__ qnn, float *__restrict__ qw) {
+// (rows of ld entries, the first nns of the seed's item used, like nnf / dis; maps of W x H = N pixels per item)
+__global__ void k_query_weights(int ns, int ld, SeedItems si, const int *__restrict__ seeds, int W, size_t N, const int *__restrict__ labels,
+                                const float *__restrict__ dmap, const int *__restrict__ nnf, const float *__restrict__ dis, float coef, int *__restrict__ qnn,
+                                float *__restrict__ qw) {
     const int i = blockIdx.x, j = threadIdx.x;
     if (i >= ns) return;
-    const size_t p = (size_t)seeds[2 * i + 1] * W + seeds[2 * i];
+    const int it = si.item[i], nn = si.nns[it];
+    const size_t p = it * N + (size_t)seeds[2 * i + 1] * W + seeds[2 * i];
     const int s = labels[p];
     const float d = dmap[p];
     for (int k = j; k < nn; k += blockDim.x) {
-        qnn[(size_t)i * nn + k] = nnf[(size_t)s * nn + k];
-        const float dist = d + dis[(size_t)s * nn + k];
-        qw[(size_t)i * nn + k] = (coef < 0.0f) ? dist : (float)((double)expf(-coef * dist) + 1e-08); // coef < 0: raw distances (operator twin)
+        qnn[(size_t)i * ld + k] = nnf[(size_t)s * ld + k];
+        const float dist = d + dis[(size_t)s * ld + k];
+        qw[(size_t)i * ld + k] = (coef < 0.0f) ? dist : (float)((double)expf(-coef * dist) + 1e-08); // coef < 0: raw distances (operator twin)
     }
 }
 // fit_nadarayawatson (epic_aux.cpp:410-428): sequential float sums in neighbour order
-__global__ void k_fit_nw(int ns, int nn, const int *__restrict__ qnn, const float *__restrict__ qw, const float *__restrict__ vects, float *__restrict__ out) {
+__global__ void k_fit_nw(int ns, int ld, SeedItems si, const int *__restrict__ qnn, const float *__restrict__ qw, const float *__restrict__ vects,
+                         float *__restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= ns) return;
+    const int nn = si.nns[si.item[i]];
     float u = 0.0f, v = 0.0f, s = 0.0f;
     for (int j = 0; j < nn; j++) {
-        const float d = qw[(size_t)i * nn + j];
-        const int jj = qnn[(size_t)i * nn + j];
+        const float d = qw[(size_t)i * ld + j];
+        const int jj = qnn[(size_t)i * ld + j];
         if (jj < 0) continue;
         u = __fadd_rn(u, __fmul_rn(d, vects[2 * jj]));
         v = __fadd_rn(v, __fmul_rn(d, vects[2 * jj + 1]));
@@ -558,10 +603,11 @@ __global__ void k_prefilter_flags(int ns, const float *__restrict__ est, const f
 }
 // fit_localaffine (epic_aux.cpp:438-481).  Rows of the reference's system are (x c, y c, c | (x + wx) c) and the same for y:
 // two weighted least-squares fits (weights c^2) of x' and y' over [x y 1].  Normal equations in double, centred on the seed.
-__global__ void k_fit_la(int ns, int nn, const int *__restrict__ qnn, const float *__restrict__ qw, const int *__restrict__ seeds,
+__global__ void k_fit_la(int ns, int ld, SeedItems si, const int *__restrict__ qnn, const float *__restrict__ qw, const int *__restrict__ seeds,
                          const float *__restrict__ vects, float *__restrict__ aff) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= ns) return;
+    const int nn = si.nns[si.item[i]];
     const double xi = seeds[2 * i], yi = seeds[2 * i + 1];
     double sxx = 0, sxy = 0, sx = 0, syy = 0, sy = 0, s1 = 0, bx0 = 0, bx1 = 0, bx2 = 0, by0 = 0, by1 = 0, by2 = 0;
     auto add = [&](double x, double y, double wx, double wy, float cf) {
@@ -575,9 +621,9 @@ __global__ void k_fit_la(int ns, int nn, const int *__restrict__ qnn, const floa
     };
     float coefi = 0.0f;
     for (int j = 0; j < nn; j++) {
-        const int s = qnn[(size_t)i * nn + j];
+        const int s = qnn[(size_t)i * ld + j];
         if (s < 0) continue;
-        float coef = qw[(size_t)i * nn + j];
+        float coef = qw[(size_t)i * ld + j];
         if (s == i) { coefi = 0.01f * coef; coef *= 0.96f; }
         add((double)seeds[2 * s], (double)seeds[2 * s + 1], (double)vects[2 * s], (double)vects[2 * s + 1], coef);
     }
@@ -600,13 +646,14 @@ __global__ void k_fit_la(int ns, int nn, const int *__restrict__ qnn, const floa
     m[0] = (float)a0; m[1] = (float)a1; m[2] = (float)(a2 + xi - a0 * xi - a1 * yi);
     m[3] = (float)a3; m[4] = (float)a4; m[5] = (float)(a5 + yi - a3 * xi - a4 * yi);
 }
-// apply_localaffine / apply_nadarayawatson (epic_aux.cpp:430-436, 483-492) straight into the flow planes (stride S)
+// apply_localaffine / apply_nadarayawatson (epic_aux.cpp:430-436, 483-492) straight into the flow planes (stride S);
+// blockIdx.z is the item: its label map is W x H further on, its flow planes zs floats
 __global__ void __launch_bounds__(256) k_apply(Geom g, const int *__restrict__ labels, const float *__restrict__ model, int affine, float *__restrict__ fx,
-                                               float *__restrict__ fy) {
+                                               float *__restrict__ fy, size_t zs) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
     if (i >= g.W || j >= g.H) return;
-    const int s = labels[(size_t)j * g.W + i];
-    const size_t o = (size_t)j * g.S + i;
+    const int s = labels[(size_t)j * g.W + i + (size_t)blockIdx.z * g.W * g.H];
+    const size_t o = (size_t)j * g.S + i + blockIdx.z * zs;
     if (s < 0) { fx[o] = 0.0f; fy[o] = 0.0f; return; }
     if (affine) {
         const float *m = model + (size_t)6 * s;
@@ -681,67 +728,113 @@ struct EpicGeo {
     int W, H;
 };
 
-// dist_trf_nnfield_subset with the seeds as query points, followed by the kernel weights: fills qnn / qw (ns x nn) and
-// leaves the label map of the seeds in `labels`.  Everything is queued on the context's stream; returns after one sync.
-static int nn_field(sfgpu_ctx *c, const EpicGeo &eg, const float *d_cost, int ns, int nn, const int *d_seeds, float coef, int *d_labels,
+// The seeds of the n items of one call, host side of SeedItems: item k owns the global ids off[k] .. off[k+1]-1 and
+// searches nns[k] neighbours.
+struct EpicItems {
+    int n = 0;
+    std::vector<int> off, nns, item;
+    SeedItems d{};
+    int ns() const { return off[n]; }
+    int nnmax() const { return *std::max_element(nns.begin(), nns.end()); }
+    int nsmax() const {
+        int m = 0;
+        for (int k = 0; k < n; k++) m = std::max(m, off[k + 1] - off[k]);
+        return m;
+    }
+    int upload(cudaStream_t st) { // the device copies, in the arena
+        item.resize(ns());
+        for (int k = 0; k < n; k++) std::fill(item.begin() + off[k], item.begin() + off[k + 1], k);
+        DevBuf di, doff, dnns;
+        if (!di.alloc(item.size() * 4) || !doff.alloc((size_t)(n + 1) * 4) || !dnns.alloc((size_t)n * 4)) return SFGPU_ERR_CUDA;
+        if (!item.empty()) SF_CUDA(cudaMemcpyAsync(di.p, item.data(), item.size() * 4, cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(doff.p, off.data(), (size_t)(n + 1) * 4, cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(dnns.p, nns.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+        d = SeedItems{di.as<int>(), doff.as<int>(), dnns.as<int>()};
+        return SFGPU_OK;
+    }
+};
+
+// dist_trf_nnfield_subset with the seeds as query points, followed by the kernel weights, for all items of `it` at once:
+// fills qnn / qw (rows of it.nnmax() entries, the first nns of the seed's item used) and leaves the label maps (W x H per
+// item, global seed ids) in `labels`.  Everything is queued on the context's stream; returns after one sync.
+static int nn_field(sfgpu_ctx *c, const EpicGeo &eg, const float *d_cost, const EpicItems &it, const int *d_seeds, float coef, int *d_labels,
                     float *d_dmap, int *d_qnn, float *d_qw, int *sweeps_out) {
     cudaStream_t st = c->stream;
     EpicTrace tr(st);
     ArenaScope scope; // (the caller's buffers were allocated before; the stream is idle when the scratch is released)
-    const int W = eg.W, H = eg.H;
+    const int W = eg.W, H = eg.H, n = it.n, ns = it.ns(), ld = it.nnmax();
     const size_t N = (size_t)W * H;
     const int NS = (H + DT_TILE - 1) / DT_TILE, NB = (W + DT_TILE - 1) / DT_TILE;
-    DevBuf ctrl, prog;
-    if (!ctrl.alloc(sizeof(DtCtrl)) || !prog.alloc((size_t)NS * sizeof(int))) return SFGPU_ERR_CUDA;
-    SF_CUDA(cudaMemsetAsync(ctrl.p, 0, sizeof(DtCtrl), st));
-    SF_CUDA(cudaMemsetAsync(prog.p, 0, (size_t)NS * sizeof(int), st));
-    {
-        const int four = 4;
-        SF_CUDA(cudaMemcpyAsync(&ctrl.as<DtCtrl>()->end_iter, &four, sizeof(int), cudaMemcpyHostToDevice, st)); // end_iter = 4 (:168)
-    }
-    k_fill_u32<<<592, 256, 0, st>>>(N, reinterpret_cast<unsigned *>(d_dmap), EPIC_UNSEEN);
-    k_fill_u32<<<592, 256, 0, st>>>(N, reinterpret_cast<unsigned *>(d_labels), 0xFFFFFFFFu);
-    k_dt_seed_labels<<<(ns + 255) / 256, 256, 0, st>>>(ns, d_seeds, W, d_labels);
-    k_dt_seed_dist<<<(ns + 255) / 256, 256, 0, st>>>(ns, d_seeds, W, d_cost, d_dmap);
-    // sweeps i = 1 .. : direction (x[i % 4], y[i % 4]) with x = {-1, 1, 1, -1}, y = {1, 1, -1, -1} (:165-172).  One warp
-    // per strip of 32 rows; every strip must be resident together with the one above it: tickets hand the strips out in
-    // sweep order, and the grid (one block of two warps and 40 KB of shared memory per strip) is far below the 148 x 5
-    // resident blocks for any real image
-    static const int dx[4] = {-1, 1, 1, -1}, dy[4] = {1, 1, -1, -1};
+    // One block of two warps and 40 KB of shared memory per strip of 32 rows; every strip must be resident together with the
+    // one above it (tickets hand the strips out in sweep order), and 4 blocks per SM always fit.  So the transforms of a
+    // batch run in groups of items whose strips number at most 4 per SM, one group after the other.
     if (NS > c->num_sms * 4) {
         set_error("sfgpu_epic: image too tall for the strip pipeline of the distance transform");
         return SFGPU_ERR_UNSUPPORTED;
     }
-    for (int k = 1; k <= DT_MAX_SWEEPS; k++) {
-        DtSweepArgs a;
-        a.W = W; a.H = H; a.NS = NS; a.NB = NB;
-        a.cost = d_cost; a.A = d_dmap; a.L = d_labels;
-        a.sx = dx[k % 4]; a.sy = dy[k % 4];
-        a.k = k;
-        a.ctrl = ctrl.as<DtCtrl>();
-        a.prog = prog.as<int>();
-        k_dt_sweep<<<NS, 64, 0, st>>>(a);
-        k_dt_control<<<1, 1, 0, st>>>(ctrl.as<DtCtrl>(), k, 1.0f, DT_MAX_SWEEPS); // default dt_params: max_iter 40, min_change 1 (:151-154)
+    const int per_group = std::min(n, c->num_sms * 4 / NS), ngroups = (n + per_group - 1) / per_group;
+    DevBuf ctrl, grp, prog;
+    if (!ctrl.alloc((size_t)n * sizeof(DtCtrl)) || !grp.alloc((size_t)ngroups * sizeof(DtGroup)) || !prog.alloc((size_t)n * NS * sizeof(int)))
+        return SFGPU_ERR_CUDA;
+    std::vector<DtCtrl> h_ctrl((size_t)n);
+    std::vector<DtGroup> h_grp((size_t)ngroups);
+    memset(h_ctrl.data(), 0, h_ctrl.size() * sizeof(DtCtrl));
+    memset(h_grp.data(), 0, h_grp.size() * sizeof(DtGroup));
+    for (auto &x : h_ctrl) x.end_iter = 4; // (:168)
+    for (auto &x : h_grp) x.end_iter = 4;
+    SF_CUDA(cudaMemcpyAsync(ctrl.p, h_ctrl.data(), h_ctrl.size() * sizeof(DtCtrl), cudaMemcpyHostToDevice, st));
+    SF_CUDA(cudaMemcpyAsync(grp.p, h_grp.data(), h_grp.size() * sizeof(DtGroup), cudaMemcpyHostToDevice, st));
+    SF_CUDA(cudaMemsetAsync(prog.p, 0, (size_t)n * NS * sizeof(int), st));
+    k_fill_u32<<<592, 256, 0, st>>>(n * N, reinterpret_cast<unsigned *>(d_dmap), EPIC_UNSEEN);
+    k_fill_u32<<<592, 256, 0, st>>>(n * N, reinterpret_cast<unsigned *>(d_labels), 0xFFFFFFFFu);
+    k_dt_seed_labels<<<(ns + 255) / 256, 256, 0, st>>>(ns, d_seeds, it.d.item, W, N, d_labels);
+    k_dt_seed_dist<<<(ns + 255) / 256, 256, 0, st>>>(ns, d_seeds, it.d.item, W, N, d_cost, d_dmap);
+    // sweeps i = 1 .. : direction (x[i % 4], y[i % 4]) with x = {-1, 1, 1, -1}, y = {1, 1, -1, -1} (:165-172)
+    static const int dx[4] = {-1, 1, 1, -1}, dy[4] = {1, 1, -1, -1};
+    for (int g0 = 0, gi = 0; g0 < n; g0 += per_group, gi++) {
+        const int gn = std::min(per_group, n - g0);
+        for (int k = 1; k <= DT_MAX_SWEEPS; k++) {
+            DtSweepArgs a;
+            a.W = W; a.H = H; a.NS = NS; a.NB = NB; a.n = gn;
+            a.cost = d_cost + g0 * N; a.A = d_dmap + g0 * N; a.L = d_labels + g0 * N;
+            a.sx = dx[k % 4]; a.sy = dy[k % 4];
+            a.k = k;
+            a.ctrl = ctrl.as<DtCtrl>() + g0;
+            a.grp = grp.as<DtGroup>() + gi;
+            a.prog = prog.as<int>() + (size_t)g0 * NS;
+            k_dt_sweep<<<gn * NS, 64, 0, st>>>(a);
+            // default dt_params: max_iter 40, min_change 1 (:151-154)
+            k_dt_control<<<1, gn, 0, st>>>(ctrl.as<DtCtrl>() + g0, grp.as<DtGroup>() + gi, gn, k, 1.0f, DT_MAX_SWEEPS);
+        }
     }
-    c->prof_acc.kernel_launches += 4 + 2 * DT_MAX_SWEEPS;
+    c->prof_acc.kernel_launches += 4 + 2 * DT_MAX_SWEEPS * ngroups;
     tr.mark("distance transform");
 
     // ---- neighbourhood graph
-    // label borders: every border pixel pair emits two entries; ~6 sqrt(N ns) in practice, 4 N at worst
-    const int cap = (int)std::min<size_t>(4 * N, (size_t)(32.0 * sqrt((double)N * (double)ns)) + ((size_t)1 << 20));
+    // label borders: every border pixel pair emits two entries; ~6 sqrt(N ns) per item in practice, 4 N at worst
+    size_t cap_all = 0;
+    for (int k = 0; k < n; k++) cap_all += std::min<size_t>(4 * N, (size_t)(32.0 * sqrt((double)N * (double)(it.off[k + 1] - it.off[k]))) + ((size_t)1 << 20));
+    const int cap = (int)std::min<size_t>(cap_all, (size_t)1 << 30);
     DevBuf keys, vals, keys2, vals2, count, ukeys, uvals, nruns, tmp;
     if (!keys.alloc((size_t)cap * 8) || !vals.alloc((size_t)cap * 4) || !keys2.alloc((size_t)cap * 8) || !vals2.alloc((size_t)cap * 4) ||
         !count.alloc(8) || !nruns.alloc(8))
         return SFGPU_ERR_CUDA;
     SF_CUDA(cudaMemsetAsync(count.p, 0, 8, st));
-    k_border_emit<<<grid2(W, H), dim3(32, 8), 0, st>>>(W, H, d_labels, d_dmap, keys.as<unsigned long long>(), vals.as<float>(), count.as<int>(), cap);
+    dim3 bgrid = grid2(W, H);
+    bgrid.z = n;
+    k_border_emit<<<bgrid, dim3(32, 8), 0, st>>>(W, H, d_labels, d_dmap, keys.as<unsigned long long>(), vals.as<float>(), count.as<int>(), cap);
     int h_count = 0;
-    DtCtrl h_ctrl;
     SF_CUDA(cudaMemcpyAsync(&h_count, count.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    SF_CUDA(cudaMemcpyAsync(&h_ctrl, ctrl.p, sizeof(DtCtrl), cudaMemcpyDeviceToHost, st));
+    SF_CUDA(cudaMemcpyAsync(h_ctrl.data(), ctrl.p, h_ctrl.size() * sizeof(DtCtrl), cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaStreamSynchronize(st));
-    if (sweeps_out) *sweeps_out = h_ctrl.sweeps_run;
-    if (tr.on) fprintf(stderr, "  epic: (distance transform: %d sweeps, %d strips x %d blocks)\n", h_ctrl.sweeps_run, NS, NB);
+    int most_sweeps = 0;
+    for (int k = 0; k < n; k++) {
+        if (sweeps_out) sweeps_out[k] = h_ctrl[k].sweeps_run;
+        most_sweeps = std::max(most_sweeps, h_ctrl[k].sweeps_run);
+    }
+    if (tr.on)
+        fprintf(stderr, "  epic: (distance transform: %d item(s) in %d group(s), up to %d sweeps, %d strips x %d blocks per item)\n", n, ngroups,
+                most_sweeps, NS, NB);
     tr.mark("border emit (+allocs)");
     if (h_count + 1 >= cap) {
         set_error("sfgpu_epic: label border list overflow (more than 32 sqrt(N ns) + 1M border entries)");
@@ -774,18 +867,19 @@ static int nn_field(sfgpu_ctx *c, const EpicGeo &eg, const float *d_cost, int ns
     // latency of its dependent loads: what counts is how many searches are in flight.  The heap lives in shared memory, so
     // its capacity sets the residency: first a pass with 1024 entries per warp (3 blocks of 8 warps per SM; a search for
     // nn = 100 neighbours on the planar seed graph keeps a few hundred entries open), and only if a heap overflowed the
-    // pass with the full 2048 entries (1 block per SM).
+    // pass with the full 2048 entries (1 block per SM).  An overflow reruns the search of every item.
     const int warps_per_block = 8;
     int blocks_per_sm = 3;
     int blocks = std::min((ns + warps_per_block - 1) / warps_per_block, c->num_sms * blocks_per_sm);
-    // the per-warp tentative-distance arrays: ns floats per resident warp (bounded to 1 GB)
-    while (blocks > 1 && (size_t)blocks * warps_per_block * ns * 4 > ((size_t)1 << 30)) blocks /= 2;
+    // the per-warp tentative-distance arrays: one entry per seed of the largest item per resident warp (bounded to 1 GB)
+    const int nsmax = it.nsmax();
+    while (blocks > 1 && (size_t)blocks * warps_per_block * nsmax * 4 > ((size_t)1 << 30)) blocks /= 2;
     DevBuf done_all, touched, nnf, dis, overflow;
     const size_t nwarps = (size_t)blocks * warps_per_block;
-    if (!done_all.alloc(nwarps * ns * 4) || !touched.alloc(nwarps * KNN_HEAP * 2 * 4) || !nnf.alloc((size_t)ns * nn * 4) || !dis.alloc((size_t)ns * nn * 4) ||
-        !overflow.alloc(4))
+    if (!done_all.alloc(nwarps * nsmax * 4) || !touched.alloc(nwarps * KNN_HEAP * 2 * 4) || !nnf.alloc((size_t)ns * ld * 4) ||
+        !dis.alloc((size_t)ns * ld * 4) || !overflow.alloc(4))
         return SFGPU_ERR_CUDA;
-    k_fill_u32<<<592, 256, 0, st>>>(nwarps * ns, done_all.as<unsigned>(), EPIC_UNSEEN);
+    k_fill_u32<<<592, 256, 0, st>>>(nwarps * nsmax, done_all.as<unsigned>(), EPIC_UNSEEN);
     SF_CUDA(cudaMemsetAsync(overflow.p, 0, 4, st));
     tr.mark("knn allocs + fill");
     SF_CUDA(cudaFuncSetAttribute(k_knn_graph, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((size_t)warps_per_block * KNN_HEAP * sizeof(HeapItem))));
@@ -793,15 +887,16 @@ static int nn_field(sfgpu_ctx *c, const EpicGeo &eg, const float *d_cost, int ns
     for (int heap_cap = KNN_HEAP / 2; heap_cap <= KNN_HEAP; heap_cap *= 2) {
         const size_t smem = (size_t)warps_per_block * heap_cap * sizeof(HeapItem);
         const int nblocks = heap_cap == KNN_HEAP ? std::min(blocks, c->num_sms) : blocks; // (a retry: every entry of done_all is EPIC_UNSEEN again)
-        k_knn_graph<<<nblocks, warps_per_block * 32, smem, st>>>(ns, nn, indptr.as<int>(), indices.as<int>(), uvals.as<float>(), done_all.as<unsigned>(),
-                                                                 touched.as<int>(), nnf.as<int>(), dis.as<float>(), overflow.as<int>(), heap_cap);
+        k_knn_graph<<<nblocks, warps_per_block * 32, smem, st>>>(ns, ld, nsmax, it.d, indptr.as<int>(), indices.as<int>(), uvals.as<float>(),
+                                                                 done_all.as<unsigned>(), touched.as<int>(), nnf.as<int>(), dis.as<float>(), overflow.as<int>(),
+                                                                 heap_cap);
         c->prof_acc.kernel_launches++;
         SF_CUDA(cudaMemcpyAsync(&h_over, overflow.p, 4, cudaMemcpyDeviceToHost, st));
         SF_CUDA(cudaStreamSynchronize(st));
         if (!h_over) break;
         if (heap_cap < KNN_HEAP) SF_CUDA(cudaMemsetAsync(overflow.p, 0, 4, st));
     }
-    k_query_weights<<<ns, 128, 0, st>>>(ns, nn, d_seeds, W, d_labels, d_dmap, nnf.as<int>(), dis.as<float>(), coef, d_qnn, d_qw);
+    k_query_weights<<<ns, 128, 0, st>>>(ns, ld, it.d, d_seeds, W, N, d_labels, d_dmap, nnf.as<int>(), dis.as<float>(), coef, d_qnn, d_qw);
     SF_CUDA(cudaStreamSynchronize(st));
     SF_CUDA(cudaGetLastError());
     c->prof_acc.kernel_launches += 5;
@@ -861,214 +956,292 @@ template <typename F> static int with_arena(sfgpu_ctx *c, size_t first_guess, F 
     return SFGPU_ERR_NOMEM;
 }
 
-static int epic_impl(sfgpu_ctx *c, image_t *flowx, image_t *flowy, const color_image_t *im, const float_image *input_matches, float_image *edges,
-                     const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    if (!c || !flowx || !flowy || !im || !input_matches || !edges || !params || !flowx->data || !flowy->data || !im->c1 ||
-        !input_matches->pixels || !edges->pixels) {
-        set_error("sfgpu_epic: null argument");
-        return SFGPU_ERR_ARG;
-    }
-    const int W = im->width, H = im->height;
-    if (edges->tx != W || edges->ty != H || flowx->width != W || flowx->height != H || flowy->width != W || flowy->height != H ||
-        flowx->stride != ((W + 3) / 4) * 4 || flowy->stride != flowx->stride || im->stride != flowx->stride || input_matches->tx < 4) {
-        set_error("sfgpu_epic: geometry mismatch (edges and flow planes must have the image's size; matches need >= 4 columns)");
-        return SFGPU_ERR_ARG;
-    }
-    const bool la = strcmp(params->method, "LA") == 0, nw = strcmp(params->method, "NW") == 0;
-    if (!la && !nw) {
-        set_error(std::string("sfgpu_epic: method ") + params->method + " not recognized");
-        return SFGPU_ERR_ARG;
-    }
-    SF_CUDA(cudaSetDevice(c->device));
+// names the entry point, and for a batch the item, in error messages
+struct EpicCaller {
+    const char *fn;
+    bool batch;
+    std::string at(int k) const { return batch ? std::string(fn) + ": item " + std::to_string(k) + ": " : std::string(fn) + ": "; }
+};
+
+// epic() on n items of one geometry (the checks of epic_batch have passed, euc is in the edge maps).  Every step runs over all
+// items at once; the host filters and compacts each item's match list in the reference's order.
+static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                     const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
+                     const EpicCaller &who) {
+    const int W = im[0]->width, H = im[0]->height;
+    const bool la = strcmp(params->method, "LA") == 0;
     cudaStream_t st = c->stream;
     EpicTrace trace(st);
-    const Geom g{W, H, flowx->stride};
+    const Geom g{W, H, flowx[0]->stride};
     const size_t N = (size_t)W * H, P = g.plane();
-    sfgpu_epic_stats_t sstat;
-    memset(&sstat, 0, sizeof(sstat));
+    std::vector<sfgpu_epic_stats_t> sstat((size_t)n);
+    memset(sstat.data(), 0, sstat.size() * sizeof(sfgpu_epic_stats_t));
 
     // ---- rectify_corres (epic.cpp:13-27)
-    std::vector<float> m4((size_t)input_matches->ty * 4);
-    int nm = input_matches->ty;
-    for (int i = 0; i < nm; i++) {
-        const float *r = input_matches->pixels + (size_t)i * input_matches->tx;
-        m4[4 * i + 0] = std::max(0.0f, std::min(r[0], (float)(W - 1)));
-        m4[4 * i + 1] = std::max(0.0f, std::min(r[1], (float)(H - 1)));
-        m4[4 * i + 2] = std::max(0.0f, std::min(r[2], (float)(W - 1)));
-        m4[4 * i + 3] = std::max(0.0f, std::min(r[3], (float)(H - 1)));
+    std::vector<std::vector<float>> m4((size_t)n);
+    std::vector<int> nm((size_t)n);
+    for (int k = 0; k < n; k++) {
+        const float_image *in = input_matches[k];
+        nm[k] = in->ty;
+        m4[k].resize((size_t)in->ty * 4);
+        for (int i = 0; i < nm[k]; i++) {
+            const float *r = in->pixels + (size_t)i * in->tx;
+            m4[k][4 * i + 0] = std::max(0.0f, std::min(r[0], (float)(W - 1)));
+            m4[k][4 * i + 1] = std::max(0.0f, std::min(r[1], (float)(H - 1)));
+            m4[k][4 * i + 2] = std::max(0.0f, std::min(r[2], (float)(W - 1)));
+            m4[k][4 * i + 3] = std::max(0.0f, std::min(r[3], (float)(H - 1)));
+        }
+        sstat[k].matches_in = nm[k];
     }
-    sstat.matches_in = nm;
-    // ---- the edge costs (the entry point has already added euc in the caller's array, :155-163) go to the device
+    // ---- the edge costs (the entry point has already added euc in the caller's arrays, :155-163) go to the device
     DevBuf d_cost, d_labels, d_dmap;
-    if (!d_cost.alloc(N * 4) || !d_labels.alloc(N * 4) || !d_dmap.alloc(N * 4)) return SFGPU_ERR_CUDA;
+    if (!d_cost.alloc(n * N * 4) || !d_labels.alloc(n * N * 4) || !d_dmap.alloc(n * N * 4)) return SFGPU_ERR_CUDA;
     {   // (pageable caller arrays go through the multi-threaded staging path, sf_hostcopy.cu: 30+ instead of 11 GB/s)
-        const int rcu = host_copies(c, {{d_cost.p, edges->pixels, N * 4}}, true);
+        std::vector<HostCopy> up;
+        for (int k = 0; k < n; k++) up.push_back({d_cost.as<float>() + k * N, edges[k]->pixels, N * 4});
+        const int rcu = host_copies(c, up, true);
         if (rcu != SFGPU_OK) return rcu;
     }
 
     EpicGeo eg;
     eg.W = W; eg.H = H;
 
-    auto seeds_of = [&](std::vector<int> &seeds, std::vector<float> &vects) { // matches_to_seeds / matches_to_vects (:30-57)
-        seeds.resize((size_t)nm * 2);
-        vects.resize((size_t)nm * 2);
-        for (int i = 0; i < nm; i++) {
-            seeds[2 * i] = (int)m4[4 * i];
-            seeds[2 * i + 1] = (int)m4[4 * i + 1];
-            vects[2 * i] = m4[4 * i + 2] - m4[4 * i];
-            vects[2 * i + 1] = m4[4 * i + 3] - m4[4 * i + 1];
-        }
-    };
-    auto compact = [&](const std::vector<unsigned char> &keep) {
+    auto compact = [&](int k, const unsigned char *keep) {
         int ii = 0;
-        for (int i = 0; i < nm; i++)
+        for (int i = 0; i < nm[k]; i++)
             if (keep[i]) {
-                if (ii != i) memcpy(&m4[4 * (size_t)ii], &m4[4 * (size_t)i], 4 * sizeof(float));
+                if (ii != i) memcpy(&m4[k][4 * (size_t)ii], &m4[k][4 * (size_t)i], 4 * sizeof(float));
                 ii++;
             }
-        nm = ii;
+        nm[k] = ii;
+    };
+    auto all_have_matches = [&]() {
+        for (int k = 0; k < n; k++)
+            if (nm[k] <= 0) {
+                set_error(who.at(k) + "no match survived the filters");
+                return false;
+            }
+        return true;
     };
 
-    // ---- saliency filter (epic.cpp:60-77)
+    // ---- saliency filter (epic.cpp:60-77); an item's 16 work planes follow those of the item before it
     if (params->saliency_th) {
         ArenaScope sal_scope;
         DevBuf work;
-        if (!work.alloc(16 * P * 4)) return SFGPU_ERR_CUDA;
+        const size_t zs = 16 * P;
+        if (!work.alloc(n * zs * 4)) return SFGPU_ERR_CUDA;
         float *d_im = work.as<float>(), *d_tmp = d_im + 3 * P, *d_sm = d_im + 6 * P, *d_ix = d_im + 9 * P, *d_iy = d_im + 12 * P;
         float *d_xx = d_im + 15 * P; // xy, yy reuse d_tmp / d_sm planes below
         {
-            const int rcu = host_copies(c, {{d_im, im->c1, 3 * P * 4}}, true);
+            std::vector<HostCopy> up;
+            for (int k = 0; k < n; k++) up.push_back({d_im + k * zs, im[k]->c1, 3 * P * 4});
+            const int rcu = host_copies(c, up, true);
             if (rcu != SFGPU_OK) return rcu;
         }
         const ConvTaps pre = gaussian_taps(0.8f), post = gaussian_taps(1.0f);
         ConvTaps der;
         memset(&der, 0, sizeof(der));
         der.order = 1; der.c[0] = -0.5f; der.c[1] = 0.0f; der.c[2] = 0.5f; // convolution_new(1, {0, -0.5}, odd)
-        k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_im, d_tmp, pre, 0, 3);
-        k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_tmp, d_sm, pre, 1, 3);
-        k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_sm, d_ix, der, 0, 3);
-        k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_sm, d_iy, der, 1, 3);
+        dim3 grid = grid2(W, H);
+        grid.z = n;
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_im, d_tmp, pre, 0, 3, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_tmp, d_sm, pre, 1, 3, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_ix, der, 0, 3, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_iy, der, 1, 3, zs);
         float *d_xy = d_tmp, *d_yy = d_tmp + P, *d_t = d_tmp + 2 * P, *d_sal = d_sm;
-        k_autocorr<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_ix, d_iy, d_xx, d_xy, d_yy);
+        k_autocorr<<<grid, dim3(32, 8), 0, st>>>(g, d_ix, d_iy, d_xx, d_xy, d_yy, zs);
         float *planes[3] = {d_xx, d_xy, d_yy};
         for (int k = 0; k < 3; k++) {
-            k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, planes[k], d_t, post, 0, 1);
-            k_conv_any<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_t, planes[k], post, 1, 1);
+            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, planes[k], d_t, post, 0, 1, zs);
+            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_t, planes[k], post, 1, 1, zs);
         }
-        k_min_eig<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_xx, d_xy, d_yy, d_sal);
+        k_min_eig<<<grid, dim3(32, 8), 0, st>>>(g, d_xx, d_xy, d_yy, d_sal, zs);
         c->prof_acc.kernel_launches += 12;
-        std::vector<int> pos((size_t)nm * 2);
-        for (int i = 0; i < nm; i++) { // the reference indexes with (int)(y * stride + x) on the float coordinates
-            const int idx = (int)(m4[4 * i + 1] * (float)g.S + m4[4 * i]);
-            pos[2 * i] = idx % g.S;
-            pos[2 * i + 1] = idx / g.S;
-        }
+        std::vector<int> pos;
+        for (int k = 0; k < n; k++)
+            for (int i = 0; i < nm[k]; i++) { // the reference indexes with (int)(y * stride + x) on the float coordinates
+                const int idx = (int)(m4[k][4 * i + 1] * (float)g.S + m4[k][4 * i]);
+                pos.push_back(idx % g.S);
+                pos.push_back(idx / g.S);
+                pos.push_back(k);
+            }
+        const int total = (int)(pos.size() / 3);
         DevBuf d_pos, d_val;
-        if (!d_pos.alloc(pos.size() * 4 + 4) || !d_val.alloc((size_t)nm * 4 + 4)) return SFGPU_ERR_CUDA;
-        std::vector<float> sal((size_t)nm);
-        if (nm > 0) {
+        if (!d_pos.alloc(pos.size() * 4 + 4) || !d_val.alloc((size_t)total * 4 + 4)) return SFGPU_ERR_CUDA;
+        std::vector<float> sal((size_t)total);
+        if (total > 0) {
             SF_CUDA(cudaMemcpyAsync(d_pos.p, pos.data(), pos.size() * 4, cudaMemcpyHostToDevice, st));
-            k_gather_plane<<<(nm + 255) / 256, 256, 0, st>>>(nm, d_pos.as<int>(), g, d_sal, d_val.as<float>());
-            SF_CUDA(cudaMemcpyAsync(sal.data(), d_val.p, (size_t)nm * 4, cudaMemcpyDeviceToHost, st));
+            k_gather_plane<<<(total + 255) / 256, 256, 0, st>>>(total, d_pos.as<int>(), g, d_sal, zs, d_val.as<float>());
+            SF_CUDA(cudaMemcpyAsync(sal.data(), d_val.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
         }
         SF_CUDA(cudaStreamSynchronize(st));
-        std::vector<unsigned char> keep((size_t)nm);
-        for (int i = 0; i < nm; i++) keep[i] = sal[i] >= params->saliency_th;
-        compact(keep);
+        std::vector<unsigned char> keep((size_t)total);
+        for (int i = 0; i < total; i++) keep[i] = sal[i] >= params->saliency_th;
+        for (int k = 0, at = 0; k < n; k++) {
+            const int before = nm[k];
+            compact(k, keep.data() + at);
+            at += before;
+        }
     }
-    sstat.matches_after_saliency = nm;
+    for (int k = 0; k < n; k++) sstat[k].matches_after_saliency = nm[k];
     trace.mark("[rectify + saliency filter]");
+    if (!all_have_matches()) return SFGPU_ERR_ARG;
 
+    // the match lists of all items, concatenated: seed ids are global (EpicItems)
     std::vector<int> seeds;
     std::vector<float> vects;
+    EpicItems items;
     DevBuf d_seeds, d_vects, d_qnn, d_qw, d_est, d_keep;
     const size_t match_mark = g_arena->mark();
-    auto upload_matches = [&](int nn) -> int {
-        seeds_of(seeds, vects);
-        g_arena->release(match_mark); // the buffers of the previous (larger) match list
-        if (!d_seeds.alloc((size_t)nm * 8) || !d_vects.alloc((size_t)nm * 8) || !d_qnn.alloc((size_t)nm * nn * 4) || !d_qw.alloc((size_t)nm * nn * 4) ||
-            !d_est.alloc((size_t)nm * 6 * 4) || !d_keep.alloc((size_t)nm + 4))
-            return SFGPU_ERR_CUDA;
-        if (nm > 0) {
-            SF_CUDA(cudaMemcpyAsync(d_seeds.p, seeds.data(), (size_t)nm * 8, cudaMemcpyHostToDevice, st));
-            SF_CUDA(cudaMemcpyAsync(d_vects.p, vects.data(), (size_t)nm * 8, cudaMemcpyHostToDevice, st));
+    auto upload_matches = [&](int nn) -> int { // nns = min(nn, the item's matches) per item
+        g_arena->release(match_mark); // the buffers of the previous (larger) match lists
+        items.n = n;
+        items.off.assign(1, 0);
+        items.nns.clear();
+        seeds.clear();
+        vects.clear();
+        for (int k = 0; k < n; k++) { // matches_to_seeds / matches_to_vects (:30-57)
+            items.off.push_back(items.off.back() + nm[k]);
+            items.nns.push_back(std::min(nn, nm[k]));
+            for (int i = 0; i < nm[k]; i++) {
+                const float *r = &m4[k][4 * (size_t)i];
+                seeds.push_back((int)r[0]);
+                seeds.push_back((int)r[1]);
+                vects.push_back(r[2] - r[0]);
+                vects.push_back(r[3] - r[1]);
+            }
         }
+        const size_t ns = (size_t)items.ns(), ld = (size_t)items.nnmax();
+        if (!d_seeds.alloc(ns * 8) || !d_vects.alloc(ns * 8) || !d_qnn.alloc(ns * ld * 4) || !d_qw.alloc(ns * ld * 4) || !d_est.alloc(ns * 6 * 4) ||
+            !d_keep.alloc(ns + 4))
+            return SFGPU_ERR_CUDA;
+        const int rcu = items.upload(st);
+        if (rcu != SFGPU_OK) return rcu;
+        SF_CUDA(cudaMemcpyAsync(d_seeds.p, seeds.data(), ns * 8, cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(d_vects.p, vects.data(), ns * 8, cudaMemcpyHostToDevice, st));
         return SFGPU_OK;
     };
+    std::vector<int> sweeps((size_t)n);
 
     // ---- consistency filter (prefiltering, epic.cpp:80-127)
-    if (params->pref_nn && nm > 0) {
-        const int nns = std::min(params->pref_nn + 1, nm);
-        int rc = upload_matches(nns);
+    if (params->pref_nn) {
+        int rc = upload_matches(params->pref_nn + 1);
         if (rc != SFGPU_OK) return rc;
-        rc = nn_field(c, eg, d_cost.as<float>(), nm, nns, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
-                      d_qw.as<float>(), &sstat.sweeps_prefilter);
+        const int ns = items.ns(), ld = items.nnmax();
+        rc = nn_field(c, eg, d_cost.as<float>(), items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
+                      d_qw.as<float>(), sweeps.data());
         if (rc != SFGPU_OK) return rc;
-        k_fit_nw<<<(nm + 127) / 128, 128, 0, st>>>(nm, nns, d_qnn.as<int>(), d_qw.as<float>(), d_vects.as<float>(), d_est.as<float>());
-        k_prefilter_flags<<<(nm + 127) / 128, 128, 0, st>>>(nm, d_est.as<float>(), d_vects.as<float>(), params->pref_th * params->pref_th,
+        for (int k = 0; k < n; k++) sstat[k].sweeps_prefilter = sweeps[k];
+        k_fit_nw<<<(ns + 127) / 128, 128, 0, st>>>(ns, ld, items.d, d_qnn.as<int>(), d_qw.as<float>(), d_vects.as<float>(), d_est.as<float>());
+        k_prefilter_flags<<<(ns + 127) / 128, 128, 0, st>>>(ns, d_est.as<float>(), d_vects.as<float>(), params->pref_th * params->pref_th,
                                                           d_keep.as<unsigned char>());
         c->prof_acc.kernel_launches += 2;
-        std::vector<unsigned char> keep((size_t)nm);
-        SF_CUDA(cudaMemcpyAsync(keep.data(), d_keep.p, (size_t)nm, cudaMemcpyDeviceToHost, st));
+        std::vector<unsigned char> keep((size_t)ns);
+        SF_CUDA(cudaMemcpyAsync(keep.data(), d_keep.p, (size_t)ns, cudaMemcpyDeviceToHost, st));
         SF_CUDA(cudaStreamSynchronize(st));
-        compact(keep);
+        for (int k = 0; k < n; k++) compact(k, keep.data() + items.off[k]);
     }
-    sstat.matches_after_consistency = nm;
+    for (int k = 0; k < n; k++) sstat[k].matches_after_consistency = nm[k];
     trace.mark("[consistency filter total]");
-    if (nm <= 0) {
-        set_error("sfgpu_epic: no match survived the filters");
-        return SFGPU_ERR_ARG;
-    }
+    if (!all_have_matches()) return SFGPU_ERR_ARG;
 
     // ---- interpolation (epic.cpp:184-219)
-    const int nns = std::min(params->nn, nm);
-    int rc = upload_matches(nns);
+    int rc = upload_matches(params->nn);
     if (rc != SFGPU_OK) return rc;
-    rc = nn_field(c, eg, d_cost.as<float>(), nm, nns, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
-                  d_qw.as<float>(), &sstat.sweeps_interpolation);
+    const int ns = items.ns(), ld = items.nnmax();
+    rc = nn_field(c, eg, d_cost.as<float>(), items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
+                  d_qw.as<float>(), sweeps.data());
     if (rc != SFGPU_OK) return rc;
-    DevBuf d_flow;
-    if (!d_flow.alloc(2 * P * 4)) return SFGPU_ERR_CUDA;
-    SF_CUDA(cudaMemsetAsync(d_flow.p, 0, 2 * P * 4, st));
-    if (la) k_fit_la<<<(nm + 127) / 128, 128, 0, st>>>(nm, nns, d_qnn.as<int>(), d_qw.as<float>(), d_seeds.as<int>(), d_vects.as<float>(), d_est.as<float>());
-    else k_fit_nw<<<(nm + 127) / 128, 128, 0, st>>>(nm, nns, d_qnn.as<int>(), d_qw.as<float>(), d_vects.as<float>(), d_est.as<float>());
-    k_apply<<<grid2(W, H), dim3(32, 8), 0, st>>>(g, d_labels.as<int>(), d_est.as<float>(), la ? 1 : 0, d_flow.as<float>(), d_flow.as<float>() + P);
+    for (int k = 0; k < n; k++) sstat[k].sweeps_interpolation = sweeps[k];
+    DevBuf d_flow; // item k: flow x at 2 k P, flow y at (2 k + 1) P
+    if (!d_flow.alloc(n * 2 * P * 4)) return SFGPU_ERR_CUDA;
+    SF_CUDA(cudaMemsetAsync(d_flow.p, 0, n * 2 * P * 4, st));
+    if (la)
+        k_fit_la<<<(ns + 127) / 128, 128, 0, st>>>(ns, ld, items.d, d_qnn.as<int>(), d_qw.as<float>(), d_seeds.as<int>(), d_vects.as<float>(),
+                                                   d_est.as<float>());
+    else k_fit_nw<<<(ns + 127) / 128, 128, 0, st>>>(ns, ld, items.d, d_qnn.as<int>(), d_qw.as<float>(), d_vects.as<float>(), d_est.as<float>());
+    dim3 grid = grid2(W, H);
+    grid.z = n;
+    k_apply<<<grid, dim3(32, 8), 0, st>>>(g, d_labels.as<int>(), d_est.as<float>(), la ? 1 : 0, d_flow.as<float>(), d_flow.as<float>() + P, 2 * P);
     c->prof_acc.kernel_launches += 2;
     trace.mark("[interpolation total]");
-    rc = host_copies(c, {{d_flow.p, flowx->data, P * 4}, {d_flow.as<float>() + P, flowy->data, P * 4}}, false);
+    SF_CUDA(cudaGetLastError());
+    // every check has passed: only now are the caller's flow planes written
+    std::vector<HostCopy> down;
+    for (int k = 0; k < n; k++) {
+        down.push_back({d_flow.as<float>() + 2 * k * P, flowx[k]->data, P * 4});
+        down.push_back({d_flow.as<float>() + (2 * k + 1) * P, flowy[k]->data, P * 4});
+    }
+    rc = host_copies(c, down, false);
     if (rc != SFGPU_OK) return rc;
     SF_CUDA(cudaStreamSynchronize(st));
     trace.mark("[flow download]");
     SF_CUDA(cudaGetLastError());
-    if (stats) *stats = sstat;
+    if (stats)
+        for (int k = 0; k < n; k++) stats[k] = sstat[k];
     return SFGPU_OK;
+}
+
+// the argument checks of epic() on n items, all before anything is touched; then edges += euc in every caller's array, like
+// the reference (epic.cpp:155-163), once whatever the arena does below
+static int epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
+                      const EpicCaller &who) {
+    if (n < 1) {
+        set_error(std::string(who.fn) + ": no item (n < 1)");
+        return SFGPU_ERR_ARG;
+    }
+    if (!c || !flowx || !flowy || !im || !input_matches || !edges || !params) {
+        set_error(std::string(who.fn) + ": null argument");
+        return SFGPU_ERR_ARG;
+    }
+    for (int k = 0; k < n; k++) {
+        if (!flowx[k] || !flowy[k] || !im[k] || !input_matches[k] || !edges[k] || !flowx[k]->data || !flowy[k]->data || !im[k]->c1 ||
+            !input_matches[k]->pixels || !edges[k]->pixels) {
+            set_error(who.at(k) + "null argument");
+            return SFGPU_ERR_ARG;
+        }
+        const int W = im[k]->width, H = im[k]->height;
+        if (edges[k]->tx != W || edges[k]->ty != H || flowx[k]->width != W || flowx[k]->height != H || flowy[k]->width != W || flowy[k]->height != H ||
+            flowx[k]->stride != ((W + 3) / 4) * 4 || flowy[k]->stride != flowx[k]->stride || im[k]->stride != flowx[k]->stride || input_matches[k]->tx < 4) {
+            set_error(who.at(k) + "geometry mismatch (edges and flow planes must have the image's size; matches need >= 4 columns)");
+            return SFGPU_ERR_ARG;
+        }
+        if (W != im[0]->width || H != im[0]->height) {
+            set_error(who.at(k) + "items of different geometry (" + std::to_string(W) + "x" + std::to_string(H) + ", item 0 is " +
+                      std::to_string(im[0]->width) + "x" + std::to_string(im[0]->height) + ")");
+            return SFGPU_ERR_ARG;
+        }
+    }
+    if (strcmp(params->method, "LA") != 0 && strcmp(params->method, "NW") != 0) {
+        set_error(std::string(who.fn) + ": method " + params->method + " not recognized");
+        return SFGPU_ERR_ARG;
+    }
+    SF_CUDA(cudaSetDevice(c->device));
+    const size_t N = (size_t)im[0]->width * im[0]->height;
+    if (params->euc)
+        for (int k = 0; k < n; k++)
+            for (size_t i = 0; i < N; i++) edges[k]->pixels[i] += params->euc;
+    const size_t guess = n * N * 4 * 24 + ((size_t)64 << 20);
+    return with_arena(c, guess, [&]() { return epic_impl(c, n, flowx, flowy, im, input_matches, edges, params, stats, who); });
 }
 
 extern "C" {
 
 int sfgpu_epic(sfgpu_ctx *c, image_t *flowx, image_t *flowy, const color_image_t *im, const float_image *input_matches, float_image *edges,
                const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    if (!c || !im || !edges || !edges->pixels || !params) {
-        set_error("sfgpu_epic: null argument");
-        return SFGPU_ERR_ARG;
-    }
-    SF_CUDA(cudaSetDevice(c->device));
-    const size_t N = (size_t)im->width * im->height;
-    if (edges->tx != im->width || edges->ty != im->height) {
-        set_error("sfgpu_epic: the edge map must have the image's size");
-        return SFGPU_ERR_ARG;
-    }
-    // edges += euc in the caller's array, like the reference (epic.cpp:155-163); once, whatever the arena does below
-    if (params->euc)
-        for (size_t i = 0; i < N; i++) edges->pixels[i] += params->euc;
-    const size_t guess = N * 4 * 24 + ((size_t)64 << 20);
-    return with_arena(c, guess, [&]() { return epic_impl(c, flowx, flowy, im, input_matches, edges, params, stats); });
+    return epic_batch(c, 1, &flowx, &flowy, &im, &input_matches, &edges, params, stats, EpicCaller{"sfgpu_epic", false});
 }
+
+int sfgpu_epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                     const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats) {
+    return epic_batch(c, n, flowx, flowy, im, input_matches, edges, params, stats, EpicCaller{"sfgpu_epic_batch", true});
+}
+
+} // extern "C"
 
 // operator twin of dist_trf_nnfield_subset (epic_aux.cpp:350) with the seeds as query points: labels (W*H), best and dist
 // (ns x nn; dist BEFORE the exp kernel) for operator-level parity tests
-} // extern "C"
-
 static int nnfield_impl(sfgpu_ctx *c, int *best, float *dist, int *labels, const int *seeds, int ns, int nn, const float *cost, int w, int h,
                         int *sweeps) {
     if (!c || !best || !dist || !labels || !seeds || !cost || ns < 1 || nn < 1 || nn > ns || w < 1 || h < 1) {
@@ -1080,14 +1253,20 @@ static int nnfield_impl(sfgpu_ctx *c, int *best, float *dist, int *labels, const
     const size_t N = (size_t)w * h;
     EpicGeo eg;
     eg.W = w; eg.H = h;
+    EpicItems items;
+    items.n = 1;
+    items.off = {0, ns};
+    items.nns = {nn};
     DevBuf d_cost, d_labels, d_dmap, d_seeds, d_qnn, d_qw;
     if (!d_cost.alloc(N * 4) || !d_labels.alloc(N * 4) || !d_dmap.alloc(N * 4) || !d_seeds.alloc((size_t)ns * 8) || !d_qnn.alloc((size_t)ns * nn * 4) ||
         !d_qw.alloc((size_t)ns * nn * 4))
         return SFGPU_ERR_CUDA;
+    int rc = items.upload(st);
+    if (rc != SFGPU_OK) return rc;
     SF_CUDA(cudaMemcpyAsync(d_cost.p, cost, N * 4, cudaMemcpyHostToDevice, st));
     SF_CUDA(cudaMemcpyAsync(d_seeds.p, seeds, (size_t)ns * 8, cudaMemcpyHostToDevice, st));
-    int rc = nn_field(c, eg, d_cost.as<float>(), ns, nn, d_seeds.as<int>(), -1.0f /* raw distances */, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(), d_qw.as<float>(),
-                      sweeps);
+    rc = nn_field(c, eg, d_cost.as<float>(), items, d_seeds.as<int>(), -1.0f /* raw distances */, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
+                  d_qw.as<float>(), sweeps);
     if (rc != SFGPU_OK) return rc;
     SF_CUDA(cudaMemcpyAsync(labels, d_labels.p, N * 4, cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaMemcpyAsync(best, d_qnn.p, (size_t)ns * nn * 4, cudaMemcpyDeviceToHost, st));
@@ -1110,3 +1289,4 @@ int sfgpu_epic_nnfield(sfgpu_ctx *c, int *best, float *dist, int *labels, const 
 }
 
 } // extern "C"
+
