@@ -340,6 +340,29 @@ int sfgpu_epic(sfgpu_ctx *ctx, image_t *flowx, image_t *flowy, const color_image
 int sfgpu_epic_batch(sfgpu_ctx *ctx, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params,
                      sfgpu_epic_stats_t *stats);
+/* replaces rgb_to_lab (image.c:694; callers epicflow.cpp:124, adaptiveFR.cpp:568, slow_flow.cpp:814): the first image of
+ * epic() in Lab with the reference's attenuation of dark and light colours.  dst: same geometry as src (planar, stride =
+ * ceil4(width)).  Whole stride rows are converted, padding columns included, like the reference's loop over stride*height.
+ * Same arithmetic as the reference operation for operation (C's float / double promotions, no FMA); the device's double
+ * pow / exp may, very rarely, round a result one float ulp away from glibc's. */
+int sfgpu_rgb_to_lab(sfgpu_ctx *ctx, color_image_t *dst, const color_image_t *src);
+/* The EpicFlow two-step (epicflow.cpp:124-129, adaptiveFR.cpp:568-574) over n_pairs consecutive pairs of ONE geometry:
+ * pair k = frames[k], frames[k+1] (RGB in [0,255], as variational() takes them).  Pair k's wx[k], wy[k] are, bit for bit,
+ *   lab = rgb_to_lab(frames[k]); sfgpu_epic(wx[k], wy[k], lab, matches[k], edges[k], epic_params, &stats[k]);
+ *   sfgpu_variational(wx[k], wy[k], frames[k], frames[k+1], flow_params);
+ * (the incoming contents of wx, wy are not read).  epic_params is required; flow_params == NULL -> defaults.  euc is added
+ * once to every edges[k] (distinct arrays), like epic().  stats: n_pairs entries or NULL.
+ * Each frame is uploaded once for both steps, the Lab planes are made on the device and the interpolated flows stay there
+ * until they are refined.  Pairs run in chunks of 8 EPIC items; with page-locked memory the next chunk's uploads and the
+ * refined flows' downloads overlap the computation (pageable memory is staged as in sfgpu_variational_sequence).
+ * Errors: every argument check (those of sfgpu_epic_batch and sfgpu_variational) runs first, and a failed check writes no
+ * flow plane and no edge array.  A pair left with no match after the filters is found while running: the chunks before
+ * its chunk are then complete (flows, stats, edges), its chunk and the later pairs' flows are not written, the later
+ * chunks' edges are untouched, and the message names the pair.  A following sfgpu_variational_sequence_u8/u16 cannot use
+ * continue_from_previous. */
+int sfgpu_epicflow_sequence(sfgpu_ctx *ctx, int n_pairs, const color_image_t *const *frames, const float_image *const *matches,
+                            float_image *const *edges, const epic_params_t *epic_params, const variational_params_t *flow_params,
+                            image_t *const *wx, image_t *const *wy, sfgpu_epic_stats_t *stats);
 /* operator twin of dist_trf_nnfield_subset (epic_aux.cpp:350-401) with the seeds as the query points: the label map
  * (w*h), and per seed the nn nearest seeds over the geodesic neighbourhood graph with their distances */
 int sfgpu_epic_nnfield(sfgpu_ctx *ctx, int *best, float *dist, int *labels, const int *seeds, int ns, int nn,

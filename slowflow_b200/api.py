@@ -64,7 +64,7 @@ ABI_SYMBOLS = [
     "sfgpu_host_unregister", "sfgpu_variational_mt", "sfgpu_mt_frame_cache", "sfgpu_normalize", "sfgpu_get_mt_stats", "sfgpu_profile_enable",
     "sfgpu_profile_reset", "sfgpu_profile_get", "sfgpu_image_warp", "sfgpu_warp_frame_derivs", "sfgpu_compute_dpsis_weight",
     "sfgpu_compute_smoothness", "sfgpu_compute_data_and_match", "sfgpu_prep_two_frame", "sfgpu_sub_laplacian", "sfgpu_sor_coupled",
-    "sfgpu_epic", "sfgpu_epic_batch", "sfgpu_epic_nnfield", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
+    "sfgpu_epic", "sfgpu_epic_batch", "sfgpu_epic_nnfield", "sfgpu_rgb_to_lab", "sfgpu_epicflow_sequence", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
     "sfgpu_write_flo", "sfgpu_read_flo_size", "sfgpu_read_flo", "sfgpu_write_occlusion_pbm", "sfgpu_set_device", "sfgpu_get_device",
     "sfgpu_convolve_horiz", "sfgpu_convolve_vert", "sfgpu_color_image_convolve_hv", "sfgpu_get_derivatives",
 ]
@@ -139,6 +139,10 @@ def load_library(path=None):
                                C.POINTER(EpicStats)]
     lib.sfgpu_epic_batch.argtypes = [C.c_void_p, C.c_int, C.POINTER(IP), C.POINTER(IP), C.POINTER(CP), C.POINTER(C.POINTER(FloatImage)),
                                      C.POINTER(C.POINTER(FloatImage)), C.POINTER(EpicParams), C.POINTER(EpicStats)]
+    lib.sfgpu_rgb_to_lab.argtypes = [C.c_void_p, CP, CP]
+    lib.sfgpu_epicflow_sequence.argtypes = [C.c_void_p, C.c_int, C.POINTER(CP), C.POINTER(C.POINTER(FloatImage)),
+                                            C.POINTER(C.POINTER(FloatImage)), C.POINTER(EpicParams), VP, C.POINTER(IP), C.POINTER(IP),
+                                            C.POINTER(EpicStats)]
     lib.sfgpu_epic_nnfield.argtypes = [C.c_void_p, C.POINTER(C.c_int), FP, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int, C.c_int, FP,
                                        C.c_int, C.c_int, C.POINTER(C.c_int)]
     lib.sfgpu_grid_mincut.argtypes = [C.c_int, C.c_int, FP, FP, C.c_float, C.c_int, C.POINTER(C.c_int)]
@@ -292,6 +296,36 @@ class Context:
                                                    (IP * n)(*[C.pointer(f.c) for f in flowsy]), (CP * n)(*[C.pointer(i.c) for i in ims]),
                                                    (FIP * n)(*[C.pointer(m) for m in ms]), (FIP * n)(*[C.pointer(e) for e in es]),
                                                    C.byref(params), st), "sfgpu_epic_batch")
+        return list(st[:n])
+
+    def rgb_to_lab(self, src):
+        """rgb_to_lab (image.c:694) of a ColorImage in [0, 255] -> a new ColorImage (whole stride rows converted)."""
+        dst = ColorImage(src.width, src.height)
+        _check(self.lib, self.lib.sfgpu_rgb_to_lab(self.h, dst.ptr(), src.ptr()), "sfgpu_rgb_to_lab")
+        return dst
+
+    def epicflow_sequence(self, frames, matches, edges, wxs, wys, epic_params=None, flow_params=None):
+        """The EpicFlow two-step over n consecutive pairs of one geometry (sfgpu_epicflow_sequence): pair k writes exactly
+        what ``epic(wxs[k], wys[k], rgb_to_lab(frames[k]), matches[k], edges[k], epic_params)`` followed by
+        ``variational(wxs[k], wys[k], frames[k], frames[k + 1], flow_params)`` would.  frames: n + 1 RGB ColorImages;
+        epic_params.euc is added IN PLACE to every edges[k].  Returns the list of the pairs' EpicStats."""
+        import numpy as np
+        n = len(wxs)
+        assert len(frames) == n + 1 and len(wys) == n and len(matches) == n and len(edges) == n
+        for m, e in zip(matches, edges):
+            assert m.dtype == np.float32 and m.flags.c_contiguous and m.ndim == 2
+            assert e.dtype == np.float32 and e.flags.c_contiguous and e.shape == (frames[0].height, frames[0].width)
+        if epic_params is None:
+            epic_params = epic_params_default()
+        FP, IP, CP, FIP = C.POINTER(C.c_float), C.POINTER(image_t), C.POINTER(color_image_t), C.POINTER(FloatImage)
+        ms = [FloatImage(m.ctypes.data_as(FP), m.shape[1], m.shape[0]) for m in matches]
+        es = [FloatImage(e.ctypes.data_as(FP), e.shape[1], e.shape[0]) for e in edges]
+        st = (EpicStats * max(n, 1))()
+        _check(self.lib, self.lib.sfgpu_epicflow_sequence(
+            self.h, n, (CP * (n + 1))(*[C.pointer(f.c) for f in frames]), (FIP * max(n, 1))(*[C.pointer(m) for m in ms]),
+            (FIP * max(n, 1))(*[C.pointer(e) for e in es]), C.byref(epic_params),
+            C.byref(flow_params) if flow_params is not None else None, (IP * max(n, 1))(*[C.pointer(w.c) for w in wxs]),
+            (IP * max(n, 1))(*[C.pointer(w.c) for w in wys]), st), "sfgpu_epicflow_sequence")
         return list(st[:n])
 
     def epic_nnfield(self, seeds, nn, cost):

@@ -98,10 +98,33 @@ int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d
 // argument check shared by the host-buffer entries: one geometry, stride = ceil4(width), planar contiguous colour
 bool check_pair(const image_t *wx, const image_t *wy, const color_image_t *im1, const color_image_t *im2);
 bool is_pageable(const void *p);
+// the copy streams h2d / d2h and the event rings seq_ev of the sequence pipelines, created at first use (sf_sequence.cu)
+int ensure_seq_events(sfgpu_ctx *c);
 // exact binary Potts min-cut on the device (sf_mincut.cu); results in occ / device_cut_labels(), status after a stream sync
 int device_grid_mincut(sfgpu_ctx *c, DeviceCut *&cut, int W, int H, long long *tr_dev, long long pair_cap, float *occ, int S);
 const int *device_cut_status(const DeviceCut *cut);       // {0 = converged, phases, grid-wide passes}
 const unsigned char *device_cut_labels(const DeviceCut *cut); // dense W*H labels (device memory)
 // one sor_coupled call on the context's SOR arena (profiled)
 int run_sor(sfgpu_ctx *c, int iterations, float omega, int *cur, bool zero_init);
+
+// ---- EPIC interpolation (sf_epic.cu)
+// names the entry point in error messages, and for a batch the item ("item" / "pair" numbered from `first`; null: none)
+struct EpicCaller {
+    const char *fn;
+    const char *item;
+    int first;
+    std::string at(int k) const;
+};
+// the argument checks of sfgpu_epic_batch on n items: null pointers, one geometry, stride = ceil4(width), >= 4 match
+// columns, the method.  Touches nothing.
+int epic_check_args(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const EpicCaller &who);
+// edges[k] += euc in the caller's arrays (epic.cpp:155-163)
+void epic_add_euc(int n, float_image *const *edges, float euc);
+// epic() on n items of one geometry on device planes, after epic_check_args and epic_add_euc.  d_cost: the items' W x H
+// edge costs one after another; d_lab: their Lab images, 3 planes of g each (read by the saliency filter only; may be null
+// when it is off); d_flow: item k's flow x at 2 k P and flow y at (2 k + 1) P, whole planes with zeroed padding.  stats: n
+// entries.  The last kernels are left queued on the context's stream; on an error d_flow is not fully written.
+int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d_lab, const float_image *const *input_matches,
+                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const EpicCaller &who);
 } // namespace sf

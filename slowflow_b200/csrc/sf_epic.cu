@@ -46,13 +46,13 @@ constexpr unsigned EPIC_UNSEEN = 0x7F7F7F7Fu; // memset(…, 0x7F, …) pattern 
 // ------------------------------------------------------------------------------------------ saliency (image.c:728-790)
 struct ConvTaps { int order; float c[17]; }; // c[order + k] = weight of src[i + k]
 // The image-sized kernels of a call cover all its items at once: blockIdx.z is the item, and the item's planes lie zs floats
-// after those of the item before it.
+// after those of the item before it (k_conv_any: src_zs in its source, which may be another buffer).
 __global__ void __launch_bounds__(256) k_conv_any(Geom g, const float *__restrict__ src, float *__restrict__ dst, ConvTaps t, int vertical,
-                                                  int planes, size_t zs) {
+                                                  int planes, size_t zs, size_t src_zs) {
     const int i = blockIdx.x * 32 + threadIdx.x, j = blockIdx.y * 8 + threadIdx.y;
     if (i >= g.W || j >= g.H) return;
     const size_t P = g.plane();
-    src += blockIdx.z * zs;
+    src += blockIdx.z * src_zs;
     dst += blockIdx.z * zs;
     for (int c = 0; c < planes; c++) {
         const float *s = src + c * P;
@@ -956,26 +956,19 @@ template <typename F> static int with_arena(sfgpu_ctx *c, size_t first_guess, F 
     return SFGPU_ERR_NOMEM;
 }
 
-// names the entry point, and for a batch the item, in error messages
-struct EpicCaller {
-    const char *fn;
-    bool batch;
-    std::string at(int k) const { return batch ? std::string(fn) + ": item " + std::to_string(k) + ": " : std::string(fn) + ": "; }
-};
-
-// epic() on n items of one geometry (the checks of epic_batch have passed, euc is in the edge maps).  Every step runs over all
-// items at once; the host filters and compacts each item's match list in the reference's order.
-static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
-                     const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
-                     const EpicCaller &who) {
-    const int W = im[0]->width, H = im[0]->height;
+// epic() on n items of one geometry on device planes (the checks of epic_check_args have passed, euc is in the edge costs).
+// Every step runs over all items at once; the host filters and compacts each item's match list in the reference's order.
+// d_cost: the items' W x H edge costs one after another; d_lab: their Lab images, 3 planes of g each (only the saliency
+// filter reads them; null when it is off); d_flow: item k's flow x at 2 k P, flow y at (2 k + 1) P, written whole (padding
+// zeroed).  Runs with the arena installed; the flow kernels are left queued on the context's stream.  sstat: n entries.
+static int epic_core(sfgpu_ctx *c, int n, Geom g, const float *d_cost_in, const float *d_lab, const float_image *const *input_matches,
+                     const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *sstat, const EpicCaller &who) {
+    const int W = g.W, H = g.H;
     const bool la = strcmp(params->method, "LA") == 0;
     cudaStream_t st = c->stream;
     EpicTrace trace(st);
-    const Geom g{W, H, flowx[0]->stride};
     const size_t N = (size_t)W * H, P = g.plane();
-    std::vector<sfgpu_epic_stats_t> sstat((size_t)n);
-    memset(sstat.data(), 0, sstat.size() * sizeof(sfgpu_epic_stats_t));
+    memset(sstat, 0, (size_t)n * sizeof(sfgpu_epic_stats_t));
 
     // ---- rectify_corres (epic.cpp:13-27)
     std::vector<std::vector<float>> m4((size_t)n);
@@ -993,15 +986,8 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
         }
         sstat[k].matches_in = nm[k];
     }
-    // ---- the edge costs (the entry point has already added euc in the caller's arrays, :155-163) go to the device
-    DevBuf d_cost, d_labels, d_dmap;
-    if (!d_cost.alloc(n * N * 4) || !d_labels.alloc(n * N * 4) || !d_dmap.alloc(n * N * 4)) return SFGPU_ERR_CUDA;
-    {   // (pageable caller arrays go through the multi-threaded staging path, sf_hostcopy.cu: 30+ instead of 11 GB/s)
-        std::vector<HostCopy> up;
-        for (int k = 0; k < n; k++) up.push_back({d_cost.as<float>() + k * N, edges[k]->pixels, N * 4});
-        const int rcu = host_copies(c, up, true);
-        if (rcu != SFGPU_OK) return rcu;
-    }
+    DevBuf d_labels, d_dmap;
+    if (!d_labels.alloc(n * N * 4) || !d_dmap.alloc(n * N * 4)) return SFGPU_ERR_CUDA;
 
     EpicGeo eg;
     eg.W = W; eg.H = H;
@@ -1024,36 +1010,30 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
         return true;
     };
 
-    // ---- saliency filter (epic.cpp:60-77); an item's 16 work planes follow those of the item before it
+    // ---- saliency filter (epic.cpp:60-77) on the Lab planes; an item's 13 work planes follow those of the item before it
     if (params->saliency_th) {
         ArenaScope sal_scope;
         DevBuf work;
-        const size_t zs = 16 * P;
+        const size_t zs = 13 * P;
         if (!work.alloc(n * zs * 4)) return SFGPU_ERR_CUDA;
-        float *d_im = work.as<float>(), *d_tmp = d_im + 3 * P, *d_sm = d_im + 6 * P, *d_ix = d_im + 9 * P, *d_iy = d_im + 12 * P;
-        float *d_xx = d_im + 15 * P; // xy, yy reuse d_tmp / d_sm planes below
-        {
-            std::vector<HostCopy> up;
-            for (int k = 0; k < n; k++) up.push_back({d_im + k * zs, im[k]->c1, 3 * P * 4});
-            const int rcu = host_copies(c, up, true);
-            if (rcu != SFGPU_OK) return rcu;
-        }
+        float *d_tmp = work.as<float>(), *d_sm = d_tmp + 3 * P, *d_ix = d_tmp + 6 * P, *d_iy = d_tmp + 9 * P;
+        float *d_xx = d_tmp + 12 * P; // xy, yy reuse d_tmp / d_sm planes below
         const ConvTaps pre = gaussian_taps(0.8f), post = gaussian_taps(1.0f);
         ConvTaps der;
         memset(&der, 0, sizeof(der));
         der.order = 1; der.c[0] = -0.5f; der.c[1] = 0.0f; der.c[2] = 0.5f; // convolution_new(1, {0, -0.5}, odd)
         dim3 grid = grid2(W, H);
         grid.z = n;
-        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_im, d_tmp, pre, 0, 3, zs);
-        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_tmp, d_sm, pre, 1, 3, zs);
-        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_ix, der, 0, 3, zs);
-        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_iy, der, 1, 3, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_lab, d_tmp, pre, 0, 3, zs, 3 * P);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_tmp, d_sm, pre, 1, 3, zs, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_ix, der, 0, 3, zs, zs);
+        k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_sm, d_iy, der, 1, 3, zs, zs);
         float *d_xy = d_tmp, *d_yy = d_tmp + P, *d_t = d_tmp + 2 * P, *d_sal = d_sm;
         k_autocorr<<<grid, dim3(32, 8), 0, st>>>(g, d_ix, d_iy, d_xx, d_xy, d_yy, zs);
         float *planes[3] = {d_xx, d_xy, d_yy};
         for (int k = 0; k < 3; k++) {
-            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, planes[k], d_t, post, 0, 1, zs);
-            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_t, planes[k], post, 1, 1, zs);
+            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, planes[k], d_t, post, 0, 1, zs, zs);
+            k_conv_any<<<grid, dim3(32, 8), 0, st>>>(g, d_t, planes[k], post, 1, 1, zs, zs);
         }
         k_min_eig<<<grid, dim3(32, 8), 0, st>>>(g, d_xx, d_xy, d_yy, d_sal, zs);
         c->prof_acc.kernel_launches += 12;
@@ -1128,7 +1108,7 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
         int rc = upload_matches(params->pref_nn + 1);
         if (rc != SFGPU_OK) return rc;
         const int ns = items.ns(), ld = items.nnmax();
-        rc = nn_field(c, eg, d_cost.as<float>(), items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
+        rc = nn_field(c, eg, d_cost_in, items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
                       d_qw.as<float>(), sweeps.data());
         if (rc != SFGPU_OK) return rc;
         for (int k = 0; k < n; k++) sstat[k].sweeps_prefilter = sweeps[k];
@@ -1149,23 +1129,45 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
     int rc = upload_matches(params->nn);
     if (rc != SFGPU_OK) return rc;
     const int ns = items.ns(), ld = items.nnmax();
-    rc = nn_field(c, eg, d_cost.as<float>(), items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
+    rc = nn_field(c, eg, d_cost_in, items, d_seeds.as<int>(), params->coef_kernel, d_labels.as<int>(), d_dmap.as<float>(), d_qnn.as<int>(),
                   d_qw.as<float>(), sweeps.data());
     if (rc != SFGPU_OK) return rc;
     for (int k = 0; k < n; k++) sstat[k].sweeps_interpolation = sweeps[k];
-    DevBuf d_flow; // item k: flow x at 2 k P, flow y at (2 k + 1) P
-    if (!d_flow.alloc(n * 2 * P * 4)) return SFGPU_ERR_CUDA;
-    SF_CUDA(cudaMemsetAsync(d_flow.p, 0, n * 2 * P * 4, st));
+    SF_CUDA(cudaMemsetAsync(d_flow, 0, n * 2 * P * 4, st));
     if (la)
         k_fit_la<<<(ns + 127) / 128, 128, 0, st>>>(ns, ld, items.d, d_qnn.as<int>(), d_qw.as<float>(), d_seeds.as<int>(), d_vects.as<float>(),
                                                    d_est.as<float>());
     else k_fit_nw<<<(ns + 127) / 128, 128, 0, st>>>(ns, ld, items.d, d_qnn.as<int>(), d_qw.as<float>(), d_vects.as<float>(), d_est.as<float>());
     dim3 grid = grid2(W, H);
     grid.z = n;
-    k_apply<<<grid, dim3(32, 8), 0, st>>>(g, d_labels.as<int>(), d_est.as<float>(), la ? 1 : 0, d_flow.as<float>(), d_flow.as<float>() + P, 2 * P);
+    k_apply<<<grid, dim3(32, 8), 0, st>>>(g, d_labels.as<int>(), d_est.as<float>(), la ? 1 : 0, d_flow, d_flow + P, 2 * P);
     c->prof_acc.kernel_launches += 2;
     trace.mark("[interpolation total]");
     SF_CUDA(cudaGetLastError());
+    return SFGPU_OK;
+}
+
+// sfgpu_epic / sfgpu_epic_batch: the caller's edge costs and Lab images go up, the flows come down
+static int epic_host(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                     const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
+                     const EpicCaller &who) {
+    const Geom g{im[0]->width, im[0]->height, flowx[0]->stride};
+    const size_t N = (size_t)g.W * g.H, P = g.plane();
+    const bool sal = params->saliency_th != 0;
+    DevBuf d_cost, d_lab, d_flow;
+    if (!d_cost.alloc(n * N * 4) || !d_flow.alloc(n * 2 * P * 4) || (sal && !d_lab.alloc(n * 3 * P * 4))) return SFGPU_ERR_CUDA;
+    {   // (pageable caller arrays go through the multi-threaded staging path, sf_hostcopy.cu: 30+ instead of 11 GB/s)
+        std::vector<HostCopy> up;
+        for (int k = 0; k < n; k++) up.push_back({d_cost.as<float>() + k * N, edges[k]->pixels, N * 4});
+        if (sal)
+            for (int k = 0; k < n; k++) up.push_back({d_lab.as<float>() + k * 3 * P, im[k]->c1, 3 * P * 4});
+        const int rcu = host_copies(c, up, true);
+        if (rcu != SFGPU_OK) return rcu;
+    }
+    std::vector<sfgpu_epic_stats_t> sstat((size_t)n);
+    int rc = epic_core(c, n, g, d_cost.as<float>(), sal ? d_lab.as<float>() : nullptr, input_matches, params, d_flow.as<float>(), sstat.data(), who);
+    if (rc != SFGPU_OK) return rc;
+    EpicTrace trace(c->stream);
     // every check has passed: only now are the caller's flow planes written
     std::vector<HostCopy> down;
     for (int k = 0; k < n; k++) {
@@ -1174,7 +1176,7 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
     }
     rc = host_copies(c, down, false);
     if (rc != SFGPU_OK) return rc;
-    SF_CUDA(cudaStreamSynchronize(st));
+    SF_CUDA(cudaStreamSynchronize(c->stream));
     trace.mark("[flow download]");
     SF_CUDA(cudaGetLastError());
     if (stats)
@@ -1182,11 +1184,14 @@ static int epic_impl(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
     return SFGPU_OK;
 }
 
-// the argument checks of epic() on n items, all before anything is touched; then edges += euc in every caller's array, like
-// the reference (epic.cpp:155-163), once whatever the arena does below
-static int epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
-                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
-                      const EpicCaller &who) {
+namespace sf {
+
+std::string EpicCaller::at(int k) const {
+    return item ? std::string(fn) + ": " + item + " " + std::to_string(first + k) + ": " : std::string(fn) + ": ";
+}
+
+int epic_check_args(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const EpicCaller &who) {
     if (n < 1) {
         set_error(std::string(who.fn) + ": no item (n < 1)");
         return SFGPU_ERR_ARG;
@@ -1217,25 +1222,50 @@ static int epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const
         set_error(std::string(who.fn) + ": method " + params->method + " not recognized");
         return SFGPU_ERR_ARG;
     }
+    return SFGPU_OK;
+}
+
+void epic_add_euc(int n, float_image *const *edges, float euc) {
+    if (!euc) return;
+    for (int k = 0; k < n; k++) {
+        const size_t N = (size_t)edges[k]->tx * edges[k]->ty;
+        for (size_t i = 0; i < N; i++) edges[k]->pixels[i] += euc;
+    }
+}
+
+size_t epic_arena_guess(int n, size_t N) { return n * N * 4 * 24 + ((size_t)64 << 20); }
+
+int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d_lab, const float_image *const *input_matches,
+                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const EpicCaller &who) {
+    return with_arena(c, epic_arena_guess(n, (size_t)g.W * g.H),
+                      [&]() { return epic_core(c, n, g, d_cost, d_lab, input_matches, params, d_flow, stats, who); });
+}
+
+} // namespace sf
+
+// the argument checks of epic() on n items, all before anything is touched; then edges += euc in every caller's array, like
+// the reference (epic.cpp:155-163), once whatever the arena does below
+static int epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
+                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
+                      const EpicCaller &who) {
+    const int rc = epic_check_args(c, n, flowx, flowy, im, input_matches, edges, params, who);
+    if (rc != SFGPU_OK) return rc;
     SF_CUDA(cudaSetDevice(c->device));
-    const size_t N = (size_t)im[0]->width * im[0]->height;
-    if (params->euc)
-        for (int k = 0; k < n; k++)
-            for (size_t i = 0; i < N; i++) edges[k]->pixels[i] += params->euc;
-    const size_t guess = n * N * 4 * 24 + ((size_t)64 << 20);
-    return with_arena(c, guess, [&]() { return epic_impl(c, n, flowx, flowy, im, input_matches, edges, params, stats, who); });
+    epic_add_euc(n, edges, params->euc);
+    return with_arena(c, epic_arena_guess(n, (size_t)im[0]->width * im[0]->height),
+                      [&]() { return epic_host(c, n, flowx, flowy, im, input_matches, edges, params, stats, who); });
 }
 
 extern "C" {
 
 int sfgpu_epic(sfgpu_ctx *c, image_t *flowx, image_t *flowy, const color_image_t *im, const float_image *input_matches, float_image *edges,
                const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    return epic_batch(c, 1, &flowx, &flowy, &im, &input_matches, &edges, params, stats, EpicCaller{"sfgpu_epic", false});
+    return epic_batch(c, 1, &flowx, &flowy, &im, &input_matches, &edges, params, stats, EpicCaller{"sfgpu_epic", nullptr, 0});
 }
 
 int sfgpu_epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    return epic_batch(c, n, flowx, flowy, im, input_matches, edges, params, stats, EpicCaller{"sfgpu_epic_batch", true});
+    return epic_batch(c, n, flowx, flowy, im, input_matches, edges, params, stats, EpicCaller{"sfgpu_epic_batch", "item", 0});
 }
 
 } // extern "C"

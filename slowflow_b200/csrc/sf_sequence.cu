@@ -52,7 +52,7 @@ struct SeqFrames { // where the frames of a call come from
     const void *host(int f) const { return ints ? ints[f].data : (const void *)f32[f]->c1; }
 };
 
-static int ensure_seq_events(sfgpu_ctx *c) {
+int ensure_seq_events(sfgpu_ctx *c) {
     for (auto &ring : c->seq_ev)
         for (auto &e : ring)
             if (!e) SF_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
