@@ -369,7 +369,7 @@ void sfgpu_destroy(sfgpu_ctx *c) {
     if (c->ws) cudaFree(c->ws);
     sf::sor_plan_release(c->sor);
     if (c->io) cudaFree(c->io);
-    for (auto &ring : c->seq_ev)
+    for (auto &ring : c->copy_ev)
         for (auto e : ring)
             if (e) cudaEventDestroy(e);
     if (c->seq_raw) cudaFree(c->seq_raw);

@@ -47,9 +47,9 @@ struct sfgpu_ctx {
     float *io = nullptr; // im1(3) im2(3) wx wy   [+ ring for the sequence API]
     size_t io_floats = 0;
 
-    // ---- sequence pipeline (sf_sequence.cu)
+    // ---- copy pipeline (CopyPipeline, sf_hostcopy.cu; created at first use) and sequence frames (sf_sequence.cu)
     cudaStream_t h2d = nullptr, d2h = nullptr;
-    cudaEvent_t seq_ev[3][4] = {}; // rings of "uploaded" / "solved" / "downloaded" events, created at first use
+    cudaEvent_t copy_ev[3][4] = {}; // rings of "uploaded" / "compute passed" / "drained" events
     unsigned char *seq_raw = nullptr; // 3 slots of packed 8-/16-bit frames awaiting their on-device conversion
     size_t seq_raw_bytes = 0;        // bytes per slot
     sf::Geom seq_geom{0, 0, 0};      // geometry of the frame ring left by the last sequence call
@@ -92,14 +92,33 @@ struct sfgpu_ctx {
 namespace sf {
 // copies between caller (host) buffers and the device for one call, one direction (sf_hostcopy.cu)
 int host_copies(sfgpu_ctx *c, const std::vector<HostCopy> &list, bool h2d);
+// The copies of a call that streams caller memory stage by stage (0, 1, 2, ...: pairs, chunks) while the compute stream
+// works (sf_hostcopy.cu).  start() decides once: if any caller buffer is pageable, every copy is a host_copies() on the
+// compute stream in program order and the ordering calls do nothing.  Otherwise uploads and downloads run on their own
+// streams, ordered by rings of 4 events per kind (stage & 3), so a stage waited for must be one of the last 4 of its kind.
+// A stage argument < 0 means no wait.
+class CopyPipeline {
+  public:
+    explicit CopyPipeline(sfgpu_ctx *c) : c(c) {}
+    // buffers: every caller buffer of the call.  The first upload comes after the work already on the compute stream.
+    int start(const std::vector<const void *> &buffers);
+    // stage k's uploads, after compute has passed stage `passed` and stage `drained`'s downloads have finished
+    int upload(int k, const std::vector<HostCopy> &list, int passed = -1, int drained = -1);
+    int wait(int uploaded, int drained = -1); // the compute stream waits for these stages' uploads / downloads
+    int pass(int k);                          // compute has passed stage k with the work queued so far
+    // stage k's downloads, after compute has passed it (the last pass(k)); may be called several times per stage
+    int download(int k, const std::vector<HostCopy> &list);
+    int finish(int status); // drains all three streams; returns `status` if it is an error, else the first error met
+
+  private:
+    sfgpu_ctx *c;
+    bool pageable = false;
+};
 // two-frame refinement on device planes (variational.c:19-82 + :101-143)
 int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d_im1, const float *d_im2,
                   const variational_params_t *params);
 // argument check shared by the host-buffer entries: one geometry, stride = ceil4(width), planar contiguous colour
 bool check_pair(const image_t *wx, const image_t *wy, const color_image_t *im1, const color_image_t *im2);
-bool is_pageable(const void *p);
-// the copy streams h2d / d2h and the event rings seq_ev of the sequence pipelines, created at first use (sf_sequence.cu)
-int ensure_seq_events(sfgpu_ctx *c);
 // exact binary Potts min-cut on the device (sf_mincut.cu); results in occ / device_cut_labels(), status after a stream sync
 int device_grid_mincut(sfgpu_ctx *c, DeviceCut *&cut, int W, int H, long long *tr_dev, long long pair_cap, float *occ, int S);
 const int *device_cut_status(const DeviceCut *cut);       // {0 = converged, phases, grid-wide passes}

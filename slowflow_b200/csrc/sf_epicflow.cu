@@ -55,9 +55,10 @@ static bool planar(const color_image_t *im) {
 constexpr int EF_CHUNK = 8;
 
 // The argument checks have passed.  Pair j of chunk q = j / EF_CHUNK.  Per chunk, on the one compute stream: the Lab planes
-// of its first frames, the EPIC batch into the chunk's flow buffer, then run_two_frame on each pair in place.  With
-// page-locked caller memory the next chunk's frames and edge costs go up on h2d while this chunk's pairs are refined, and
-// each refined pair goes down on d2h while the next one computes.  Device layout (the context's io area):
+// of its first frames, the EPIC batch into the chunk's flow buffer, then run_two_frame on each pair in place.  The copies
+// go through CopyPipeline (sf_hostcopy.cu), one stage per chunk: with page-locked caller memory the next chunk's frames
+// and edge costs go up while this chunk's pairs are refined, and each refined pair goes down while the next one computes.
+// Device layout (the context's io area):
 //   frame ring: 2 * EF_CHUNK + 2 frames, frame f in slot f % R, so the frames of two consecutive chunks never share a slot
 //   Lab planes of one chunk | flows of two chunks (by chunk parity) | edge costs of two chunks (by chunk parity)
 static int run_epicflow(sfgpu_ctx *c, int n_pairs, const color_image_t *const *frames, const float_image *const *matches,
@@ -69,58 +70,34 @@ static int run_epicflow(sfgpu_ctx *c, int n_pairs, const color_image_t *const *f
     const bool sal = ep->saliency_th != 0;
     int rc = c->ensure_io((size_t)R * 3 * P + (size_t)CH * 3 * P + 2 * (size_t)CH * 2 * P + 2 * (size_t)CH * N); // (also ends a _u8/_u16 sequence)
     if (rc != SFGPU_OK) return rc;
-    rc = ensure_seq_events(c);
-    if (rc != SFGPU_OK) return rc;
     float *ring = c->io, *lab = ring + (size_t)R * 3 * P, *flow0 = lab + (size_t)CH * 3 * P, *cost0 = flow0 + 2 * (size_t)CH * 2 * P;
     auto frame = [&](int f) { return ring + (size_t)(f % R) * 3 * P; };
     auto flows = [&](int q) { return flow0 + (size_t)(q & 1) * CH * 2 * P; };
     auto costs = [&](int q) { return cost0 + (size_t)(q & 1) * CH * N; };
     auto count = [&](int q) { return std::min(CH, n_pairs - q * CH); };
-    cudaEvent_t ev_up = c->seq_ev[0][0], ev_chunk = c->seq_ev[1][0], ev_pair = c->seq_ev[1][1], ev_start = c->seq_ev[1][2];
-    cudaEvent_t ev_down[2] = {c->seq_ev[2][0], c->seq_ev[2][1]};
 
-    // pageable caller memory takes the staged copies of sf_hostcopy.cu on the compute stream, without overlap
-    bool pageable = false;
-    for (int f = 0; f <= n_pairs && !pageable; f++) pageable = is_pageable(frames[f]->c1);
-    for (int j = 0; j < n_pairs && !pageable; j++)
-        pageable = is_pageable(wx[j]->data) || is_pageable(wy[j]->data) || is_pageable(edges[j]->pixels);
-
-    // chunk q's inputs: its frames (frame q * CH is already resident for q > 0) and its edge costs after += euc
+    CopyPipeline pipe(c); // stage q = chunk q
+    // chunk q's inputs: its frames (frame q * CH is already resident for q > 0) and its edge costs after += euc.  The frame
+    // slots and the cost parity it fills were last read by chunk q - 2.
     auto upload = [&](int q) -> int {
         const int j0 = q * CH, m = count(q);
         epic_add_euc(m, edges + j0, ep->euc);
         std::vector<HostCopy> up;
         for (int f = q == 0 ? 0 : j0 + 1; f <= j0 + m; f++) up.push_back({frame(f), frames[f]->c1, 3 * P * sizeof(float)});
         for (int k = 0; k < m; k++) up.push_back({costs(q) + k * N, edges[j0 + k]->pixels, N * sizeof(float)});
-        if (pageable) return host_copies(c, up, true);
-        // the slots it fills were last read by chunk q - 2, which ended before the last record of ev_chunk
-        if (q >= 2) SF_CUDA(cudaStreamWaitEvent(c->h2d, ev_chunk, 0));
-        for (const HostCopy &hc : up) SF_CUDA(cudaMemcpyAsync(hc.dev, hc.host, hc.bytes, cudaMemcpyHostToDevice, c->h2d));
-        SF_CUDA(cudaEventRecord(ev_up, c->h2d));
-        return SFGPU_OK;
-    };
-    auto download = [&](int j, const float *d_fx) -> int {
-        if (pageable) return host_copies(c, {{const_cast<float *>(d_fx), wx[j]->data, P * sizeof(float)}, {const_cast<float *>(d_fx + P), wy[j]->data, P * sizeof(float)}}, false);
-        SF_CUDA(cudaEventRecord(ev_pair, c->stream));
-        SF_CUDA(cudaStreamWaitEvent(c->d2h, ev_pair, 0));
-        SF_CUDA(cudaMemcpyAsync(wx[j]->data, d_fx, P * sizeof(float), cudaMemcpyDeviceToHost, c->d2h));
-        SF_CUDA(cudaMemcpyAsync(wy[j]->data, d_fx + P, P * sizeof(float), cudaMemcpyDeviceToHost, c->d2h));
-        return SFGPU_OK;
+        return pipe.upload(q, up, q - 2);
     };
 
-    // earlier work on the compute stream may still read the io area
-    int status = SFGPU_OK;
-    if (!cuda_ok(cudaEventRecord(ev_start, c->stream), "record") || !cuda_ok(cudaStreamWaitEvent(c->h2d, ev_start, 0), "wait"))
-        status = SFGPU_ERR_CUDA;
+    std::vector<const void *> buffers;
+    for (int f = 0; f <= n_pairs; f++) buffers.push_back(frames[f]->c1);
+    for (int j = 0; j < n_pairs; j++) buffers.insert(buffers.end(), {wx[j]->data, wy[j]->data, edges[j]->pixels});
+    int status = pipe.start(buffers);
     if (status == SFGPU_OK) status = upload(0);
     std::vector<sfgpu_epic_stats_t> st((size_t)CH);
     for (int q = 0; q < n_chunks && status == SFGPU_OK; q++) {
         const int j0 = q * CH, m = count(q);
-        if (!pageable) {
-            if (!cuda_ok(cudaStreamWaitEvent(c->stream, ev_up, 0), "wait up")) { status = SFGPU_ERR_CUDA; break; }
-            // the flow buffer of this parity was last drained by chunk q - 2's downloads
-            if (q >= 2 && !cuda_ok(cudaStreamWaitEvent(c->stream, ev_down[q & 1], 0), "wait down")) { status = SFGPU_ERR_CUDA; break; }
-        }
+        // the flow buffer of this parity was last drained by chunk q - 2's downloads
+        if ((status = pipe.wait(q, q - 2)) != SFGPU_OK) break;
         if (sal)
             for (int k = 0; k < m; k++) launch_rgb_to_lab(c, P, frame(j0 + k), lab + (size_t)k * 3 * P);
         status = epic_device(c, m, g, costs(q), sal ? lab : nullptr, matches + j0, ep, flows(q), st.data(), EpicCaller{"sfgpu_epicflow_sequence", "pair", j0});
@@ -131,16 +108,11 @@ static int run_epicflow(sfgpu_ctx *c, int n_pairs, const color_image_t *const *f
         for (int k = 0; k < m && status == SFGPU_OK; k++) {
             float *fx = flows(q) + (size_t)k * 2 * P;
             status = run_two_frame(c, g, fx, fx + P, frame(j0 + k), frame(j0 + k + 1), vp);
-            if (status == SFGPU_OK) status = download(j0 + k, fx);
+            if (status == SFGPU_OK) status = pipe.pass(q); // re-marked per pair: the last mark ends chunk q
+            if (status == SFGPU_OK) status = pipe.download(q, {{fx, wx[j0 + k]->data, P * sizeof(float)}, {fx + P, wy[j0 + k]->data, P * sizeof(float)}});
         }
-        if (status != SFGPU_OK) break;
-        if (!pageable && (!cuda_ok(cudaEventRecord(ev_chunk, c->stream), "record chunk") || !cuda_ok(cudaEventRecord(ev_down[q & 1], c->d2h), "record down")))
-            status = SFGPU_ERR_CUDA;
     }
-    cudaStreamSynchronize(c->h2d);
-    cudaStreamSynchronize(c->stream);
-    if (!cuda_ok(cudaStreamSynchronize(c->d2h), "sync d2h") && status == SFGPU_OK) status = SFGPU_ERR_CUDA;
-    return status;
+    return pipe.finish(status);
 }
 
 } // namespace sf

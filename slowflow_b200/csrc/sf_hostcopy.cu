@@ -1,12 +1,16 @@
-// sf_hostcopy.cu -- transfers between ORDINARY (pageable) caller memory and the device for the drop-in entry points.
+// sf_hostcopy.cu -- transfers between caller memory and the device for the host-buffer entry points.
 //
 // The reference allocates its images with plain malloc (image.c:17-33), so an unmodified call site hands the library
 // pageable buffers.  cudaMemcpyAsync stages those through the driver's own bounce buffer on ONE host thread: ~11 GB/s
 // measured, i.e. 10 ms for the 117 MB of a 2560x1440 pair against 2.5 ms of GPU work.  Here large pageable copies are
 // cut into chunks that a few short-lived host threads copy into page-locked slots of the context and hand to the DMA
-// engine on their own streams; page-locked or registered caller memory takes the direct path.
+// engine on their own streams; page-locked or registered caller memory takes the direct path (host_copies).
+//
+// CopyPipeline moves the caller memory of the calls that stream many stages (sf_sequence.cu, sf_epicflow.cu): with
+// page-locked memory, uploads run on an h2d stream and downloads on a d2h stream while the compute stream works.
 #include <string.h>
 
+#include <algorithm>
 #include <thread>
 #include <vector>
 
@@ -61,7 +65,7 @@ struct HostStager {
 
 void host_stager_free(HostStager *h) { delete h; }
 
-bool is_pageable(const void *p) {
+static bool is_pageable(const void *p) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
         cudaGetLastError();
@@ -150,21 +154,73 @@ static int staged_batch(sfgpu_ctx *c, const std::vector<HostCopy> &list, bool h2
 // Copies of one call in one direction.  Pageable buffers of at least 2 chunks go through the staged path (together, so
 // that the worker threads are spawned once); everything else is a plain cudaMemcpyAsync on the context's stream.
 int host_copies(sfgpu_ctx *c, const std::vector<HostCopy> &list, bool h2d) {
-    std::vector<HostCopy> staged;
-    const bool allow = c->staged_host_copies;
-    for (const HostCopy &hc : list) {
-        if (allow && hc.bytes >= 2 * HC_CHUNK && is_pageable(hc.host)) staged.push_back(hc);
-        else if (h2d) SF_CUDA(cudaMemcpyAsync(hc.dev, hc.host, hc.bytes, cudaMemcpyHostToDevice, c->stream));
-    }
+    std::vector<HostCopy> staged, direct;
+    for (const HostCopy &hc : list)
+        (c->staged_host_copies && hc.bytes >= 2 * HC_CHUNK && is_pageable(hc.host) ? staged : direct).push_back(hc);
+    if (h2d)
+        for (const HostCopy &hc : direct) SF_CUDA(cudaMemcpyAsync(hc.dev, hc.host, hc.bytes, cudaMemcpyHostToDevice, c->stream));
     if (!staged.empty()) {
         const int rc = staged_batch(c, staged, h2d);
         if (rc != SFGPU_OK) return rc;
     }
     if (!h2d)
-        for (const HostCopy &hc : list)
-            if (!(allow && hc.bytes >= 2 * HC_CHUNK && is_pageable(hc.host)))
-                SF_CUDA(cudaMemcpyAsync(hc.host, hc.dev, hc.bytes, cudaMemcpyDeviceToHost, c->stream));
+        for (const HostCopy &hc : direct) SF_CUDA(cudaMemcpyAsync(hc.host, hc.dev, hc.bytes, cudaMemcpyDeviceToHost, c->stream));
     return SFGPU_OK;
+}
+
+enum { UPLOADED, PASSED, DRAINED }; // the event rings of sfgpu_ctx::copy_ev
+
+// Pageable caller memory (the reference's image_new is malloc): cudaMemcpyAsync would stage it synchronously through the
+// driver and no transfer would overlap anything, so such a call takes the staged copies above, stage by stage.
+int CopyPipeline::start(const std::vector<const void *> &buffers) {
+    pageable = std::any_of(buffers.begin(), buffers.end(), is_pageable);
+    if (pageable) return SFGPU_OK;
+    for (cudaStream_t *st : {&c->h2d, &c->d2h})
+        if (!*st) SF_CUDA(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+    for (auto &ring : c->copy_ev)
+        for (cudaEvent_t &e : ring)
+            if (!e) SF_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    // the previous call may still read the io area: compute has passed stage -1 (slot 3, free until pass(3))
+    SF_CUDA(cudaEventRecord(c->copy_ev[PASSED][3], c->stream));
+    SF_CUDA(cudaStreamWaitEvent(c->h2d, c->copy_ev[PASSED][3], 0));
+    return SFGPU_OK;
+}
+
+int CopyPipeline::upload(int k, const std::vector<HostCopy> &list, int passed, int drained) {
+    if (pageable) return host_copies(c, list, true);
+    if (passed >= 0) SF_CUDA(cudaStreamWaitEvent(c->h2d, c->copy_ev[PASSED][passed & 3], 0));
+    if (drained >= 0) SF_CUDA(cudaStreamWaitEvent(c->h2d, c->copy_ev[DRAINED][drained & 3], 0));
+    for (const HostCopy &hc : list) SF_CUDA(cudaMemcpyAsync(hc.dev, hc.host, hc.bytes, cudaMemcpyHostToDevice, c->h2d));
+    SF_CUDA(cudaEventRecord(c->copy_ev[UPLOADED][k & 3], c->h2d));
+    return SFGPU_OK;
+}
+
+int CopyPipeline::wait(int uploaded, int drained) {
+    if (pageable) return SFGPU_OK;
+    if (uploaded >= 0) SF_CUDA(cudaStreamWaitEvent(c->stream, c->copy_ev[UPLOADED][uploaded & 3], 0));
+    if (drained >= 0) SF_CUDA(cudaStreamWaitEvent(c->stream, c->copy_ev[DRAINED][drained & 3], 0));
+    return SFGPU_OK;
+}
+
+int CopyPipeline::pass(int k) {
+    if (!pageable) SF_CUDA(cudaEventRecord(c->copy_ev[PASSED][k & 3], c->stream));
+    return SFGPU_OK;
+}
+
+int CopyPipeline::download(int k, const std::vector<HostCopy> &list) {
+    if (pageable) return host_copies(c, list, false);
+    SF_CUDA(cudaStreamWaitEvent(c->d2h, c->copy_ev[PASSED][k & 3], 0));
+    for (const HostCopy &hc : list) SF_CUDA(cudaMemcpyAsync(hc.host, hc.dev, hc.bytes, cudaMemcpyDeviceToHost, c->d2h));
+    SF_CUDA(cudaEventRecord(c->copy_ev[DRAINED][k & 3], c->d2h));
+    return SFGPU_OK;
+}
+
+int CopyPipeline::finish(int status) {
+    for (cudaStream_t st : {c->h2d, c->stream, c->d2h}) {
+        const cudaError_t e = st ? cudaStreamSynchronize(st) : cudaSuccess;
+        if (status == SFGPU_OK && !cuda_ok(e, "copy pipeline: cudaStreamSynchronize")) status = SFGPU_ERR_CUDA;
+    }
+    return status;
 }
 
 } // namespace sf

@@ -3,7 +3,8 @@
 // sfgpu_variational_sequence_u8 / _u16 (the integer images the reference holds before its float conversion,
 // adaptiveFR.cpp:450-464 colorMat2colorImg<Vec3b> / mat2colorImg<uchar>, slow_flow.cpp:470-477 convertTo(CV_32F)).
 //
-// Three streams and events only: uploads of pair j+1 and downloads of pair j-1 overlap the solve of pair j.  A frame
+// The copies go through CopyPipeline (sf_hostcopy.cu), one stage per pair: with page-locked caller memory the upload of
+// pair j+1 and the download of pair j-1 overlap the solve of pair j; pageable memory takes the staged copies.  A frame
 // shared by two pairs is uploaded once (3-slot device ring); with `continue_from_previous` the first frame of a call is
 // the last frame of the previous call and is not uploaded at all.  Integer frames cross PCIe as they are (1 or 2 bytes
 // per sample, interleaved) and are converted to the planar fp32 layout of image.c:71-89 on the device -- exact, since
@@ -52,15 +53,6 @@ struct SeqFrames { // where the frames of a call come from
     const void *host(int f) const { return ints ? ints[f].data : (const void *)f32[f]->c1; }
 };
 
-int ensure_seq_events(sfgpu_ctx *c) {
-    for (auto &ring : c->seq_ev)
-        for (auto &e : ring)
-            if (!e) SF_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    if (!c->h2d) SF_CUDA(cudaStreamCreateWithFlags(&c->h2d, cudaStreamNonBlocking));
-    if (!c->d2h) SF_CUDA(cudaStreamCreateWithFlags(&c->d2h, cudaStreamNonBlocking));
-    return SFGPU_OK;
-}
-
 static void launch_unpack(sfgpu_ctx *c, Geom g, const SeqFrames &src, int f, const unsigned char *raw, float *dst) {
     const dim3 grid((g.S / 4 + 255) / 256, g.H);
     if (src.depth == 8)
@@ -92,8 +84,6 @@ static int run_sequence(sfgpu_ctx *c, int n_pairs, const SeqFrames &src, image_t
     }
     rc = c->ensure_workspace(g);
     if (rc != SFGPU_OK) return rc;
-    rc = ensure_seq_events(c);
-    if (rc != SFGPU_OK) return rc;
     size_t raw_slot = 0;
     if (src.ints) {
         for (int f = 0; f <= n_pairs; f++) raw_slot = std::max(raw_slot, src.raw_bytes(f));
@@ -111,78 +101,39 @@ static int run_sequence(sfgpu_ctx *c, int n_pairs, const SeqFrames &src, image_t
     auto frame_slot = [&](int f) { return c->io + (size_t)((f + base) % 3) * 3 * P; };
     auto raw_of = [&](int f) { return c->seq_raw + (size_t)((f + base) % 3) * raw_slot; };
     auto flow_slot = [&](int j) { return c->io + 9 * P + (size_t)(j % 3) * 2 * P; };
-    cudaEvent_t *up = c->seq_ev[0], *done = c->seq_ev[1], *down = c->seq_ev[2]; // rings of 4: index j & 3
-
-    // Pageable caller memory (the reference's image_new is malloc): cudaMemcpyAsync would stage it synchronously through
-    // the driver and no transfer would overlap anything.  Such callers take the multi-threaded staged copies of
-    // sf_hostcopy.cu pair by pair (frames are still uploaded once); page-locked / registered memory is pipelined.
-    bool pageable = false;
-    for (int f = 0; f <= n_pairs && !pageable; f++) pageable = is_pageable(src.host(f));
-    for (int j = 0; j < n_pairs && !pageable; j++) pageable = is_pageable(wx[j]->data) || is_pageable(wy[j]->data);
-
     auto frame_copy = [&](int f) -> HostCopy {
         if (src.ints) return HostCopy{raw_of(f), const_cast<void *>(src.host(f)), src.raw_bytes(f)};
         return HostCopy{frame_slot(f), const_cast<void *>(src.host(f)), 3 * P * sizeof(float)};
     };
-    if (pageable) {
-        for (int j = 0; j < n_pairs; j++) {
-            std::vector<HostCopy> upl;
-            if (j == 0 && !keep) upl.push_back(frame_copy(0));
-            upl.push_back(frame_copy(j + 1));
-            upl.push_back(HostCopy{flow_slot(j), wx[j]->data, P * sizeof(float)});
-            upl.push_back(HostCopy{flow_slot(j) + P, wy[j]->data, P * sizeof(float)});
-            rc = host_copies(c, upl, true);
-            if (rc != SFGPU_OK) return rc;
-            if (src.ints) {
-                if (j == 0 && !keep) launch_unpack(c, g, src, 0, raw_of(0), frame_slot(0));
-                launch_unpack(c, g, src, j + 1, raw_of(j + 1), frame_slot(j + 1));
-            }
-            rc = run_two_frame(c, g, flow_slot(j), flow_slot(j) + P, frame_slot(j), frame_slot(j + 1), params);
-            if (rc != SFGPU_OK) return rc;
-            rc = host_copies(c, {{flow_slot(j), wx[j]->data, P * sizeof(float)}, {flow_slot(j) + P, wy[j]->data, P * sizeof(float)}}, false);
-            if (rc != SFGPU_OK) return rc;
-            SF_CUDA(cudaStreamSynchronize(c->stream));
-        }
-        c->seq_geom = g;
-        c->seq_last_slot = (n_pairs + base) % 3;
-        return SFGPU_OK;
-    }
-
-    int status = SFGPU_OK;
-    auto h2d_copy = [&](const HostCopy &hc) { return cuda_ok(cudaMemcpyAsync(hc.dev, hc.host, hc.bytes, cudaMemcpyHostToDevice, c->h2d), "h2d"); };
-    auto upload = [&](int j) -> bool { // inputs of pair j: frame j+1 (and frame 0 for j == 0) + initial flow j
-        if (j >= 2 && !cuda_ok(cudaStreamWaitEvent(c->h2d, done[(j - 2) & 3], 0), "wait done")) return false; // frame slot (j+1)%3 last read by pair j-2
-        if (j >= 3 && !cuda_ok(cudaStreamWaitEvent(c->h2d, down[(j - 3) & 3], 0), "wait down")) return false; // flow slot j%3 last drained for pair j-3
-        if (j == 0 && !keep && !h2d_copy(frame_copy(0))) return false;
-        if (!h2d_copy(frame_copy(j + 1))) return false;
-        if (!h2d_copy(HostCopy{flow_slot(j), wx[j]->data, P * sizeof(float)})) return false;
-        if (!h2d_copy(HostCopy{flow_slot(j) + P, wy[j]->data, P * sizeof(float)})) return false;
-        return cuda_ok(cudaEventRecord(up[j & 3], c->h2d), "record up");
+    auto flow_copies = [&](int j) -> std::vector<HostCopy> {
+        return {{flow_slot(j), wx[j]->data, P * sizeof(float)}, {flow_slot(j) + P, wy[j]->data, P * sizeof(float)}};
     };
-    auto download = [&](int j) -> bool {
-        if (!cuda_ok(cudaStreamWaitEvent(c->d2h, done[j & 3], 0), "wait done")) return false;
-        if (!cuda_ok(cudaMemcpyAsync(wx[j]->data, flow_slot(j), P * sizeof(float), cudaMemcpyDeviceToHost, c->d2h), "d2h wx")) return false;
-        if (!cuda_ok(cudaMemcpyAsync(wy[j]->data, flow_slot(j) + P, P * sizeof(float), cudaMemcpyDeviceToHost, c->d2h), "d2h wy")) return false;
-        return cuda_ok(cudaEventRecord(down[j & 3], c->d2h), "record down");
+    CopyPipeline pipe(c); // stage j = pair j
+    // inputs of pair j: frame j+1 (and frame 0 for j == 0) + initial flow j.  Frame slot (j+1)%3 was last read by pair
+    // j-2, flow slot j%3 last drained for pair j-3.
+    auto upload = [&](int j) {
+        std::vector<HostCopy> up = flow_copies(j);
+        up.insert(up.begin(), frame_copy(j + 1));
+        if (j == 0 && !keep) up.insert(up.begin(), frame_copy(0));
+        return pipe.upload(j, up, j - 2, j - 3);
     };
-    // the previous work on the compute stream may still use the io ring (done[3] is free until pair 3 records it)
-    if (!cuda_ok(cudaEventRecord(done[3], c->stream), "record") || !cuda_ok(cudaStreamWaitEvent(c->h2d, done[3], 0), "wait")) status = SFGPU_ERR_CUDA;
-    if (status == SFGPU_OK && !upload(0)) status = SFGPU_ERR_CUDA;
+    std::vector<const void *> buffers;
+    for (int f = 0; f <= n_pairs; f++) buffers.push_back(src.host(f));
+    for (int j = 0; j < n_pairs; j++) buffers.insert(buffers.end(), {wx[j]->data, wy[j]->data});
+    int status = pipe.start(buffers);
+    if (status == SFGPU_OK) status = upload(0);
     for (int j = 0; j < n_pairs && status == SFGPU_OK; j++) {
-        if (!cuda_ok(cudaStreamWaitEvent(c->stream, up[j & 3], 0), "wait up")) { status = SFGPU_ERR_CUDA; break; }
+        if ((status = pipe.wait(j)) != SFGPU_OK) break;
         if (src.ints) {
             if (j == 0 && !keep) launch_unpack(c, g, src, 0, raw_of(0), frame_slot(0));
             launch_unpack(c, g, src, j + 1, raw_of(j + 1), frame_slot(j + 1));
         }
-        status = run_two_frame(c, g, flow_slot(j), flow_slot(j) + P, frame_slot(j), frame_slot(j + 1), params);
-        if (status != SFGPU_OK) break;
-        if (!cuda_ok(cudaEventRecord(done[j & 3], c->stream), "record done")) { status = SFGPU_ERR_CUDA; break; }
-        if (j + 1 < n_pairs && !upload(j + 1)) { status = SFGPU_ERR_CUDA; break; }
-        if (!download(j)) { status = SFGPU_ERR_CUDA; break; }
+        if ((status = run_two_frame(c, g, flow_slot(j), flow_slot(j) + P, frame_slot(j), frame_slot(j + 1), params)) != SFGPU_OK) break;
+        if ((status = pipe.pass(j)) != SFGPU_OK) break;
+        if (j + 1 < n_pairs && (status = upload(j + 1)) != SFGPU_OK) break;
+        status = pipe.download(j, flow_copies(j));
     }
-    cudaStreamSynchronize(c->h2d);
-    cudaStreamSynchronize(c->stream);
-    if (!cuda_ok(cudaStreamSynchronize(c->d2h), "sync d2h") && status == SFGPU_OK) status = SFGPU_ERR_CUDA;
+    status = pipe.finish(status);
     if (status == SFGPU_OK) {
         c->seq_geom = g;
         c->seq_last_slot = (n_pairs + base) % 3;
