@@ -28,7 +28,9 @@ extern "C" {
 #endif
 
 /* ---- containers: identical layout to epic_flow_extended/image.h:17-34.  If the reference's
- * image.h was included first its definitions are used (same names, same fields). ---- */
+ * image.h was included first its definitions are used (same names, same fields).  Every sfgpu_* entry that takes them
+ * returns SFGPU_ERR_ARG, before it touches the device or any buffer, when an argument has NULL data, width or height
+ * < 1, a stride other than ceil4(width), colour planes that are not contiguous, or another geometry than the call's. ---- */
 #ifndef __IMAGE_H_
 typedef struct image_s {
     int width;   /* valid columns */
@@ -162,8 +164,9 @@ int sfgpu_host_unregister(void *ptr);
 
 /* multi-frame refinement (replaces Variational_MT::variational, variational_mt.cpp:526-784).
  * im: F = 2*(S-1)+1 host colour images, reference frame at index S-1.  channel_w may be NULL (all
- * ones, variational_mt.cpp:535-538).  occlusions_out may be NULL; otherwise receives the -1/0/+1
- * labels of the finest level (Variational_MT::getOcclusions).  avg_change_out: the returned Point2f. */
+ * ones, variational_mt.cpp:535-538).  occlusions_out may be NULL (or have NULL data); otherwise receives the -1/0/+1
+ * labels of the finest level (Variational_MT::getOcclusions).  channel_w and occlusions_out, when given, have the
+ * flow's geometry.  avg_change_out: the returned Point2f. */
 int sfgpu_variational_mt(sfgpu_ctx *ctx, image_t *wx, image_t *wy, const color_image_t *const *im,
                          const sf_mt_params_t *params, const color_image_t *channel_w,
                          image_t *occlusions_out, float avg_change_out[2]);

@@ -27,6 +27,13 @@ Penalty make_penalty(int type, float eps, float trunc) {
     return p;
 }
 
+// the 5-tap derivative filter of the two-frame path (image.c:425)
+static bool at_least_5x5(const std::string &at, Geom g) {
+    if (g.W >= 5 && g.H >= 5) return true;
+    set_error(at + "image must be at least 5x5 (5-tap derivative filter, image.c:425)");
+    return false;
+}
+
 } // namespace sf
 
 using namespace sf;
@@ -35,10 +42,7 @@ using namespace sf;
 enum { PROF_SOR = 0, PROF_DATA = 1, PROF_CUT = 2 };
 
 int sfgpu_ctx::ensure_workspace(Geom geom) {
-    if (geom.W < 5 || geom.H < 5) {
-        set_error("image must be at least 5x5 (5-tap derivative filter, image.c:425)");
-        return SFGPU_ERR_ARG;
-    }
+    if (!at_least_5x5("", geom)) return SFGPU_ERR_ARG;
     const size_t P = geom.plane();
     const size_t need = (size_t)(SP_COUNT + 3 + 1 + 2 + 1) * P;
     if (need > ws_floats) {
@@ -262,30 +266,49 @@ int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d
     return SFGPU_OK;
 }
 
-} // namespace sf
+// ------------------------------------------------------------------------------------------ argument checks
+std::string Caller::at(int k) const {
+    return item ? std::string(fn) + ": " + item + " " + std::to_string(first + k) + ": " : std::string(fn) + ": ";
+}
 
-bool sf::check_pair(const image_t *wx, const image_t *wy, const color_image_t *im1, const color_image_t *im2) {
-    if (!wx || !wy || !im1 || !im2 || !wx->data || !wy->data || !im1->c1 || !im2->c1) {
-        set_error("null image argument");
+static float *data_of(const image_t *a) { return a->data; }
+static float *data_of(const color_image_t *a) { return a->c1; }
+static bool contiguous(const image_t *) { return true; }
+static bool contiguous(const color_image_t *a) { // image.c:80-87; the geometry has been checked
+    const size_t P = (size_t)a->stride * a->height;
+    return a->c2 == a->c1 + P && a->c3 == a->c2 + P;
+}
+static std::string dims(int w, int h, int s) { return std::to_string(w) + "x" + std::to_string(h) + " stride " + std::to_string(s); }
+
+// sets_g: `a` gives the call's geometry g, else it must have it
+template <typename Image>
+static bool check_image(const std::string &at, const std::string &name, const Image *a, Geom &g, bool sets_g) {
+    std::string what;
+    if (!a || !data_of(a))
+        what = "null image";
+    else if (!sets_g && (a->width != g.W || a->height != g.H || a->stride != g.S))
+        what = "different geometry (" + dims(a->width, a->height, a->stride) + "; the images of a call share width/height/stride, here " +
+               dims(g.W, g.H, g.S) + ")";
+    else if (a->width < 1 || a->height < 1)
+        what = "width and height must be >= 1 (" + dims(a->width, a->height, a->stride) + ")";
+    else if (a->stride != (((long long)a->width + 3) / 4) * 4)
+        what = "stride must be ceil4(width) (image.c:25), not " + dims(a->width, a->height, a->stride);
+    else if (!contiguous(a))
+        what = "colour images must be planar and contiguous (image.c:80-87)";
+    if (!what.empty()) {
+        set_error(at + name + ": " + what);
         return false;
     }
-    const int w = wx->width, h = wx->height, s = wx->stride;
-    if (s != ((w + 3) / 4) * 4) {
-        set_error("stride must be ceil4(width) (image.c:25)");
-        return false;
-    }
-    if (wy->width != w || wy->height != h || wy->stride != s || im1->width != w || im1->height != h ||
-        im1->stride != s || im2->width != w || im2->height != h || im2->stride != s) {
-        set_error("flow planes and images must share width/height/stride");
-        return false;
-    }
-    const size_t P = (size_t)s * h;
-    if (im1->c2 != im1->c1 + P || im1->c3 != im1->c2 + P || im2->c2 != im2->c1 + P || im2->c3 != im2->c2 + P) {
-        set_error("colour images must be planar and contiguous (image.c:80-87)");
-        return false;
-    }
+    if (sets_g) g = make_geom(a->width, a->height);
     return true;
 }
+
+bool arg_geom(const std::string &at, const std::string &name, const image_t *a, Geom &g) { return check_image(at, name, a, g, true); }
+bool arg_geom(const std::string &at, const std::string &name, const color_image_t *a, Geom &g) { return check_image(at, name, a, g, true); }
+bool arg_is(const std::string &at, const std::string &name, const image_t *a, Geom g) { return check_image(at, name, a, g, false); }
+bool arg_is(const std::string &at, const std::string &name, const color_image_t *a, Geom g) { return check_image(at, name, a, g, false); }
+
+} // namespace sf
 
 // ------------------------------------------------------------------------------------------ ABI: basics
 extern "C" {
@@ -462,7 +485,7 @@ int sfgpu_variational_dev(sfgpu_ctx *c, float *d_wx, float *d_wy, const float *d
         set_error("sfgpu_variational_dev: null argument");
         return SFGPU_ERR_ARG;
     }
-    if (stride != ((width + 3) / 4) * 4) {
+    if (stride != make_geom(width, height).S) {
         set_error("stride must be ceil4(width)");
         return SFGPU_ERR_ARG;
     }
@@ -472,10 +495,11 @@ int sfgpu_variational_dev(sfgpu_ctx *c, float *d_wx, float *d_wy, const float *d
 
 int sfgpu_variational(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_image_t *im1, const color_image_t *im2,
                       const variational_params_t *params) {
-    if (!c) return SFGPU_ERR_ARG;
-    if (!check_pair(wx, wy, im1, im2)) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_variational: ";
+    Geom g;
+    if (!c || !arg_geom(at, "wx", wx, g) || !arg_is(at, "wy", wy, g) || !arg_is(at, "im1", im1, g) || !arg_is(at, "im2", im2, g))
+        return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{wx->width, wx->height, wx->stride};
     const size_t P = g.plane();
     int rc = c->ensure_io(8 * P);
     if (rc != SFGPU_OK) return rc;
@@ -518,8 +542,6 @@ void variational(image_t *wx, image_t *wy, const color_image_t *im1, const color
 }
 
 // ------------------------------------------------------------------------------------------ ABI: operator twins
-static bool same_geom(const image_t *a, int w, int h, int s) { return a && a->data && a->width == w && a->height == h && a->stride == s; }
-
 struct DevPlanes { // scratch device planes for the operator twins
     float *p = nullptr;
     ~DevPlanes() { if (p) cudaFree(p); }
@@ -530,9 +552,12 @@ struct DevPlanes { // scratch device planes for the operator twins
 
 int sfgpu_image_warp(sfgpu_ctx *c, color_image_t *dst, image_t *mask, const color_image_t *src, const image_t *wx,
                      const image_t *wy, int factor) {
-    if (!c || !dst || !src || !wx || !wy) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_image_warp: ";
+    Geom g;
+    if (!c || !arg_geom(at, "src", src, g) || !arg_is(at, "dst", dst, g) || !arg_is(at, "wx", wx, g) || !arg_is(at, "wy", wy, g) ||
+        (mask && !arg_is(at, "mask", mask, g)))
+        return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{src->width, src->height, src->stride};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -548,26 +573,22 @@ int sfgpu_image_warp(sfgpu_ctx *c, color_image_t *dst, image_t *mask, const colo
     return SFGPU_OK;
 }
 
-static bool same_cgeom(const color_image_t *a, int w, int h, int s) { return a && a->c1 && a->width == w && a->height == h && a->stride == s; }
-
 int sfgpu_warp_frame_derivs(sfgpu_ctx *c, const color_image_t *src, const image_t *wx, const image_t *wy, int factor, int variant,
                             color_image_t *warped, image_t *mask, color_image_t *dx, color_image_t *dy, color_image_t *dxx,
                             color_image_t *dxy, color_image_t *dyy) {
-    if (!c || !src || !src->c1 || !wx || !wy || !mask || variant < 0 || variant > 1) {
+    const char *at = "sfgpu_warp_frame_derivs: ";
+    if (!c || variant < 0 || variant > 1) {
         set_error("sfgpu_warp_frame_derivs: bad argument");
         return SFGPU_ERR_ARG;
     }
-    const int w = src->width, h = src->height, sd = src->stride;
-    color_image_t *outs[6] = {warped, dx, dy, dxx, dxy, dyy};
-    for (int k = 0; k < 6; k++)
-        if (!same_cgeom(outs[k], w, h, sd)) { set_error("sfgpu_warp_frame_derivs: geometry"); return SFGPU_ERR_ARG; }
-    if (wx->width != w || wx->height != h || wx->stride != sd || wy->width != w || wy->height != h || wy->stride != sd ||
-        mask->width != w || mask->height != h || mask->stride != sd) {
-        set_error("sfgpu_warp_frame_derivs: geometry");
+    Geom g;
+    if (!arg_geom(at, "src", src, g) || !arg_is(at, "wx", wx, g) || !arg_is(at, "wy", wy, g) || !arg_is(at, "mask", mask, g))
         return SFGPU_ERR_ARG;
-    }
+    color_image_t *outs[6] = {warped, dx, dy, dxx, dxy, dyy};
+    const char *names[6] = {"warped", "dx", "dy", "dxx", "dxy", "dyy"};
+    for (int k = 0; k < 6; k++)
+        if (!arg_is(at, names[k], outs[k], g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{w, h, sd};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -591,10 +612,15 @@ int sfgpu_warp_frame_derivs(sfgpu_ctx *c, const color_image_t *src, const image_
     return SFGPU_OK;
 }
 
-static int convolve_planes(sfgpu_ctx *c, float *dst, const float *src, Geom g, int planes, int horder, const float *hc, int vorder,
+extern "C++" { // Image: image_t (planes = 1) or color_image_t (planes = 3)
+template <typename Image>
+static int convolve_planes(sfgpu_ctx *c, Image *dst, const Image *src, int planes, int horder, const float *hc, int vorder,
                            const float *vc, const char *what) {
-    if (!c || !dst || !src || (!hc && !vc) || (hc && (horder < 1 || horder > 2)) || (vc && (vorder < 1 || vorder > 2))) {
-        set_error(std::string(what) + ": bad argument (order 1 = 3 taps, 2 = 5 taps)");
+    const std::string at = std::string(what) + ": ";
+    Geom g;
+    if (!arg_geom(at, "src", src, g) || !arg_is(at, "dst", dst, g)) return SFGPU_ERR_ARG;
+    if (!c || (!hc && !vc) || (hc && (horder < 1 || horder > 2)) || (vc && (vorder < 1 || vorder > 2))) {
+        set_error(at + "bad argument (order 1 = 3 taps, 2 = 5 taps)");
         return SFGPU_ERR_ARG;
     }
     SF_CUDA(cudaSetDevice(c->device));
@@ -603,7 +629,7 @@ static int convolve_planes(sfgpu_ctx *c, float *dst, const float *src, Geom g, i
     if (rc != SFGPU_OK) return rc;
     cudaStream_t st = c->stream;
     float *d_src = c->io, *d_tmp = c->io + n, *d_dst = c->io + 2 * n;
-    SF_CUDA(cudaMemcpyAsync(d_src, src, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    SF_CUDA(cudaMemcpyAsync(d_src, data_of(src), n * sizeof(float), cudaMemcpyHostToDevice, st));
     if (hc && vc) { // image.c:665-680: horizontal into a temporary, then vertical
         launch_convolve(st, g, d_src, d_tmp, false, horder, hc, planes);
         launch_convolve(st, g, d_tmp, d_dst, true, vorder, vc, planes);
@@ -612,38 +638,36 @@ static int convolve_planes(sfgpu_ctx *c, float *dst, const float *src, Geom g, i
         launch_convolve(st, g, d_src, d_dst, vc != nullptr, hc ? horder : vorder, hc ? hc : vc, planes);
         c->prof_acc.kernel_launches++;
     }
-    SF_CUDA(cudaMemcpyAsync(dst, d_dst, n * sizeof(float), cudaMemcpyDeviceToHost, st));
+    SF_CUDA(cudaMemcpyAsync(data_of(dst), d_dst, n * sizeof(float), cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaStreamSynchronize(st));
     return SFGPU_OK;
 }
+} // extern "C++"
 
 int sfgpu_convolve_horiz(sfgpu_ctx *c, image_t *dst, const image_t *src, int order, const float *coeffs) {
-    if (!src || !same_geom(dst, src->width, src->height, src->stride)) { set_error("sfgpu_convolve_horiz: geometry"); return SFGPU_ERR_ARG; }
-    return convolve_planes(c, dst->data, src->data, Geom{src->width, src->height, src->stride}, 1, order, coeffs, 0, nullptr, "sfgpu_convolve_horiz");
+    return convolve_planes(c, dst, src, 1, order, coeffs, 0, nullptr, "sfgpu_convolve_horiz");
 }
 int sfgpu_convolve_vert(sfgpu_ctx *c, image_t *dst, const image_t *src, int order, const float *coeffs) {
-    if (!src || !same_geom(dst, src->width, src->height, src->stride)) { set_error("sfgpu_convolve_vert: geometry"); return SFGPU_ERR_ARG; }
-    return convolve_planes(c, dst->data, src->data, Geom{src->width, src->height, src->stride}, 1, 0, nullptr, order, coeffs, "sfgpu_convolve_vert");
+    return convolve_planes(c, dst, src, 1, 0, nullptr, order, coeffs, "sfgpu_convolve_vert");
 }
 int sfgpu_color_image_convolve_hv(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src, int horiz_order, const float *horiz_coeffs,
                                   int vert_order, const float *vert_coeffs) {
-    if (!src || !same_cgeom(dst, src->width, src->height, src->stride)) { set_error("sfgpu_color_image_convolve_hv: geometry"); return SFGPU_ERR_ARG; }
-    return convolve_planes(c, dst->c1, src->c1, Geom{src->width, src->height, src->stride}, 3, horiz_order, horiz_coeffs, vert_order, vert_coeffs,
-                           "sfgpu_color_image_convolve_hv");
+    return convolve_planes(c, dst, src, 3, horiz_order, horiz_coeffs, vert_order, vert_coeffs, "sfgpu_color_image_convolve_hv");
 }
 
 // get_derivatives (variational_aux.c:55-78) with the 5-tap derivative filter of variational.c:118-119
 int sfgpu_get_derivatives(sfgpu_ctx *c, const color_image_t *im1, const color_image_t *im2, color_image_t *dx, color_image_t *dy,
                           color_image_t *dt, color_image_t *dxx, color_image_t *dxy, color_image_t *dyy, color_image_t *dxt,
                           color_image_t *dyt) {
-    if (!c || !im1 || !im1->c1) { set_error("sfgpu_get_derivatives: null argument"); return SFGPU_ERR_ARG; }
-    const int w = im1->width, h = im1->height, sd = im1->stride;
+    const char *at = "sfgpu_get_derivatives: ";
+    Geom g;
+    if (!c) { set_error("sfgpu_get_derivatives: null argument"); return SFGPU_ERR_ARG; }
+    if (!arg_geom(at, "im1", im1, g) || !arg_is(at, "im2", im2, g)) return SFGPU_ERR_ARG;
     color_image_t *outs[8] = {dx, dy, dt, dxx, dxy, dyy, dxt, dyt};
-    if (!same_cgeom(im2, w, h, sd)) { set_error("sfgpu_get_derivatives: geometry"); return SFGPU_ERR_ARG; }
+    const char *names[8] = {"dx", "dy", "dt", "dxx", "dxy", "dyy", "dxt", "dyt"};
     for (int k = 0; k < 8; k++)
-        if (!same_cgeom(outs[k], w, h, sd)) { set_error("sfgpu_get_derivatives: geometry"); return SFGPU_ERR_ARG; }
+        if (!arg_is(at, names[k], outs[k], g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{w, h, sd};
     const size_t n = 3 * g.plane();
     int rc = c->ensure_io(11 * n);
     if (rc != SFGPU_OK) return rc;
@@ -669,9 +693,10 @@ int sfgpu_get_derivatives(sfgpu_ctx *c, const color_image_t *im1, const color_im
 
 int sfgpu_compute_dpsis_weight(sfgpu_ctx *c, image_t *dst, const color_image_t *im, float coef, const float *avg3,
                                const float *std3, int hbit) {
-    if (!c || !dst || !im) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_compute_dpsis_weight: ";
+    Geom g;
+    if (!c || !arg_geom(at, "im", im, g) || !arg_is(at, "dst", dst, g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{im->width, im->height, im->stride};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -689,13 +714,16 @@ int sfgpu_compute_dpsis_weight(sfgpu_ctx *c, image_t *dst, const color_image_t *
 int sfgpu_compute_smoothness(sfgpu_ctx *c, image_t *dst_horiz, image_t *dst_vert, const image_t *uu, const image_t *vv,
                              const image_t *w, float alpha_factor, int robust_reg, float reg_eps, float reg_trunc,
                              int mode) {
-    if (!c || !dst_horiz || !dst_vert || !uu || !vv || !w) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_compute_smoothness: ";
+    Geom g;
+    if (!c || !arg_geom(at, "uu", uu, g) || !arg_is(at, "vv", vv, g) || !arg_is(at, "dpsis_weight", w, g) ||
+        !arg_is(at, "dst_horiz", dst_horiz, g) || !arg_is(at, "dst_vert", dst_vert, g))
+        return SFGPU_ERR_ARG;
     if (mode < 0 || mode > 1) {
         set_error("smoothing modes >= 2 are not supported (reference bug Q6)");
         return SFGPU_ERR_UNSUPPORTED;
     }
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{uu->width, uu->height, uu->stride};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -713,10 +741,13 @@ int sfgpu_compute_smoothness(sfgpu_ctx *c, image_t *dst_horiz, image_t *dst_vert
 int sfgpu_compute_data_and_match(sfgpu_ctx *c, image_t *a11, image_t *a12, image_t *a22, image_t *b1, image_t *b2,
                                  const image_t *mask, const image_t *du, const image_t *dv, const color_image_t *im1,
                                  const color_image_t *im2w, float half_delta_over3, float half_gamma_over3) {
-    if (!c || !a11 || !a12 || !a22 || !b1 || !b2 || !mask || !du || !dv || !im1 || !im2w) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_compute_data_and_match: ";
+    Geom g;
+    if (!c || !arg_geom(at, "im1", im1, g) || !arg_is(at, "im2w", im2w, g) || !arg_is(at, "mask", mask, g) || !arg_is(at, "du", du, g) ||
+        !arg_is(at, "dv", dv, g) || !arg_is(at, "a11", a11, g) || !arg_is(at, "a12", a12, g) || !arg_is(at, "a22", a22, g) ||
+        !arg_is(at, "b1", b1, g) || !arg_is(at, "b2", b2, g) || !at_least_5x5(at, g))
+        return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{im1->width, im1->height, im1->stride};
-    if (g.W < 5 || g.H < 5) return SFGPU_ERR_ARG;
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -740,18 +771,18 @@ int sfgpu_compute_data_and_match(sfgpu_ctx *c, image_t *a11, image_t *a12, image
 int sfgpu_prep_two_frame(sfgpu_ctx *c, image_t *a11, image_t *a12, image_t *a22, image_t *b1, image_t *b2, const color_image_t *im1,
                          const color_image_t *im2, const image_t *wx, const image_t *wy, const image_t *du, const image_t *dv,
                          const image_t *ph, const image_t *pv, float half_delta_over3, float half_gamma_over3) {
-    if (!c || !a11 || !a12 || !a22 || !b1 || !b2 || !ph || !pv || (du == nullptr) != (dv == nullptr)) {
+    const char *at = "sfgpu_prep_two_frame: ";
+    Geom g;
+    if (!c || (du == nullptr) != (dv == nullptr)) {
         set_error("sfgpu_prep_two_frame: null argument");
         return SFGPU_ERR_ARG;
     }
-    if (!check_pair(wx, wy, im1, im2)) return SFGPU_ERR_ARG;
-    const int w = wx->width, h = wx->height, sd = wx->stride;
-    const image_t *planes[9] = {a11, a12, a22, b1, b2, ph, pv, du, dv};
-    for (int k = 0; k < 9; k++)
-        if (planes[k] && !same_geom(planes[k], w, h, sd)) { set_error("sfgpu_prep_two_frame: geometry"); return SFGPU_ERR_ARG; }
-    if (w < 5 || h < 5) { set_error("image must be at least 5x5 (5-tap derivative filter, image.c:425)"); return SFGPU_ERR_ARG; }
+    if (!arg_geom(at, "wx", wx, g) || !arg_is(at, "wy", wy, g) || !arg_is(at, "im1", im1, g) || !arg_is(at, "im2", im2, g) ||
+        (du && (!arg_is(at, "du", du, g) || !arg_is(at, "dv", dv, g))) || !arg_is(at, "dpsis_horiz", ph, g) ||
+        !arg_is(at, "dpsis_vert", pv, g) || !arg_is(at, "a11", a11, g) || !arg_is(at, "a12", a12, g) || !arg_is(at, "a22", a22, g) ||
+        !arg_is(at, "b1", b1, g) || !arg_is(at, "b2", b2, g) || !at_least_5x5(at, g))
+        return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{w, h, sd};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -774,9 +805,12 @@ int sfgpu_prep_two_frame(sfgpu_ctx *c, image_t *a11, image_t *a12, image_t *a22,
 }
 
 int sfgpu_sub_laplacian(sfgpu_ctx *c, image_t *dst, const image_t *src, const image_t *wh, const image_t *wv) {
-    if (!c || !dst || !src || !wh || !wv) return SFGPU_ERR_ARG;
+    const char *at = "sfgpu_sub_laplacian: ";
+    Geom g;
+    if (!c || !arg_geom(at, "src", src, g) || !arg_is(at, "dst", dst, g) || !arg_is(at, "weight_horiz", wh, g) ||
+        !arg_is(at, "weight_vert", wv, g))
+        return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{src->width, src->height, src->stride};
     const size_t P = g.plane();
     cudaStream_t st = c->stream;
     DevPlanes d;
@@ -793,15 +827,13 @@ int sfgpu_sub_laplacian(sfgpu_ctx *c, image_t *dst, const image_t *src, const im
 int sfgpu_sor_coupled(sfgpu_ctx *c, image_t *du, image_t *dv, image_t *a11, image_t *a12, image_t *a22,
                       const image_t *b1, const image_t *b2, const image_t *ph, const image_t *pv, int iterations,
                       float omega) {
-    if (!c || !du || !dv || !a11 || !a12 || !a22 || !b1 || !b2 || !ph || !pv) return SFGPU_ERR_ARG;
-    const int w = du->width, h = du->height, s = du->stride;
-    if (!same_geom(dv, w, h, s) || !same_geom(a11, w, h, s) || !same_geom(a12, w, h, s) || !same_geom(a22, w, h, s) ||
-        !same_geom(b1, w, h, s) || !same_geom(b2, w, h, s) || !same_geom(ph, w, h, s) || !same_geom(pv, w, h, s)) {
-        set_error("sfgpu_sor_coupled: geometry mismatch");
+    const char *at = "sfgpu_sor_coupled: ";
+    Geom g;
+    if (!c || !arg_geom(at, "du", du, g) || !arg_is(at, "dv", dv, g) || !arg_is(at, "a11", a11, g) || !arg_is(at, "a12", a12, g) ||
+        !arg_is(at, "a22", a22, g) || !arg_is(at, "b1", b1, g) || !arg_is(at, "b2", b2, g) || !arg_is(at, "dpsis_horiz", ph, g) ||
+        !arg_is(at, "dpsis_vert", pv, g))
         return SFGPU_ERR_ARG;
-    }
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{w, h, s};
     int rc = c->ensure_workspace(g);
     if (rc != SFGPU_OK) return rc;
     const size_t P = g.plane();

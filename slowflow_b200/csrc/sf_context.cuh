@@ -117,8 +117,27 @@ class CopyPipeline {
 // two-frame refinement on device planes (variational.c:19-82 + :101-143)
 int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d_im1, const float *d_im2,
                   const variational_params_t *params);
-// argument check shared by the host-buffer entries: one geometry, stride = ceil4(width), planar contiguous colour
-bool check_pair(const image_t *wx, const image_t *wy, const color_image_t *im1, const color_image_t *im2);
+
+// ---- image arguments of the host-buffer entries (the container contract of slowflow_gpu.h:30-44).  An entry copies whole
+// planes of P = stride * height floats (3 P from a colour image's c1), with P from the call's one geometry.
+// Names the entry point in error messages, and in a batch or sequence the item ("item" / "pair" numbered from `first`;
+// null: none): at(k) is "<fn>: " or "<fn>: <item> <first + k>: ".
+struct Caller {
+    const char *fn;
+    const char *item;
+    int first;
+    std::string at(int k) const;
+};
+// A failed check sets "<at><name>: <what>" and returns false; the entry then returns SFGPU_ERR_ARG before it touches the
+// device or any caller buffer.
+// arg_geom: the call's geometry g from argument `name`: non-null data, width and height >= 1, stride = ceil4(width), and
+// a colour image planar and contiguous (c2 = c1 + P, c3 = c2 + P).
+bool arg_geom(const std::string &at, const std::string &name, const image_t *a, Geom &g);
+bool arg_geom(const std::string &at, const std::string &name, const color_image_t *a, Geom &g);
+// arg_is: argument `name` has non-null data and exactly the geometry g (a colour image: also planar and contiguous)
+bool arg_is(const std::string &at, const std::string &name, const image_t *a, Geom g);
+bool arg_is(const std::string &at, const std::string &name, const color_image_t *a, Geom g);
+
 // exact binary Potts min-cut on the device (sf_mincut.cu); results in occ / device_cut_labels(), status after a stream sync
 int device_grid_mincut(sfgpu_ctx *c, DeviceCut *&cut, int W, int H, long long *tr_dev, long long pair_cap, float *occ, int S);
 const int *device_cut_status(const DeviceCut *cut);       // {0 = converged, phases, grid-wide passes}
@@ -127,17 +146,13 @@ const unsigned char *device_cut_labels(const DeviceCut *cut); // dense W*H label
 int run_sor(sfgpu_ctx *c, int iterations, float omega, int *cur, bool zero_init);
 
 // ---- EPIC interpolation (sf_epic.cu)
-// names the entry point in error messages, and for a batch the item ("item" / "pair" numbered from `first`; null: none)
-struct EpicCaller {
-    const char *fn;
-    const char *item;
-    int first;
-    std::string at(int k) const;
-};
-// the argument checks of sfgpu_epic_batch on n items: null pointers, one geometry, stride = ceil4(width), >= 4 match
-// columns, the method.  Touches nothing.
+// The argument checks of sfgpu_epic_batch on n items: null pointers, the call's geometry g from im[0], flows and edges of
+// that geometry, >= 4 match columns, the method.  Touches nothing.  names: of flowx, flowy and im[0] in the caller's
+// signature.  The callers check the other images against g: the batch its im[k], sfgpu_epicflow_sequence frame k + 1
+// under pair k, the first pair that reads it.
 int epic_check_args(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
-                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const EpicCaller &who);
+                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const Caller &who,
+                    const char *const names[3], Geom &g);
 // edges[k] += euc in the caller's arrays (epic.cpp:155-163)
 void epic_add_euc(int n, float_image *const *edges, float euc);
 // epic() on n items of one geometry on device planes, after epic_check_args and epic_add_euc.  d_cost: the items' W x H
@@ -145,5 +160,5 @@ void epic_add_euc(int n, float_image *const *edges, float euc);
 // when it is off); d_flow: item k's flow x at 2 k P and flow y at (2 k + 1) P, whole planes with zeroed padding.  stats: n
 // entries.  The last kernels are left queued on the context's stream; on an error d_flow is not fully written.
 int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d_lab, const float_image *const *input_matches,
-                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const EpicCaller &who);
+                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const Caller &who);
 } // namespace sf

@@ -962,7 +962,7 @@ template <typename F> static int with_arena(sfgpu_ctx *c, size_t first_guess, F 
 // filter reads them; null when it is off); d_flow: item k's flow x at 2 k P, flow y at (2 k + 1) P, written whole (padding
 // zeroed).  Runs with the arena installed; the flow kernels are left queued on the context's stream.  sstat: n entries.
 static int epic_core(sfgpu_ctx *c, int n, Geom g, const float *d_cost_in, const float *d_lab, const float_image *const *input_matches,
-                     const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *sstat, const EpicCaller &who) {
+                     const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *sstat, const Caller &who) {
     const int W = g.W, H = g.H;
     const bool la = strcmp(params->method, "LA") == 0;
     cudaStream_t st = c->stream;
@@ -1150,7 +1150,7 @@ static int epic_core(sfgpu_ctx *c, int n, Geom g, const float *d_cost_in, const 
 // sfgpu_epic / sfgpu_epic_batch: the caller's edge costs and Lab images go up, the flows come down
 static int epic_host(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
-                     const EpicCaller &who) {
+                     const Caller &who) {
     const Geom g{im[0]->width, im[0]->height, flowx[0]->stride};
     const size_t N = (size_t)g.W * g.H, P = g.plane();
     const bool sal = params->saliency_th != 0;
@@ -1186,12 +1186,9 @@ static int epic_host(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const 
 
 namespace sf {
 
-std::string EpicCaller::at(int k) const {
-    return item ? std::string(fn) + ": " + item + " " + std::to_string(first + k) + ": " : std::string(fn) + ": ";
-}
-
 int epic_check_args(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
-                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const EpicCaller &who) {
+                    const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, const Caller &who,
+                    const char *const names[3], Geom &g) {
     if (n < 1) {
         set_error(std::string(who.fn) + ": no item (n < 1)");
         return SFGPU_ERR_ARG;
@@ -1200,21 +1197,20 @@ int epic_check_args(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *
         set_error(std::string(who.fn) + ": null argument");
         return SFGPU_ERR_ARG;
     }
-    for (int k = 0; k < n; k++) {
-        if (!flowx[k] || !flowy[k] || !im[k] || !input_matches[k] || !edges[k] || !flowx[k]->data || !flowy[k]->data || !im[k]->c1 ||
-            !input_matches[k]->pixels || !edges[k]->pixels) {
+    for (int k = 0; k < n; k++)
+        if (!flowx[k] || !flowy[k] || !im[k] || !input_matches[k] || !edges[k] || !input_matches[k]->pixels || !edges[k]->pixels) {
             set_error(who.at(k) + "null argument");
             return SFGPU_ERR_ARG;
         }
-        const int W = im[k]->width, H = im[k]->height;
-        if (edges[k]->tx != W || edges[k]->ty != H || flowx[k]->width != W || flowx[k]->height != H || flowy[k]->width != W || flowy[k]->height != H ||
-            flowx[k]->stride != ((W + 3) / 4) * 4 || flowy[k]->stride != flowx[k]->stride || im[k]->stride != flowx[k]->stride || input_matches[k]->tx < 4) {
-            set_error(who.at(k) + "geometry mismatch (edges and flow planes must have the image's size; matches need >= 4 columns)");
+    if (!arg_geom(who.at(0), names[2], im[0], g)) return SFGPU_ERR_ARG;
+    for (int k = 0; k < n; k++) {
+        if (!arg_is(who.at(k), names[0], flowx[k], g) || !arg_is(who.at(k), names[1], flowy[k], g)) return SFGPU_ERR_ARG;
+        if (edges[k]->tx != g.W || edges[k]->ty != g.H) {
+            set_error(who.at(k) + "edges: must have the image's width x height (" + std::to_string(g.W) + "x" + std::to_string(g.H) + ")");
             return SFGPU_ERR_ARG;
         }
-        if (W != im[0]->width || H != im[0]->height) {
-            set_error(who.at(k) + "items of different geometry (" + std::to_string(W) + "x" + std::to_string(H) + ", item 0 is " +
-                      std::to_string(im[0]->width) + "x" + std::to_string(im[0]->height) + ")");
+        if (input_matches[k]->tx < 4) {
+            set_error(who.at(k) + "input_matches: need >= 4 columns (x1 y1 x2 y2)");
             return SFGPU_ERR_ARG;
         }
     }
@@ -1236,7 +1232,7 @@ void epic_add_euc(int n, float_image *const *edges, float euc) {
 size_t epic_arena_guess(int n, size_t N) { return n * N * 4 * 24 + ((size_t)64 << 20); }
 
 int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d_lab, const float_image *const *input_matches,
-                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const EpicCaller &who) {
+                const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const Caller &who) {
     return with_arena(c, epic_arena_guess(n, (size_t)g.W * g.H),
                       [&]() { return epic_core(c, n, g, d_cost, d_lab, input_matches, params, d_flow, stats, who); });
 }
@@ -1247,9 +1243,13 @@ int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d
 // the reference (epic.cpp:155-163), once whatever the arena does below
 static int epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
                       const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats,
-                      const EpicCaller &who) {
-    const int rc = epic_check_args(c, n, flowx, flowy, im, input_matches, edges, params, who);
+                      const Caller &who) {
+    const char *const names[3] = {"flowx", "flowy", "im"};
+    Geom g;
+    const int rc = epic_check_args(c, n, flowx, flowy, im, input_matches, edges, params, who, names, g);
     if (rc != SFGPU_OK) return rc;
+    for (int k = 1; k < n; k++) // im[0] gave g
+        if (!arg_is(who.at(k), "im", im[k], g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
     epic_add_euc(n, edges, params->euc);
     return with_arena(c, epic_arena_guess(n, (size_t)im[0]->width * im[0]->height),
@@ -1260,12 +1260,12 @@ extern "C" {
 
 int sfgpu_epic(sfgpu_ctx *c, image_t *flowx, image_t *flowy, const color_image_t *im, const float_image *input_matches, float_image *edges,
                const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    return epic_batch(c, 1, &flowx, &flowy, &im, &input_matches, &edges, params, stats, EpicCaller{"sfgpu_epic", nullptr, 0});
+    return epic_batch(c, 1, &flowx, &flowy, &im, &input_matches, &edges, params, stats, Caller{"sfgpu_epic", nullptr, 0});
 }
 
 int sfgpu_epic_batch(sfgpu_ctx *c, int n, image_t *const *flowx, image_t *const *flowy, const color_image_t *const *im,
                      const float_image *const *input_matches, float_image *const *edges, const epic_params_t *params, sfgpu_epic_stats_t *stats) {
-    return epic_batch(c, n, flowx, flowy, im, input_matches, edges, params, stats, EpicCaller{"sfgpu_epic_batch", "item", 0});
+    return epic_batch(c, n, flowx, flowy, im, input_matches, edges, params, stats, Caller{"sfgpu_epic_batch", "item", 0});
 }
 
 } // extern "C"

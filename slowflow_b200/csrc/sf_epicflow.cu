@@ -45,11 +45,6 @@ static void launch_rgb_to_lab(sfgpu_ctx *c, size_t P, const float *src, float *d
     c->prof_acc.kernel_launches++;
 }
 
-static bool planar(const color_image_t *im) {
-    const size_t P = (size_t)im->stride * im->height;
-    return im->c2 == im->c1 + P && im->c3 == im->c2 + P;
-}
-
 // Pairs per EPIC batch: the N at which the batch was measured (profiles/r3_epic_batch.md); EPIC's workspace takes about
 // 100 B per pixel per item, so a chunk of 2560x1440 pairs needs about 3 GB whatever n_pairs is.
 constexpr int EF_CHUNK = 8;
@@ -61,10 +56,9 @@ constexpr int EF_CHUNK = 8;
 // Device layout (the context's io area):
 //   frame ring: 2 * EF_CHUNK + 2 frames, frame f in slot f % R, so the frames of two consecutive chunks never share a slot
 //   Lab planes of one chunk | flows of two chunks (by chunk parity) | edge costs of two chunks (by chunk parity)
-static int run_epicflow(sfgpu_ctx *c, int n_pairs, const color_image_t *const *frames, const float_image *const *matches,
+static int run_epicflow(sfgpu_ctx *c, int n_pairs, Geom g, const color_image_t *const *frames, const float_image *const *matches,
                         float_image *const *edges, const epic_params_t *ep, const variational_params_t *vp, image_t *const *wx,
                         image_t *const *wy, sfgpu_epic_stats_t *stats) {
-    const Geom g{wx[0]->width, wx[0]->height, wx[0]->stride};
     const size_t P = g.plane(), N = (size_t)g.W * g.H;
     const int CH = EF_CHUNK, R = 2 * CH + 2, n_chunks = (n_pairs + CH - 1) / CH;
     const bool sal = ep->saliency_th != 0;
@@ -100,7 +94,7 @@ static int run_epicflow(sfgpu_ctx *c, int n_pairs, const color_image_t *const *f
         if ((status = pipe.wait(q, q - 2)) != SFGPU_OK) break;
         if (sal)
             for (int k = 0; k < m; k++) launch_rgb_to_lab(c, P, frame(j0 + k), lab + (size_t)k * 3 * P);
-        status = epic_device(c, m, g, costs(q), sal ? lab : nullptr, matches + j0, ep, flows(q), st.data(), EpicCaller{"sfgpu_epicflow_sequence", "pair", j0});
+        status = epic_device(c, m, g, costs(q), sal ? lab : nullptr, matches + j0, ep, flows(q), st.data(), Caller{"sfgpu_epicflow_sequence", "pair", j0});
         if (status != SFGPU_OK) break;
         if (stats)
             for (int k = 0; k < m; k++) stats[j0 + k] = st[k];
@@ -122,21 +116,14 @@ using namespace sf;
 extern "C" {
 
 int sfgpu_rgb_to_lab(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src) {
-    if (!c || !dst || !src || !dst->c1 || !src->c1) {
+    Geom g;
+    if (!c) {
         set_error("sfgpu_rgb_to_lab: null argument");
         return SFGPU_ERR_ARG;
     }
-    if (src->width < 1 || src->height < 1 || src->stride != ((src->width + 3) / 4) * 4 || dst->width != src->width ||
-        dst->height != src->height || dst->stride != src->stride) {
-        set_error("sfgpu_rgb_to_lab: dst and src must share width / height, stride = ceil4(width)");
-        return SFGPU_ERR_ARG;
-    }
-    if (!planar(src) || !planar(dst)) {
-        set_error("sfgpu_rgb_to_lab: colour images must be planar and contiguous (image.c:80-87)");
-        return SFGPU_ERR_ARG;
-    }
+    if (!arg_geom("sfgpu_rgb_to_lab: ", "src", src, g) || !arg_is("sfgpu_rgb_to_lab: ", "dst", dst, g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    const size_t P = (size_t)src->stride * src->height;
+    const size_t P = g.plane();
     int rc = c->ensure_io(6 * P);
     if (rc != SFGPU_OK) return rc;
     rc = host_copies(c, {{c->io, src->c1, 3 * P * sizeof(float)}}, true);
@@ -152,20 +139,19 @@ int sfgpu_rgb_to_lab(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src)
 int sfgpu_epicflow_sequence(sfgpu_ctx *c, int n_pairs, const color_image_t *const *frames, const float_image *const *matches,
                             float_image *const *edges, const epic_params_t *epic_params, const variational_params_t *flow_params,
                             image_t *const *wx, image_t *const *wy, sfgpu_epic_stats_t *stats) {
-    const EpicCaller who{"sfgpu_epicflow_sequence", "pair", 0};
+    const Caller who{"sfgpu_epicflow_sequence", "pair", 0};
     if (!c || n_pairs < 1 || !frames || !matches || !edges || !epic_params || !wx || !wy) {
         set_error("sfgpu_epicflow_sequence: bad argument (n_pairs >= 1, non-null context, arrays and epic_params)");
         return SFGPU_ERR_ARG;
     }
-    int rc = epic_check_args(c, n_pairs, wx, wy, frames, matches, edges, epic_params, who);
+    const char *const names[3] = {"wx", "wy", "frames[0]"};
+    Geom g;
+    int rc = epic_check_args(c, n_pairs, wx, wy, frames, matches, edges, epic_params, who, names, g);
     if (rc != SFGPU_OK) return rc;
-    for (int j = 0; j < n_pairs; j++)
-        if (!check_pair(wx[j], wy[j], frames[j], frames[j + 1])) {
-            set_error(who.at(j) + sfgpu_last_error());
-            return SFGPU_ERR_ARG;
-        }
+    for (int j = 0; j < n_pairs; j++) // frames[1..n_pairs], each under the first pair that reads it
+        if (!arg_is(who.at(j), "frames[" + std::to_string(j + 1) + "]", frames[j + 1], g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
-    return run_epicflow(c, n_pairs, frames, matches, edges, epic_params, flow_params, wx, wy, stats);
+    return run_epicflow(c, n_pairs, g, frames, matches, edges, epic_params, flow_params, wx, wy, stats);
 }
 
 } // extern "C"

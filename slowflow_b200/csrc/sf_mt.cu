@@ -887,22 +887,12 @@ int sfgpu_normalize(sfgpu_ctx *c, color_image_t *const *seq, int F, sf_mt_params
         set_error("sfgpu_normalize: bad argument");
         return SFGPU_ERR_ARG;
     }
-    for (int f = 0; f < F; f++) { // every frame like check_pair: same geometry, planar, contiguous
-        const color_image_t *q = seq[f];
-        if (!q || !q->c1 || q->width != seq[0]->width || q->height != seq[0]->height || q->stride != seq[0]->stride ||
-            q->stride != ((q->width + 3) / 4) * 4 || q->width < 1 || q->height < 1) {
-            set_error("sfgpu_normalize: frames must be non-null and share one geometry with stride = ceil4(width)");
-            return SFGPU_ERR_ARG;
-        }
-        const size_t Pq = (size_t)q->stride * q->height;
-        if (q->c2 != q->c1 + Pq || q->c3 != q->c2 + Pq) {
-            set_error("sfgpu_normalize: colour images must be planar and contiguous (image.c:80-87)");
-            return SFGPU_ERR_ARG;
-        }
-    }
+    Geom g;
+    if (!arg_geom("sfgpu_normalize: ", "seq[0]", seq[0], g)) return SFGPU_ERR_ARG;
+    for (int f = 1; f < F; f++)
+        if (!arg_is("sfgpu_normalize: ", "seq[" + std::to_string(f) + "]", seq[f], g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    const Geom g{seq[0]->width, seq[0]->height, seq[0]->stride};
     const size_t P = g.plane();
     // Short sequences (a window) stay resident between the two passes; long ones (a whole high-speed sequence, as the
     // sharded driver normalises it) are streamed through ONE frame-sized buffer twice, so device memory stays bounded.
@@ -976,20 +966,19 @@ int sfgpu_prescale_size(int width, int height, float scale, int *out_width, int 
 }
 
 int sfgpu_prescale(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src, float scale) {
-    if (!c || !dst || !src || !dst->c1 || !src->c1) {
+    if (!c) {
         set_error("sfgpu_prescale: null argument");
         return SFGPU_ERR_ARG;
     }
+    Geom gs;
+    if (!arg_geom("sfgpu_prescale: ", "src", src, gs)) return SFGPU_ERR_ARG;
     int dw = 0, dh = 0;
-    int rc = sfgpu_prescale_size(src->width, src->height, scale, &dw, &dh);
+    int rc = sfgpu_prescale_size(gs.W, gs.H, scale, &dw, &dh);
     if (rc != SFGPU_OK) return rc;
-    if (dst->width != dw || dst->height != dh || dst->stride != ((dw + 3) / 4) * 4 || src->stride != ((src->width + 3) / 4) * 4) {
-        set_error("sfgpu_prescale: dst must have the geometry sfgpu_prescale_size reports");
-        return SFGPU_ERR_ARG;
-    }
+    const Geom gd = make_geom(dw, dh); // what sfgpu_prescale_size reports
+    if (!arg_is("sfgpu_prescale: ", "dst", dst, gd)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    const Geom gs{src->width, src->height, src->stride}, gd{dw, dh, dst->stride};
     const size_t Ps = gs.plane(), Pd = gd.plane();
     rc = c->ensure_io(9 * Ps + 3 * Pd);
     if (rc != SFGPU_OK) return rc;
@@ -1008,13 +997,14 @@ int sfgpu_prescale(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src, f
 }
 
 int sfgpu_raw_weighting(sfgpu_ctx *c, color_image_t *weights, int red_x, int red_y, float weight) {
-    if (!c || !weights || !weights->c1 || weights->stride != ((weights->width + 3) / 4) * 4) {
+    Geom g;
+    if (!c) {
         set_error("sfgpu_raw_weighting: bad argument");
         return SFGPU_ERR_ARG;
     }
+    if (!arg_geom("sfgpu_raw_weighting: ", "weights", weights, g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    const Geom g{weights->width, weights->height, weights->stride};
     const size_t P = g.plane();
     int rc = c->ensure_io(3 * P);
     if (rc != SFGPU_OK) return rc;
@@ -1030,7 +1020,7 @@ int sfgpu_raw_weighting(sfgpu_ctx *c, color_image_t *weights, int red_x, int red
 int sfgpu_variational_mt(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_image_t *const *im,
                          const sf_mt_params_t *p, const color_image_t *channel_w, image_t *occlusions_out,
                          float avg_change_out[2]) {
-    if (!c || !wx || !wy || !im || !p) {
+    if (!c || !im || !p) {
         set_error("sfgpu_variational_mt: null argument");
         return SFGPU_ERR_ARG;
     }
@@ -1047,16 +1037,13 @@ int sfgpu_variational_mt(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_ima
         set_error("sfgpu_variational_mt: bad pyramid parameters");
         return SFGPU_ERR_ARG;
     }
-    const int W0 = wx->width, H0 = wx->height;
-    for (int f = 0; f < F; f++)
-        if (!im[f] || !im[f]->c1 || im[f]->width != W0 || im[f]->height != H0 || im[f]->stride != wx->stride) {
-            set_error("sfgpu_variational_mt: frames and flow must share one geometry");
-            return SFGPU_ERR_ARG;
-        }
-    if (wy->width != W0 || wy->height != H0 || wx->stride != ((W0 + 3) / 4) * 4) {
-        set_error("sfgpu_variational_mt: bad flow planes");
+    const char *at = "sfgpu_variational_mt: ";
+    Geom flow_g;
+    if (!arg_geom(at, "wx", wx, flow_g) || !arg_is(at, "wy", wy, flow_g) || (channel_w && !arg_is(at, "channel_w", channel_w, flow_g)) ||
+        (occlusions_out && occlusions_out->data && !arg_is(at, "occlusions_out", occlusions_out, flow_g)))
         return SFGPU_ERR_ARG;
-    }
+    for (int f = 0; f < F; f++)
+        if (!arg_is(at, "im[" + std::to_string(f) + "]", im[f], flow_g)) return SFGPU_ERR_ARG;
     SF_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     memset(&c->mt_stats, 0, sizeof(c->mt_stats));
@@ -1070,7 +1057,7 @@ int sfgpu_variational_mt(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_ima
     std::vector<Geom> geoms;
     int L = p->layers;
     for (int l = 0; l < L; l++) {
-        if (l == 0) geoms.push_back(make_geom(W0, H0));
+        if (l == 0) geoms.push_back(flow_g);
         else geoms.push_back(make_geom((int)floorf((float)geoms[l - 1].W * p->p_scale), (int)floorf((float)geoms[l - 1].H * p->p_scale)));
         if (floorf((float)geoms[l].W * p->p_scale) <= order + 1 || floorf((float)geoms[l].H * p->p_scale) <= order + 1) {
             L = l;
@@ -1234,7 +1221,7 @@ int sfgpu_variational_mt(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_ima
         std::vector<HostCopy> down;
         down.push_back(HostCopy{cur_x, wx->data, P0 * sizeof(float)});
         down.push_back(HostCopy{cur_y, wy->data, P0 * sizeof(float)});
-        if (occlusions_out && occlusions_out->data && occlusions_out->width == W0 && occlusions_out->height == H0)
+        if (occlusions_out && occlusions_out->data)
             down.push_back(HostCopy{occ, occlusions_out->data, P0 * sizeof(float)});
         const int rcd = host_copies(c, down, false);
         if (rcd != SFGPU_OK) return rcd;

@@ -62,10 +62,10 @@ static void launch_unpack(sfgpu_ctx *c, Geom g, const SeqFrames &src, int f, con
     c->prof_acc.kernel_launches++;
 }
 
-static int run_sequence(sfgpu_ctx *c, int n_pairs, const SeqFrames &src, image_t *const *wx, image_t *const *wy,
+// the arguments have been checked; g: their geometry
+static int run_sequence(sfgpu_ctx *c, int n_pairs, const SeqFrames &src, Geom g, image_t *const *wx, image_t *const *wy,
                         const variational_params_t *params, bool continue_from_previous) {
     SF_CUDA(cudaSetDevice(c->device));
-    const Geom g{wx[0]->width, wx[0]->height, wx[0]->stride};
     const size_t P = g.plane();
     const bool keep = continue_from_previous && c->seq_last_slot >= 0 && c->seq_geom.W == g.W && c->seq_geom.H == g.H;
     if (continue_from_previous && !keep) {
@@ -141,40 +141,35 @@ static int run_sequence(sfgpu_ctx *c, int n_pairs, const SeqFrames &src, image_t
     return status;
 }
 
-static bool check_flows(int n_pairs, image_t *const *wx, image_t *const *wy) {
-    for (int j = 0; j < n_pairs; j++) {
-        if (!wx[j] || !wy[j] || !wx[j]->data || !wy[j]->data) { set_error("sequence: null flow plane"); return false; }
-        if (wx[j]->stride != ((wx[j]->width + 3) / 4) * 4) { set_error("stride must be ceil4(width) (image.c:25)"); return false; }
-        if (wx[j]->width != wx[0]->width || wx[j]->height != wx[0]->height || wy[j]->width != wx[0]->width ||
-            wy[j]->height != wx[0]->height || wy[j]->stride != wx[0]->stride || wx[j]->stride != wx[0]->stride) {
-            set_error("sequence: all pairs must share one geometry");
-            return false;
-        }
-    }
-    return true;
-}
-
-static int sequence_int(sfgpu_ctx *c, int n_pairs, const sf_frame_int_t *frames, int depth, image_t *const *wx, image_t *const *wy,
-                        const variational_params_t *params, int continue_from_previous) {
-    if (!c || n_pairs < 0 || !frames || !wx || !wy) {
-        set_error("sfgpu_variational_sequence_u8/u16: bad argument");
+// The argument checks of the three entries, all before anything is touched: the flows' geometry from wx[0], every flow
+// plane, then frame f under the first pair that reads it.
+static int sequence(sfgpu_ctx *c, const char *fn, int n_pairs, const SeqFrames &src, image_t *const *wx, image_t *const *wy,
+                    const variational_params_t *params, int continue_from_previous) {
+    if (!c || n_pairs < 0 || !(src.f32 || src.ints) || !wx || !wy) {
+        set_error(std::string(fn) + ": bad argument");
         return SFGPU_ERR_ARG;
     }
     if (n_pairs == 0) return SFGPU_OK;
-    if (!check_flows(n_pairs, wx, wy)) return SFGPU_ERR_ARG;
-    const size_t sample = depth / 8;
+    const Caller who{fn, "pair", 0};
+    Geom g;
+    if (!arg_geom(who.at(0), "wx", wx[0], g)) return SFGPU_ERR_ARG;
+    for (int j = 0; j < n_pairs; j++)
+        if (!arg_is(who.at(j), "wx", wx[j], g) || !arg_is(who.at(j), "wy", wy[j], g)) return SFGPU_ERR_ARG;
+    const size_t sample = src.depth / 8;
     for (int f = 0; f <= n_pairs; f++) {
-        const sf_frame_int_t &q = frames[f];
-        if (!q.data || q.width != wx[0]->width || q.height != wx[0]->height || (q.channels != 1 && q.channels != 3) ||
+        const std::string at = who.at(std::max(f - 1, 0)), name = "frames[" + std::to_string(f) + "]";
+        if (src.f32) {
+            if (!arg_is(at, name, src.f32[f], g)) return SFGPU_ERR_ARG;
+            continue;
+        }
+        const sf_frame_int_t &q = src.ints[f];
+        if (!q.data || q.width != g.W || q.height != g.H || (q.channels != 1 && q.channels != 3) ||
             q.step < (size_t)q.width * q.channels * sample || (q.step % sample) != 0) {
-            set_error("sequence: integer frames must match the flow geometry, have 1 or 3 channels and step >= width*channels*bytes");
+            set_error(at + name + ": integer frames must match the flow geometry, have 1 or 3 channels and step >= width*channels*bytes");
             return SFGPU_ERR_ARG;
         }
     }
-    SeqFrames src;
-    src.ints = frames;
-    src.depth = depth;
-    return run_sequence(c, n_pairs, src, wx, wy, params, continue_from_previous != 0);
+    return run_sequence(c, n_pairs, src, g, wx, wy, params, continue_from_previous != 0);
 }
 
 } // namespace sf
@@ -185,27 +180,17 @@ extern "C" {
 
 int sfgpu_variational_sequence(sfgpu_ctx *c, int n_pairs, const color_image_t *const *frames, image_t *const *wx,
                                image_t *const *wy, const variational_params_t *params) {
-    if (!c || n_pairs < 0 || !frames || !wx || !wy) {
-        set_error("sfgpu_variational_sequence: bad argument");
-        return SFGPU_ERR_ARG;
-    }
-    if (n_pairs == 0) return SFGPU_OK;
-    for (int j = 0; j < n_pairs; j++)
-        if (!check_pair(wx[j], wy[j], frames[j], frames[j + 1])) return SFGPU_ERR_ARG;
-    if (!check_flows(n_pairs, wx, wy)) return SFGPU_ERR_ARG;
-    SeqFrames src;
-    src.f32 = frames;
-    return run_sequence(c, n_pairs, src, wx, wy, params, false);
+    return sequence(c, "sfgpu_variational_sequence", n_pairs, SeqFrames{frames}, wx, wy, params, 0);
 }
 
 int sfgpu_variational_sequence_u8(sfgpu_ctx *c, int n_pairs, const sf_frame_int_t *frames, image_t *const *wx, image_t *const *wy,
                                   const variational_params_t *params, int continue_from_previous) {
-    return sequence_int(c, n_pairs, frames, 8, wx, wy, params, continue_from_previous);
+    return sequence(c, "sfgpu_variational_sequence_u8", n_pairs, SeqFrames{nullptr, frames, 8}, wx, wy, params, continue_from_previous);
 }
 
 int sfgpu_variational_sequence_u16(sfgpu_ctx *c, int n_pairs, const sf_frame_int_t *frames, image_t *const *wx, image_t *const *wy,
                                    const variational_params_t *params, int continue_from_previous) {
-    return sequence_int(c, n_pairs, frames, 16, wx, wy, params, continue_from_previous);
+    return sequence(c, "sfgpu_variational_sequence_u16", n_pairs, SeqFrames{nullptr, frames, 16}, wx, wy, params, continue_from_previous);
 }
 
 } // extern "C"
