@@ -281,6 +281,17 @@ int sfgpu_prep_two_frame(sfgpu_ctx *ctx, image_t *a11, image_t *a12, image_t *a2
                          const color_image_t *im1, const color_image_t *im2, const image_t *wx, const image_t *wy,
                          const image_t *du, const image_t *dv, const image_t *dpsis_horiz, const image_t *dpsis_vert,
                          float half_delta_over3, float half_gamma_over3);
+/* The multi-frame path's linear system as an operator: one linearisation of compute_one_level (variational_mt.cpp:289-365)
+ * on the frames im[0 .. 2(S-1)] of one level -- warps, derivatives, the occlusion factor of occ (-1 / 0 / +1), smoothness
+ * on uu = wx + du, every data term and the Laplacian -- through the production kernels the context's switches select,
+ * followed by the block inverse of the SOR's first sweep.  du, dv may be NULL (first inner iteration); channel_w may be
+ * NULL.  Whole planes are written, stride padding included. */
+int sfgpu_mt_system(sfgpu_ctx *ctx, image_t *a11, image_t *a12, image_t *a22, image_t *b1, image_t *b2, image_t *psi_h,
+                    image_t *psi_v, const color_image_t *const *im, const image_t *wx, const image_t *wy, const image_t *du,
+                    const image_t *dv, const image_t *occ, const color_image_t *channel_w, const sf_mt_params_t *params);
+/* The data costs of the occlusion labelling (variational_aux_mt.cpp:786-848) at (wx, wy): d0 / d1 of the W x H pixels. */
+int sfgpu_mt_occ_costs(sfgpu_ctx *ctx, image_t *d0, image_t *d1, const color_image_t *const *im, const image_t *wx,
+                       const image_t *wy, const sf_mt_params_t *params);
 /* variational_aux.c:153 */
 int sfgpu_sub_laplacian(sfgpu_ctx *ctx, image_t *dst, const image_t *src, const image_t *weight_horiz,
                         const image_t *weight_vert);

@@ -59,6 +59,10 @@ class Oracle:
             L.sfo_variational_mt.argtypes = [IP, IP, C.POINTER(CP), C.POINTER(MTParams), CP, IP,
                                              C.POINTER(C.c_float), C.c_int, C.POINTER(C.c_int)]
             L.sfo_normalize.argtypes = [C.POINTER(CP), C.c_int, C.POINTER(MTParams)]
+            L.sfo_mt_smoothness.argtypes = [IP] * 5 + [C.c_float, C.c_int, C.c_int, C.c_float, C.c_float]
+            L.sfo_mt_dpsis_weight.argtypes = [IP, CP, C.c_float, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]
+            L.sfo_mt_system.argtypes = [IP] * 7 + [C.POINTER(CP)] + [IP] * 5 + [CP, C.POINTER(MTParams)]
+            L.sfo_mt_occ_costs.argtypes = [IP, IP, C.POINTER(CP), IP, IP, C.POINTER(MTParams)]
 
     def variational(self, wx, wy, im1, im2, params=None, sor_mode=SOR_LEX):
         self.lib.sfo_variational(wx.ptr(), wy.ptr(), im1.ptr(), im2.ptr(),

@@ -400,14 +400,22 @@ void dpsis_mt(const CImg *im, Img *lum, float coef, const float avg[3], const fl
     sfo_image_delete(ly);
 }
 
-/* optimizeOcc (variational_aux_mt.cpp:758-887) with the exact binary min-cut standing in for gco's expansion */
-void optimize_occ(Img *occ, Img **mask, DerivSet *succ, DerivSet *toref, int ref, const float *rho, const float *omega, float delta_over3,
-                  float gamma_over3, float penalty, float alpha, const Pen &pc, const Pen &pg, bool int_terms) {
-    const int W = occ->width, H = occ->height, S = occ->stride;
+/* the colour, gradient and regularisation penalties of a parameter set (select_robust_function,
+ * variational_aux_mt.cpp:889-926); robust_grad < 0 reuses the colour penalty */
+struct Pens {
+    Pen pc, pg, preg;
+    explicit Pens(const sfo_mt_params_t *p)
+        : pc(p->robust_color, p->robust_color_eps, p->robust_color_truncation),
+          pg(p->robust_grad >= 0 ? Pen(p->robust_grad, p->robust_grad_eps, p->robust_grad_truncation) : pc),
+          preg(p->robust_reg, p->robust_reg_eps, p->robust_reg_truncation) {}
+};
+
+/* data costs of the two occlusion labels (variational_aux_mt.cpp:786-848) from the raw masks and the derivatives of
+ * get_derivatives: d0 / d1 at the pixels of the occ plane's geometry */
+void occ_costs(Img *d0, Img *d1, Img *const *mask, const DerivSet *succ, const DerivSet *toref, int ref, const float *rho, const float *omega,
+               float delta_over3, float gamma_over3, float penalty, const Pen &pc, const Pen &pg) {
+    const int W = d0->width, H = d0->height, S = d0->stride;
     const size_t P = (size_t)S * H;
-    sfo::GridCut gc(W, H);
-    auto q = [&](double e) -> int64_t { return (int64_t)llround((int_terms ? (double)(int)e : e) * 16777216.0); };
-    const int64_t pair = q((double)alpha);
     for (int y = 0; y < H; y++)
         for (int x = 0; x < W; x++) {
             const size_t k = (size_t)y * S + x;
@@ -433,36 +441,113 @@ void optimize_occ(Img *occ, Img **mask, DerivSet *succ, DerivSet *toref, int ref
                 if (nrm[l] == 0) nrm[l] = 1;
                 d[l] = 0.01f * e[l] / nrm[l] + penalty * l;
             }
+            d0->data[k] = d[0];
+            d1->data[k] = d[1];
+        }
+}
+
+/* optimizeOcc (variational_aux_mt.cpp:758-887) with the exact binary min-cut standing in for gco's expansion */
+void optimize_occ(Img *occ, Img **mask, DerivSet *succ, DerivSet *toref, int ref, const float *rho, const float *omega, float delta_over3,
+                  float gamma_over3, float penalty, float alpha, const Pen &pc, const Pen &pg, bool int_terms) {
+    const int W = occ->width, H = occ->height, S = occ->stride;
+    Img *d0 = sfo_image_new(W, H), *d1 = sfo_image_new(W, H);
+    occ_costs(d0, d1, mask, succ, toref, ref, rho, omega, delta_over3, gamma_over3, penalty, pc, pg);
+    sfo::GridCut gc(W, H);
+    auto q = [&](double e) -> int64_t { return (int64_t)llround((int_terms ? (double)(int)e : e) * 16777216.0); };
+    const int64_t pair = q((double)alpha);
+    for (int y = 0; y < H; y++)
+        for (int x = 0; x < W; x++) {
+            const size_t k = (size_t)y * S + x;
             const int p = y * W + x;
-            gc.set_terminal(p, q((double)d[1]), q((double)d[0]));
+            gc.set_terminal(p, q((double)d1->data[k]), q((double)d0->data[k]));
             if (x + 1 < W) gc.set_edge_right(p, pair);
             if (y + 1 < H) gc.set_edge_down(p, pair);
         }
+    sfo_image_delete(d0);
+    sfo_image_delete(d1);
     gc.maxflow();
     for (int y = 0; y < H; y++)
         for (int x = 0; x < W; x++) occ->data[(size_t)y * S + x] = (float)(2 * gc.label(y * W + x) - 1);
 }
 
+/* the occlusion / window factor of variational_mt.cpp:293-320, applied in place to the raw masks of get_derivatives */
+void occ_factor(Img *const *mask, const Img *occ, const sfo_mt_params_t *p) {
+    const int ref = p->S - 1;
+    const bool one_direction = p->one_direction != 0;
+    const size_t n = (size_t)occ->stride * occ->height;
+    float data_norm = 0;
+    for (int s = 0; s < ref; s++) data_norm += p->rho[s] + p->omega[s];
+    for (size_t k = 0; k < n; k++) {
+        const float oc = occ->data[k];
+        const float fac = (1 + ((oc == 0) ? 1.0f : 0.0f)) * data_norm;
+        const float backward = ((oc >= 0) ? 1.0f : 0.0f) / fac, forward = ((oc <= 0) ? 1.0f : 0.0f) / fac;
+        for (int s = one_direction ? ref : 0; s < 2 * ref; s++)
+            mask[s]->data[k] = (s < ref) ? (1.0f * backward * mask[s]->data[k]) : (1.0f * forward * mask[s]->data[k]);
+    }
+}
+
+/* one linearisation up to the SOR (variational_mt.cpp:333-365): smoothness weights of (uu, vv), every data term of
+ * :343-361 at the increment (du, dv) on the factored masks, b -= div(psi grad uu), b -= div(psi grad vv).  The blocks are
+ * left as sor_coupled takes them (not inverted). */
+void assemble_system(Sys &A, Img *sh, Img *sv, Img *const *mask, const Img *du, const Img *dv, const DerivSet *succ, const DerivSet *toref,
+                     const Img *uu, const Img *vv, const Img *dpsis, const CImg *cw, const sfo_mt_params_t *p, const Pens &pen) {
+    const int ref = p->S - 1;
+    const size_t n = (size_t)uu->stride * uu->height;
+    const bool one_direction = p->one_direction != 0, dt_norm = p->dataterm != 0;
+    const float gamma_over3 = p->gamma / 3.0f, delta_over3 = p->delta / 3.0f;
+    smoothness_mt(p->smoothing, sh, sv, uu, vv, dpsis, p->alpha, pen.preg);
+    memset(A.a11->data, 0, n * sizeof(float)); memset(A.a12->data, 0, n * sizeof(float)); memset(A.a22->data, 0, n * sizeof(float));
+    memset(A.b1->data, 0, n * sizeof(float)); memset(A.b2->data, 0, n * sizeof(float));
+    for (int s = 0; s < ref; s++) { /* :343-361 */
+        if (!one_direction) {
+            if (p->rho[ref - 1 - s] > 0)
+                add_succ(A, mask[s], du, dv, succ[s], cw, p->rho[ref - 1 - s] * delta_over3, p->rho[ref - 1 - s] * gamma_over3, (float)(s - ref), dt_norm, pen.pc, pen.pg);
+            if (p->omega[ref - 1 - s] > 0)
+                add_ref(A, mask[s], du, dv, toref[s], cw, p->omega[ref - 1 - s] * delta_over3, p->omega[ref - 1 - s] * gamma_over3, (float)(s - ref), dt_norm, pen.pc, pen.pg);
+        }
+        if (p->rho[s] > 0)
+            add_succ(A, mask[ref + s], du, dv, succ[ref + s], cw, p->rho[s] * delta_over3, p->rho[s] * gamma_over3, (float)s, dt_norm, pen.pc, pen.pg);
+        if (p->omega[s] > 0)
+            add_ref(A, mask[ref + s], du, dv, toref[ref + s], cw, p->omega[s] * delta_over3, p->omega[s] * gamma_over3, (float)(s + 1), dt_norm, pen.pc, pen.pg);
+    }
+    sfo_sub_laplacian(A.b1, uu, sh, sv);
+    sfo_sub_laplacian(A.b2, vv, sh, sv);
+}
+
+/* the per-frame planes of one level's get_derivatives */
+struct LevelPlanes {
+    std::vector<Img *> mask;
+    std::vector<DerivSet> succ, toref;
+    CImg *ws, *wsp1;
+    LevelPlanes(int W, int H, int ref) : mask(2 * ref), succ(2 * ref), toref(2 * ref) {
+        for (int s = 0; s < 2 * ref; s++) { mask[s] = sfo_image_new(W, H); succ[s] = new_set(W, H); toref[s] = new_set(W, H); }
+        ws = sfo_color_image_new(W, H);
+        wsp1 = sfo_color_image_new(W, H);
+    }
+    ~LevelPlanes() {
+        sfo_color_image_delete(ws); sfo_color_image_delete(wsp1);
+        for (size_t s = 0; s < mask.size(); s++) { sfo_image_delete(mask[s]); free_set(succ[s]); free_set(toref[s]); }
+    }
+    void derivatives(CImg *const *im, const Img *wx, const Img *wy, int ref, bool one_direction) {
+        get_derivatives(im, wx, wy, ws, wsp1, mask.data(), succ.data(), toref.data(), ref, one_direction);
+    }
+};
+
 struct LevelOut { float cx, cy; int outer_its, gco_calls; };
 
 /* Variational_MT::compute_one_level (variational_mt.cpp:169-493) */
 LevelOut compute_one_level(Img *wx, Img *wy, CImg *const *im, const sfo_mt_params_t *p, const CImg *cw, Img *occ_out, int sor_mode,
-                           const Pen &pc, const Pen &pg, const Pen &preg) {
+                           const Pens &pen) {
     const int W = wx->width, H = wx->height, S = wx->stride, ref = p->S - 1;
     const size_t n = (size_t)S * H;
     const bool one_direction = p->one_direction != 0;
-    const float alpha = p->alpha, gamma_over3 = p->gamma / 3.0f, delta_over3 = p->delta / 3.0f;
+    const float gamma_over3 = p->gamma / 3.0f, delta_over3 = p->delta / 3.0f;
     Img *du = sfo_image_new(W, H), *dv = sfo_image_new(W, H), *odu = sfo_image_new(W, H), *odv = sfo_image_new(W, H),
         *sh = sfo_image_new(W, H), *sv = sfo_image_new(W, H), *uu = sfo_image_new(W, H), *vv = sfo_image_new(W, H);
     Sys A = {sfo_image_new(W, H), sfo_image_new(W, H), sfo_image_new(W, H), sfo_image_new(W, H), sfo_image_new(W, H)};
-    std::vector<Img *> mask(2 * ref);
-    std::vector<DerivSet> succ(2 * ref), toref(2 * ref);
-    for (int s = 0; s < 2 * ref; s++) { mask[s] = sfo_image_new(W, H); succ[s] = new_set(W, H); toref[s] = new_set(W, H); }
-    CImg *ws = sfo_color_image_new(W, H), *wsp1 = sfo_color_image_new(W, H);
+    LevelPlanes lp(W, H, ref);
     Img *occ = sfo_image_new(W, H);
     if (one_direction || p->occlusion_reasoning) std::fill_n(occ->data, n, -1.0f);
-    float data_norm = 0;
-    for (int s = 0; s < ref; s++) data_norm += p->rho[s] + p->omega[s];
     Img *dpsis = sfo_image_new(W, H);
     dpsis_mt(im[ref], dpsis, 5.0f, p->img_norm_avg, p->img_norm_std, p->hbit != 0);
     memcpy(uu->data, wx->data, n * sizeof(float));
@@ -470,44 +555,22 @@ LevelOut compute_one_level(Img *wx, Img *wy, CImg *const *im, const sfo_mt_param
     LevelOut out = {0, 0, 0, 0};
 
     for (int alter = 0; alter < p->niter_alter; alter++) {
-        get_derivatives(im, wx, wy, ws, wsp1, mask.data(), succ.data(), toref.data(), ref, one_direction);
+        lp.derivatives(im, wx, wy, ref, one_direction);
         if (alter > 0 && p->occlusion_reasoning && !one_direction) {
-            optimize_occ(occ, mask.data(), succ.data(), toref.data(), ref, p->rho, p->omega, delta_over3, gamma_over3, p->occlusion_penalty,
-                         p->occlusion_alpha, pc, pg, p->graphcut_int_terms != 0);
+            optimize_occ(occ, lp.mask.data(), lp.succ.data(), lp.toref.data(), ref, p->rho, p->omega, delta_over3, gamma_over3,
+                         p->occlusion_penalty, p->occlusion_alpha, pen.pc, pen.pg, p->graphcut_int_terms != 0);
             out.gco_calls++;
         }
         for (int outer = 0; outer < p->niter_outer; outer++) {
-            if (outer > 0) get_derivatives(im, wx, wy, ws, wsp1, mask.data(), succ.data(), toref.data(), ref, one_direction);
+            if (outer > 0) lp.derivatives(im, wx, wy, ref, one_direction);
             out.outer_its++;
-            for (size_t k = 0; k < n; k++) { /* :293-320 */
-                const float oc = occ->data[k];
-                const float fac = (1 + ((oc == 0) ? 1.0f : 0.0f)) * data_norm;
-                const float backward = ((oc >= 0) ? 1.0f : 0.0f) / fac, forward = ((oc <= 0) ? 1.0f : 0.0f) / fac;
-                for (int s = one_direction ? ref : 0; s < 2 * ref; s++)
-                    mask[s]->data[k] = (s < ref) ? (1.0f * backward * mask[s]->data[k]) : (1.0f * forward * mask[s]->data[k]);
-            }
+            occ_factor(lp.mask.data(), occ, p);
             memset(du->data, 0, n * sizeof(float));
             memset(dv->data, 0, n * sizeof(float));
             for (int inner = 0; inner < p->niter_inner; inner++) {
                 memcpy(odu->data, du->data, n * sizeof(float));
                 memcpy(odv->data, dv->data, n * sizeof(float));
-                smoothness_mt(p->smoothing, sh, sv, uu, vv, dpsis, alpha, preg);
-                memset(A.a11->data, 0, n * sizeof(float)); memset(A.a12->data, 0, n * sizeof(float)); memset(A.a22->data, 0, n * sizeof(float));
-                memset(A.b1->data, 0, n * sizeof(float)); memset(A.b2->data, 0, n * sizeof(float));
-                for (int s = 0; s < ref; s++) { /* :343-361 */
-                    if (!one_direction) {
-                        if (p->rho[ref - 1 - s] > 0)
-                            add_succ(A, mask[s], du, dv, succ[s], cw, p->rho[ref - 1 - s] * delta_over3, p->rho[ref - 1 - s] * gamma_over3, (float)(s - ref), p->dataterm != 0, pc, pg);
-                        if (p->omega[ref - 1 - s] > 0)
-                            add_ref(A, mask[s], du, dv, toref[s], cw, p->omega[ref - 1 - s] * delta_over3, p->omega[ref - 1 - s] * gamma_over3, (float)(s - ref), p->dataterm != 0, pc, pg);
-                    }
-                    if (p->rho[s] > 0)
-                        add_succ(A, mask[ref + s], du, dv, succ[ref + s], cw, p->rho[s] * delta_over3, p->rho[s] * gamma_over3, (float)s, p->dataterm != 0, pc, pg);
-                    if (p->omega[s] > 0)
-                        add_ref(A, mask[ref + s], du, dv, toref[ref + s], cw, p->omega[s] * delta_over3, p->omega[s] * gamma_over3, (float)(s + 1), p->dataterm != 0, pc, pg);
-                }
-                sfo_sub_laplacian(A.b1, uu, sh, sv);
-                sfo_sub_laplacian(A.b2, vv, sh, sv);
+                assemble_system(A, sh, sv, lp.mask.data(), du, dv, lp.succ.data(), lp.toref.data(), uu, vv, dpsis, cw, p, pen);
                 sfo_sor_coupled(du, dv, A.a11, A.a12, A.a22, A.b1, A.b2, sh, sv, p->niter_solver, p->sor_omega, sor_mode);
                 float ch_du = 0, ch_dv = 0; /* :376-402: float accumulators, |.| of each group of 4 summed left to right in float */
                 for (int j = 0; j < H; j++)
@@ -552,8 +615,6 @@ LevelOut compute_one_level(Img *wx, Img *wy, CImg *const *im, const sfo_mt_param
     sfo_image_delete(du); sfo_image_delete(dv); sfo_image_delete(odu); sfo_image_delete(odv); sfo_image_delete(sh); sfo_image_delete(sv);
     sfo_image_delete(uu); sfo_image_delete(vv); sfo_image_delete(A.a11); sfo_image_delete(A.a12); sfo_image_delete(A.a22);
     sfo_image_delete(A.b1); sfo_image_delete(A.b2); sfo_image_delete(dpsis); sfo_image_delete(occ);
-    sfo_color_image_delete(ws); sfo_color_image_delete(wsp1);
-    for (int s = 0; s < 2 * ref; s++) { sfo_image_delete(mask[s]); free_set(succ[s]); free_set(toref[s]); }
     return out;
 }
 
@@ -696,6 +757,72 @@ int sfo_mincut(int w, int h, const float *d0, const float *d1, float alpha, int 
     return 0;
 }
 
+/* ---- operator entries: the functions compute_one_level and optimize_occ are made of, on one level's planes */
+
+/* Variational_AUX_MT::compute_smoothness, modes 0 and 1; robust_reg < 0 is not a reference penalty */
+int sfo_mt_smoothness(sfo_image_t *dh, sfo_image_t *dv, const sfo_image_t *uu, const sfo_image_t *vv, const sfo_image_t *w, float alpha,
+                      int mode, int robust_reg, float eps, float trunc) {
+    if (mode < 0 || mode > 1 || robust_reg < 0) return 1;
+    smoothness_mt(mode, dh, dv, uu, vv, w, alpha, Pen(robust_reg, eps, trunc));
+    return 0;
+}
+
+/* compute_dpsis_weight of the de-normalised luminance (variational_aux_mt.cpp:673-719) */
+int sfo_mt_dpsis_weight(sfo_image_t *dst, const sfo_color_image_t *im, float coef, const float avg3[3], const float std3[3], int hbit) {
+    dpsis_mt(im, dst, coef, avg3, std3, hbit != 0);
+    return 0;
+}
+
+/* One linearisation of compute_one_level up to the SOR: get_derivatives of the level frames im[0 .. 2(S-1)] at (wx, wy),
+ * the occlusion / window factor of occ on the masks, smoothness on uu = wx + du, every data term at the increment
+ * (du, dv) (NULL: zero, the first inner iteration) and the Laplacian of uu, vv subtracted from b.  The blocks are left
+ * as sfo_sor_coupled takes them; channel_w NULL means all-ones weights. */
+int sfo_mt_system(sfo_image_t *a11, sfo_image_t *a12, sfo_image_t *a22, sfo_image_t *b1, sfo_image_t *b2, sfo_image_t *psi_h,
+                  sfo_image_t *psi_v, sfo_color_image_t *const *im, const sfo_image_t *wx, const sfo_image_t *wy, const sfo_image_t *du,
+                  const sfo_image_t *dv, const sfo_image_t *occ, const sfo_color_image_t *channel_w, const sfo_mt_params_t *p) {
+    const int W = wx->width, H = wx->height, ref = p->S - 1;
+    if (ref < 1 || ref > SF_MT_MAX_REF || p->smoothing < 0 || p->smoothing > 1 || (du == NULL) != (dv == NULL)) return 1;
+    const size_t n = (size_t)wx->stride * H;
+    const Pens pen(p);
+    CImg *ones = NULL;
+    if (!channel_w) {
+        ones = sfo_color_image_new(W, H);
+        std::fill_n(ones->c1, 3 * n, 1.0f);
+        channel_w = ones;
+    }
+    Img *zu = sfo_image_new(W, H), *zv = sfo_image_new(W, H), *uu = sfo_image_new(W, H), *vv = sfo_image_new(W, H);
+    Img *dpsis = sfo_image_new(W, H);
+    memset(zu->data, 0, n * sizeof(float));
+    memset(zv->data, 0, n * sizeof(float));
+    if (!du) { du = zu; dv = zv; }
+    for (size_t k = 0; k < n; k++) { uu->data[k] = wx->data[k] + du->data[k]; vv->data[k] = wy->data[k] + dv->data[k]; }
+    dpsis_mt(im[ref], dpsis, 5.0f, p->img_norm_avg, p->img_norm_std, p->hbit != 0);
+    {
+        LevelPlanes lp(W, H, ref);
+        lp.derivatives(im, wx, wy, ref, p->one_direction != 0);
+        occ_factor(lp.mask.data(), occ, p);
+        Sys A = {a11, a12, a22, b1, b2};
+        assemble_system(A, psi_h, psi_v, lp.mask.data(), du, dv, lp.succ.data(), lp.toref.data(), uu, vv, dpsis, channel_w, p, pen);
+    }
+    sfo_image_delete(zu); sfo_image_delete(zv); sfo_image_delete(uu); sfo_image_delete(vv); sfo_image_delete(dpsis);
+    if (ones) sfo_color_image_delete(ones);
+    return 0;
+}
+
+/* The cost half of optimizeOcc: get_derivatives of the level frames at (wx, wy) in both directions, then the data costs
+ * d0 / d1 of the two labels at every pixel (the stride padding is not written) */
+int sfo_mt_occ_costs(sfo_image_t *d0, sfo_image_t *d1, sfo_color_image_t *const *im, const sfo_image_t *wx, const sfo_image_t *wy,
+                     const sfo_mt_params_t *p) {
+    const int ref = p->S - 1;
+    if (ref < 1 || ref > SF_MT_MAX_REF) return 1;
+    const Pens pen(p);
+    LevelPlanes lp(wx->width, wx->height, ref);
+    lp.derivatives(im, wx, wy, ref, false);
+    occ_costs(d0, d1, lp.mask.data(), lp.succ.data(), lp.toref.data(), ref, p->rho, p->omega, p->delta / 3.0f, p->gamma / 3.0f,
+              p->occlusion_penalty, pen.pc, pen.pg);
+    return 0;
+}
+
 /* normalize (variational_mt.cpp:17-85) */
 int sfo_normalize(sfo_color_image_t *const *seq, int F, sfo_mt_params_t *p) {
     double avg[3] = {0, 0, 0}, sd[3] = {0, 0, 0};
@@ -739,9 +866,7 @@ int sfo_variational_mt(sfo_image_t *wx, sfo_image_t *wy, sfo_color_image_t *cons
                        const sfo_color_image_t *channel_w, sfo_image_t *occlusions_out, float avg_change[2], int sor_mode, int *stats) {
     const int ref = p->S - 1, F = 2 * ref + 1;
     int L = p->layers;
-    const Pen pc(p->robust_color, p->robust_color_eps, p->robust_color_truncation);
-    const Pen pg = (p->robust_grad >= 0) ? Pen(p->robust_grad, p->robust_grad_eps, p->robust_grad_truncation) : pc;
-    const Pen preg(p->robust_reg, p->robust_reg_eps, p->robust_reg_truncation);
+    const Pens pen(p);
     CImg *ones = NULL;
     const CImg *cw = channel_w;
     if (!cw) {
@@ -801,7 +926,7 @@ int sfo_variational_mt(sfo_image_t *wx, sfo_image_t *wy, sfo_color_image_t *cons
                 wxl = wx; wyl = wy;
             }
         }
-        last = compute_one_level(wxl, wyl, pyr[l].data(), p, cw, l == 0 ? occlusions_out : NULL, sor_mode, pc, pg, preg);
+        last = compute_one_level(wxl, wyl, pyr[l].data(), p, cw, l == 0 ? occlusions_out : NULL, sor_mode, pen);
         outer_total += last.outer_its;
         gco_total += last.gco_calls;
     }

@@ -63,7 +63,7 @@ ABI_SYMBOLS = [
     "sfgpu_variational_sequence_u16", "sfgpu_host_register",
     "sfgpu_host_unregister", "sfgpu_variational_mt", "sfgpu_mt_frame_cache", "sfgpu_normalize", "sfgpu_get_mt_stats", "sfgpu_profile_enable",
     "sfgpu_profile_reset", "sfgpu_profile_get", "sfgpu_image_warp", "sfgpu_warp_frame_derivs", "sfgpu_compute_dpsis_weight",
-    "sfgpu_compute_smoothness", "sfgpu_compute_data_and_match", "sfgpu_prep_two_frame", "sfgpu_sub_laplacian", "sfgpu_sor_coupled",
+    "sfgpu_compute_smoothness", "sfgpu_compute_data_and_match", "sfgpu_prep_two_frame", "sfgpu_mt_system", "sfgpu_mt_occ_costs", "sfgpu_sub_laplacian", "sfgpu_sor_coupled",
     "sfgpu_epic", "sfgpu_epic_batch", "sfgpu_epic_nnfield", "sfgpu_rgb_to_lab", "sfgpu_epicflow_sequence", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
     "sfgpu_write_flo", "sfgpu_read_flo_size", "sfgpu_read_flo", "sfgpu_write_occlusion_pbm", "sfgpu_set_device", "sfgpu_get_device",
     "sfgpu_convolve_horiz", "sfgpu_convolve_vert", "sfgpu_color_image_convolve_hv", "sfgpu_get_derivatives",
@@ -119,6 +119,8 @@ def load_library(path=None):
     lib.sfgpu_compute_data_and_match.argtypes = [C.c_void_p, IP, IP, IP, IP, IP, IP, IP, IP, CP, CP, C.c_float,
                                                  C.c_float]
     lib.sfgpu_prep_two_frame.argtypes = [C.c_void_p, IP, IP, IP, IP, IP, CP, CP, IP, IP, IP, IP, IP, IP, C.c_float, C.c_float]
+    lib.sfgpu_mt_system.argtypes = [C.c_void_p] + [IP] * 7 + [C.POINTER(CP)] + [IP] * 5 + [CP, C.POINTER(MTParams)]
+    lib.sfgpu_mt_occ_costs.argtypes = [C.c_void_p, IP, IP, C.POINTER(CP), IP, IP, C.POINTER(MTParams)]
     lib.sfgpu_sub_laplacian.argtypes = [C.c_void_p, IP, IP, IP, IP]
     lib.sfgpu_sor_coupled.argtypes = [C.c_void_p, IP, IP, IP, IP, IP, IP, IP, IP, IP, C.c_int, C.c_float]
     lib.sfgpu_prescale_size.argtypes = [C.c_int, C.c_int, C.c_float, C.POINTER(C.c_int), C.POINTER(C.c_int)]
@@ -416,6 +418,24 @@ class Context:
         _check(self.lib, self.lib.sfgpu_prep_two_frame(self.h, a11.ptr(), a12.ptr(), a22.ptr(), b1.ptr(), b2.ptr(), im1.ptr(),
                                                        im2.ptr(), wx.ptr(), wy.ptr(), _ip(du), _ip(dv), ph.ptr(), pv.ptr(), hd, hg),
                "sfgpu_prep_two_frame")
+
+    def mt_system(self, im, wx, wy, params, occ, du=None, dv=None, channel_w=None):
+        """One linearisation of the multi-frame solver on one level's frames -> [a11, a12, a22, b1, b2] (blocks inverted)
+        and [psi_h, psi_v], whole planes (sfgpu_mt_system)."""
+        w, h = wx.width, wx.height
+        outs = [Image(w, h) for _ in range(7)]
+        arr = (C.POINTER(color_image_t) * len(im))(*[C.pointer(f.c) for f in im])
+        _check(self.lib, self.lib.sfgpu_mt_system(self.h, *[o.ptr() for o in outs], arr, wx.ptr(), wy.ptr(), _ip(du), _ip(dv),
+                                                  occ.ptr(), _ip(channel_w), C.byref(params)), "sfgpu_mt_system")
+        return outs[:5], outs[5:]
+
+    def mt_occ_costs(self, im, wx, wy, params):
+        """Occlusion data costs (d0, d1) of one level's frames at (wx, wy) (sfgpu_mt_occ_costs)."""
+        d0, d1 = Image(wx.width, wx.height), Image(wx.width, wx.height)
+        arr = (C.POINTER(color_image_t) * len(im))(*[C.pointer(f.c) for f in im])
+        _check(self.lib, self.lib.sfgpu_mt_occ_costs(self.h, d0.ptr(), d1.ptr(), arr, wx.ptr(), wy.ptr(), C.byref(params)),
+               "sfgpu_mt_occ_costs")
+        return d0, d1
 
     def convolve(self, dst, src, coeffs, vertical=False):
         """convolve_horiz / convolve_vert (image.c:400-645) with 3 or 5 taps."""

@@ -500,9 +500,7 @@ static SinkForestCut::cap_t occ_quantise_host(double e, bool int_terms) {
     return (SinkForestCut::cap_t)llround((int_terms ? (double)(int)e : e) * 16777216.0);
 }
 
-static int optimize_occ(LevelCtx &L) { // variational_aux_mt.cpp:758-887
-    const Geom g = L.g;
-    const double t_begin = now_ms();
+static OccArgs occ_args(const LevelCtx &L) { // the inputs of k_occ_costs: warped frames, raw masks, weights, penalties
     OccArgs a;
     memset(&a, 0, sizeof(a));
     const int F = 2 * L.ref + 1;
@@ -514,6 +512,13 @@ static int optimize_occ(LevelCtx &L) { // variational_aux_mt.cpp:758-887
     a.penalty = L.p->occlusion_penalty;
     a.pc = L.pc;
     a.pg = L.pg;
+    return a;
+}
+
+static int optimize_occ(LevelCtx &L) { // variational_aux_mt.cpp:758-887
+    const Geom g = L.g;
+    const double t_begin = now_ms();
+    const OccArgs a = occ_args(L);
     // d0,d1 are two consecutive planes: reused as the dense W*H array of 64-bit terminal capacities
     const bool int_terms = L.p->graphcut_int_terms != 0;
     long long *tr_dev = reinterpret_cast<long long *>(L.d0);
@@ -550,30 +555,25 @@ static int optimize_occ(LevelCtx &L) { // variational_aux_mt.cpp:758-887
     return SFGPU_OK;
 }
 
-static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_mt.cpp:169-493
-    sfgpu_ctx *c = L.c;
-    const sf_mt_params_t *p = L.p;
-    const Geom g = L.g;
-    const size_t P = g.plane();
-    cudaStream_t st = c->stream;
-    float *A = c->sor.arena;
-    const int ref = L.ref;
-
-    // occlusion labels: 0, or -1 everywhere ("occluded in the past") when reasoning / one direction (:213-220)
-    launch_fill(st, L.occ, P, (L.one_direction || p->occlusion_reasoning) ? -1.0f : 0.0f);
+// The data terms of one level in both data-pass forms: the per-term chain (SLOWFLOW_GPU_MT_DATA_VARIANT=1) and the
+// all-terms pass.  The frames' derivative planes come from warp_all, the reference frame's from mt_system_setup.
+struct MtSystemTerms {
+    std::vector<DataTermDesc> terms; // ordered term list of :343-361
+    MtTermsArgs ta;
     float data_norm = 0.f;
-    for (int s = 0; s < ref; s++) data_norm += p->rho[s] + p->omega[s];
-    launch_dpsis_weight(st, g, L.frames[ref], L.dpsis, 5.0f, p->img_norm_avg, p->img_norm_std, p->hbit ? 65535.0f : 255.0f);
-    c->prof_acc.kernel_launches += 2;
+};
 
-    // ordered term list of :343-361
-    std::vector<DataTermDesc> terms;
+static void mt_system_setup(LevelCtx &L, MtSystemTerms &sys) {
+    const sf_mt_params_t *p = L.p;
+    const int ref = L.ref;
+    for (int s = 0; s < ref; s++) sys.data_norm += p->rho[s] + p->omega[s];
+    std::vector<DataTermDesc> &terms = sys.terms;
+    MtTermsArgs &ta = sys.ta;
     auto pair_imgs = [&](int q, int kind, const float *&Aimg, const float *&Bimg) {
         if (kind == DK_MT_SUCC) { Aimg = L.warped[q]; Bimg = L.warped[q + 1]; }
         else if (q < ref) { Aimg = L.warped[q]; Bimg = L.frames[ref]; }
         else { Aimg = L.frames[ref]; Bimg = L.warped[q + 1]; }
     };
-    MtTermsArgs ta;
     memset(&ta, 0, sizeof(ta));
     auto add_term = [&](int q, int kind, float w, float time, int dir) {
         if (ta.nterms < MT_MAX_TERMS) {
@@ -609,26 +609,75 @@ static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_
 
     if (L.fused_terms) {
         for (int f = 0; f < 2 * ref + 1; f++) { ta.I[f] = L.warped[f]; ta.D[f] = L.derivs[f]; ta.mask[f] = L.masks[f]; }
-        launch_frame_derivs(st, g, L.frames[ref], L.derivs[ref]); // the reference frame is never warped: once per level
-        c->prof_acc.kernel_launches++;
+        launch_frame_derivs(L.c->stream, L.g, L.frames[ref], L.derivs[ref]); // the reference frame is never warped: once per level
+        L.c->prof_acc.kernel_launches++;
     }
-    auto launch_terms = [&](const Geom &gk, DataCommon &cm) { // all data terms of one linearisation (:343-361)
-        if (L.fused_terms) {
-            launch_mt_terms(st, gk, ta, cm, c->mt_terms_scalar);
-            c->prof_acc.kernel_launches++;
-            c->prof_acc.data_launches++;
-            c->prof_acc.data_pixels += (long long)g.W * g.H;
-            return;
-        }
-        for (size_t k = 0; k < terms.size(); k++) {
+}
+
+// One linearisation up to the SOR (:333-365) into the arena planes SP_A11 .. SP_PV of A: smoothness weights of (uu, vv),
+// every data term at the increment (du, dv) (nullptr: zero), b -= div(psi grad uu / vv) and the 2x2 block inverse.
+static void launch_mt_system(LevelCtx &L, const MtSystemTerms &sys, const Geom &g, const float *uu, const float *vv, const float *du,
+                             const float *dv, float *A) {
+    sfgpu_ctx *c = L.c;
+    cudaStream_t st = c->stream;
+    const size_t P = g.plane();
+    launch_smoothness(st, g, uu, vv, L.dpsis, L.alpha, L.preg, L.p->smoothing, A + SP_PH * P, A + SP_PV * P); // :333
+    c->prof_acc.kernel_launches++;
+    DataCommon cm{};
+    cm.du = du;
+    cm.dv = dv;
+    cm.chw = L.chw;
+    cm.chw_pstride = L.chw_pstride;
+    cm.occ = L.occ;
+    cm.data_norm = sys.data_norm;
+    cm.dt_norm = L.p->dataterm;
+    cm.pc = L.pc;
+    cm.pg = L.pg;
+    cm.ph = A + SP_PH * P; cm.pv = A + SP_PV * P;
+    cm.lap_u = uu; cm.lap_v = vv; // MT passes uu, vv to sub_laplacian (:364-365, SURVEY Q11)
+    cm.a11 = A + SP_A11 * P; cm.a12 = A + SP_A12 * P; cm.a22 = A + SP_A22 * P;
+    cm.b1 = A + SP_B1 * P; cm.b2 = A + SP_B2 * P;
+    cudaEvent_t ev;
+    c->prof_begin(1, ev);
+    if (sys.terms.empty()) { // no active data term: the system is the smoothness term alone
+        launch_fill(st, cm.a11, 5 * P, 0.0f);
+        launch_sub_laplacian(st, g, cm.b1, uu, cm.ph, cm.pv);
+        launch_sub_laplacian(st, g, cm.b2, vv, cm.ph, cm.pv);
+        launch_invert_blocks(st, g, cm.a11, cm.a12, cm.a22, cm.ph, cm.pv);
+        c->prof_acc.kernel_launches += 4;
+    } else if (L.fused_terms) { // all data terms of one linearisation (:343-361)
+        launch_mt_terms(st, g, sys.ta, cm, c->mt_terms_scalar);
+        c->prof_acc.kernel_launches++;
+        c->prof_acc.data_launches++;
+        c->prof_acc.data_pixels += (long long)g.W * g.H;
+    } else {
+        for (size_t k = 0; k < sys.terms.size(); k++) {
             cm.accumulate = (k > 0);
-            cm.fuse_system = (k + 1 == terms.size());
-            launch_data_term(st, gk, terms[k], cm);
+            cm.fuse_system = (k + 1 == sys.terms.size());
+            launch_data_term(st, g, sys.terms[k], cm);
             c->prof_acc.kernel_launches++;
             c->prof_acc.data_launches++;
             c->prof_acc.data_pixels += (long long)g.W * g.H;
         }
-    };
+    }
+    c->prof_end(1, ev);
+}
+
+static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_mt.cpp:169-493
+    sfgpu_ctx *c = L.c;
+    const sf_mt_params_t *p = L.p;
+    const Geom g = L.g;
+    const size_t P = g.plane();
+    cudaStream_t st = c->stream;
+    float *A = c->sor.arena;
+    const int ref = L.ref;
+
+    // occlusion labels: 0, or -1 everywhere ("occluded in the past") when reasoning / one direction (:213-220)
+    launch_fill(st, L.occ, P, (L.one_direction || p->occlusion_reasoning) ? -1.0f : 0.0f);
+    launch_dpsis_weight(st, g, L.frames[ref], L.dpsis, 5.0f, p->img_norm_avg, p->img_norm_std, p->hbit ? 65535.0f : 255.0f);
+    c->prof_acc.kernel_launches += 2;
+    MtSystemTerms sys;
+    mt_system_setup(L, sys);
     const dim3 ugrid((g.W + 31) / 32, std::min((g.H + 7) / 8, 64));
     avg_change[0] = avg_change[1] = 0.f;
     const double inv_n = 1.0 / ((double)g.H * g.W);
@@ -656,32 +705,7 @@ static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_
             for (int outer = 0; outer < p->niter_outer; outer++) {
                 if (outer > 0) warp_all(L); // :289-290
                 int cur = 0;
-                launch_smoothness(st, gs, L.wx, L.wy, L.dpsis, L.alpha, L.preg, p->smoothing, A + SP_PH * P, A + SP_PV * P); // :333
-                c->prof_acc.kernel_launches++;
-                DataCommon cm{};
-                cm.du = nullptr; cm.dv = nullptr;
-                cm.chw = L.chw;
-                cm.chw_pstride = L.chw_pstride;
-                cm.occ = L.occ;
-                cm.data_norm = data_norm;
-                cm.dt_norm = p->dataterm;
-                cm.pc = L.pc;
-                cm.pg = L.pg;
-                cm.ph = A + SP_PH * P; cm.pv = A + SP_PV * P;
-                cm.lap_u = L.wx; cm.lap_v = L.wy; // uu == wx at the start of an outer iteration (:364-365, SURVEY Q11)
-                cm.a11 = A + SP_A11 * P; cm.a12 = A + SP_A12 * P; cm.a22 = A + SP_A22 * P;
-                cm.b1 = A + SP_B1 * P; cm.b2 = A + SP_B2 * P;
-                cudaEvent_t ev;
-                c->prof_begin(1, ev);
-                if (terms.empty()) { // no active data term: the system is the smoothness term alone
-                    launch_fill(st, cm.a11, 5 * P, 0.0f);
-                    launch_sub_laplacian(st, gs, cm.b1, L.wx, cm.ph, cm.pv);
-                    launch_sub_laplacian(st, gs, cm.b2, L.wy, cm.ph, cm.pv);
-                    launch_invert_blocks(st, gs, cm.a11, cm.a12, cm.a22, cm.ph, cm.pv);
-                    c->prof_acc.kernel_launches += 4;
-                }
-                if (!terms.empty()) launch_terms(gs, cm);
-                c->prof_end(1, ev);
+                launch_mt_system(L, sys, gs, L.wx, L.wy, nullptr, nullptr, A); // uu == wx at the start of an outer iteration
                 int rc = run_sor(c, p->niter_solver, p->sor_omega, &cur, true); // :368
                 if (rc != SFGPU_OK) { c->sor.g.skip = nullptr; return rc; }
                 const float *ndu = A + (size_t)(cur ? SP_DUB : SP_DUA) * P, *ndv = A + (size_t)(cur ? SP_DVB : SP_DVA) * P;
@@ -731,33 +755,7 @@ static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_
                     SF_CUDA(cudaMemcpyAsync(L.odu, du_cur, P * sizeof(float), cudaMemcpyDeviceToDevice, st));
                     SF_CUDA(cudaMemcpyAsync(L.odv, dv_cur, P * sizeof(float), cudaMemcpyDeviceToDevice, st));
                 }
-                launch_smoothness(st, g, uu, vv, L.dpsis, L.alpha, L.preg, p->smoothing, A + SP_PH * P, A + SP_PV * P); // :333
-                c->prof_acc.kernel_launches++;
-                DataCommon cm{};
-                cm.du = first ? nullptr : du_cur;
-                cm.dv = first ? nullptr : dv_cur;
-                cm.chw = L.chw;
-                cm.chw_pstride = L.chw_pstride;
-                cm.occ = L.occ;
-                cm.data_norm = data_norm;
-                cm.dt_norm = p->dataterm;
-                cm.pc = L.pc;
-                cm.pg = L.pg;
-                cm.ph = A + SP_PH * P; cm.pv = A + SP_PV * P;
-                cm.lap_u = uu; cm.lap_v = vv; // MT passes uu, vv to sub_laplacian (:364-365, SURVEY Q11)
-                cm.a11 = A + SP_A11 * P; cm.a12 = A + SP_A12 * P; cm.a22 = A + SP_A22 * P;
-                cm.b1 = A + SP_B1 * P; cm.b2 = A + SP_B2 * P;
-                cudaEvent_t ev;
-                c->prof_begin(1, ev);
-                if (terms.empty()) { // no active data term: the system is the smoothness term alone
-                    launch_fill(st, cm.a11, 5 * P, 0.0f);
-                    launch_sub_laplacian(st, g, cm.b1, uu, cm.ph, cm.pv);
-                    launch_sub_laplacian(st, g, cm.b2, vv, cm.ph, cm.pv);
-                    launch_invert_blocks(st, g, cm.a11, cm.a12, cm.a22, cm.ph, cm.pv);
-                    c->prof_acc.kernel_launches += 4;
-                }
-                if (!terms.empty()) launch_terms(g, cm);
-                c->prof_end(1, ev);
+                launch_mt_system(L, sys, g, uu, vv, first ? nullptr : du_cur, first ? nullptr : dv_cur, A);
                 int rc = run_sor(c, p->niter_solver, p->sor_omega, &cur, first); // :368
                 if (rc != SFGPU_OK) return rc;
                 c->mt_stats.sor_calls++;
@@ -1014,6 +1012,153 @@ int sfgpu_raw_weighting(sfgpu_ctx *c, color_image_t *weights, int red_x, int red
     c->prof_acc.kernel_launches++;
     SF_CUDA(cudaMemcpyAsync(weights->c1, c->io, 3 * P * sizeof(float), cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaStreamSynchronize(st));
+    return SFGPU_OK;
+}
+
+// ---- operator twins of one level: the production kernels on uploaded level frames and flow
+extern "C++" {
+struct MtTwin { // device planes of one level and the LevelCtx the production helpers take
+    float *base = nullptr;
+    LevelCtx L{};
+    ~MtTwin() { if (base) cudaFree(base); }
+};
+
+// checks the level arguments, uploads frames / flow / occlusion plane / channel weights and warps every frame
+// (plus the reference frame's derivative planes when the all-terms pass is the data pass); `extra` planes follow
+static int mt_twin_level(sfgpu_ctx *c, const char *at, const color_image_t *const *im, const image_t *wx, const image_t *wy,
+                         const image_t *occ, const color_image_t *channel_w, const sf_mt_params_t *p, bool one_direction, int extra,
+                         MtTwin &t, MtSystemTerms *sys, float **extra_planes) {
+    const std::string who(at);
+    if (!c || !im || !p) {
+        set_error(who + "null argument");
+        return SFGPU_ERR_ARG;
+    }
+    const int ref = p->S - 1, F = 2 * ref + 1;
+    if (ref < 1 || ref > SF_MT_MAX_REF || p->smoothing < 0 || p->smoothing > 1) {
+        set_error(who + "slow_flow_S or slow_flow_smoothing out of range");
+        return SFGPU_ERR_ARG;
+    }
+    Geom g;
+    if (!arg_geom(who, "wx", wx, g) || !arg_is(who, "wy", wy, g) || (occ && !arg_is(who, "occ", occ, g)) ||
+        (channel_w && !arg_is(who, "channel_w", channel_w, g)))
+        return SFGPU_ERR_ARG;
+    for (int f = 0; f < F; f++)
+        if (!arg_is(who, "im[" + std::to_string(f) + "]", im[f], g)) return SFGPU_ERR_ARG;
+    if (g.W < 5 || g.H < 5) {
+        set_error(who + "images smaller than 5x5 are not supported");
+        return SFGPU_ERR_ARG;
+    }
+    SF_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const size_t P = g.plane();
+    const bool fused = c->mt_data_variant == 0;
+    const size_t planes = (size_t)F * 3 /*frames*/ + (size_t)F * 3 /*warped*/ + F /*masks*/ + (fused ? (size_t)F * 15 : 0) +
+                          4 /*wx wy occ dpsis*/ + 3 /*channel weights*/ + extra;
+    SF_CUDA(cudaMalloc(&t.base, planes * P * sizeof(float)));
+    float *ptr = t.base;
+    auto take = [&](size_t n) { float *r = ptr; ptr += n * P; return r; };
+    LevelCtx &L = t.L;
+    L.c = c; L.p = p; L.g = g; L.ref = ref;
+    L.one_direction = one_direction;
+    L.alpha = p->alpha;
+    L.gamma_over3 = p->gamma / 3.0f;
+    L.delta_over3 = p->delta / 3.0f;
+    L.pc = make_penalty(p->robust_color, p->robust_color_eps, p->robust_color_truncation);
+    L.pg = (p->robust_grad >= 0) ? make_penalty(p->robust_grad, p->robust_grad_eps, p->robust_grad_truncation) : L.pc;
+    L.preg = make_penalty(p->robust_reg, p->robust_reg_eps, p->robust_reg_truncation);
+    L.frames.assign(F, nullptr); L.warped.assign(F, nullptr); L.masks.assign(F, nullptr); L.derivs.assign(F, nullptr);
+    for (int f = 0; f < F; f++) {
+        L.frames[f] = take(3);
+        SF_CUDA(cudaMemcpyAsync(L.frames[f], im[f]->c1, 3 * P * sizeof(float), cudaMemcpyHostToDevice, st));
+        L.warped[f] = (f == ref) ? L.frames[f] : take(3);
+        L.masks[f] = take(1);
+        if (fused) L.derivs[f] = take(15);
+    }
+    L.fused_terms = fused;
+    L.wx = take(1); L.wy = take(1); L.occ = take(1); L.dpsis = take(1);
+    L.d0 = L.d1 = nullptr; L.uu = L.vv = L.odu = L.odv = nullptr;
+    SF_CUDA(cudaMemcpyAsync(L.wx, wx->data, P * sizeof(float), cudaMemcpyHostToDevice, st));
+    SF_CUDA(cudaMemcpyAsync(L.wy, wy->data, P * sizeof(float), cudaMemcpyHostToDevice, st));
+    if (occ) SF_CUDA(cudaMemcpyAsync(L.occ, occ->data, P * sizeof(float), cudaMemcpyHostToDevice, st));
+    float *chw = take(3);
+    L.chw = nullptr;
+    L.chw_pstride = P;
+    if (channel_w) {
+        SF_CUDA(cudaMemcpyAsync(chw, channel_w->c1, 3 * P * sizeof(float), cudaMemcpyHostToDevice, st));
+        L.chw = chw;
+    }
+    L.work = nullptr;
+    *extra_planes = take(extra);
+    warp_all(L);
+    if (sys) {
+        launch_dpsis_weight(st, g, L.frames[ref], L.dpsis, 5.0f, p->img_norm_avg, p->img_norm_std, p->hbit ? 65535.0f : 255.0f);
+        mt_system_setup(L, *sys);
+    }
+    SF_CUDA(cudaGetLastError());
+    return SFGPU_OK;
+}
+} // extern "C++"
+
+int sfgpu_mt_system(sfgpu_ctx *c, image_t *a11, image_t *a12, image_t *a22, image_t *b1, image_t *b2, image_t *psi_h, image_t *psi_v,
+                    const color_image_t *const *im, const image_t *wx, const image_t *wy, const image_t *du, const image_t *dv,
+                    const image_t *occ, const color_image_t *channel_w, const sf_mt_params_t *p) {
+    const char *at = "sfgpu_mt_system: ";
+    if ((du == nullptr) != (dv == nullptr) || !occ) {
+        set_error("sfgpu_mt_system: du and dv must both be given or both be null, occ is required");
+        return SFGPU_ERR_ARG;
+    }
+    Geom g;
+    if (!arg_geom(at, "wx", wx, g) || (du && (!arg_is(at, "du", du, g) || !arg_is(at, "dv", dv, g))))
+        return SFGPU_ERR_ARG;
+    image_t *outs[7] = {a11, a12, a22, b1, b2, psi_h, psi_v}; // arena order SP_A11 .. SP_PV
+    const char *names[7] = {"a11", "a12", "a22", "b1", "b2", "psi_h", "psi_v"};
+    for (int k = 0; k < 7; k++)
+        if (!arg_is(at, names[k], outs[k], g)) return SFGPU_ERR_ARG;
+    MtTwin t;
+    MtSystemTerms sys;
+    float *A = nullptr;
+    int rc = mt_twin_level(c, at, im, wx, wy, occ, channel_w, p, p && p->one_direction != 0, 11, t, &sys, &A);
+    if (rc != SFGPU_OK) return rc;
+    cudaStream_t st = c->stream;
+    const size_t P = g.plane();
+    float *uu = A + 7 * P, *vv = A + 8 * P, *ddu = A + 9 * P, *ddv = A + 10 * P;
+    const float *su = t.L.wx, *sv = t.L.wy;
+    std::vector<float> hu, hv;
+    if (du) { // uu = wx + du (variational_mt.cpp:397-398)
+        hu.resize(P); hv.resize(P);
+        for (size_t k = 0; k < P; k++) { hu[k] = wx->data[k] + du->data[k]; hv[k] = wy->data[k] + dv->data[k]; }
+        SF_CUDA(cudaMemcpyAsync(ddu, du->data, P * sizeof(float), cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(ddv, dv->data, P * sizeof(float), cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(uu, hu.data(), P * sizeof(float), cudaMemcpyHostToDevice, st));
+        SF_CUDA(cudaMemcpyAsync(vv, hv.data(), P * sizeof(float), cudaMemcpyHostToDevice, st));
+        su = uu; sv = vv;
+    }
+    SF_CUDA(cudaMemsetAsync(A, 0xff, 7 * P * sizeof(float), st)); // NaN pattern: every element must be written
+    launch_mt_system(t.L, sys, g, su, sv, du ? ddu : nullptr, du ? ddv : nullptr, A);
+    for (int k = 0; k < 7; k++)
+        SF_CUDA(cudaMemcpyAsync(outs[k]->data, A + (size_t)k * P, P * sizeof(float), cudaMemcpyDeviceToHost, st));
+    SF_CUDA(cudaStreamSynchronize(st));
+    SF_CUDA(cudaGetLastError());
+    return SFGPU_OK;
+}
+
+int sfgpu_mt_occ_costs(sfgpu_ctx *c, image_t *d0, image_t *d1, const color_image_t *const *im, const image_t *wx, const image_t *wy,
+                       const sf_mt_params_t *p) {
+    const char *at = "sfgpu_mt_occ_costs: ";
+    Geom g;
+    if (!arg_geom(at, "wx", wx, g) || !arg_is(at, "d0", d0, g) || !arg_is(at, "d1", d1, g)) return SFGPU_ERR_ARG;
+    MtTwin t;
+    float *D = nullptr;
+    int rc = mt_twin_level(c, at, im, wx, wy, nullptr, nullptr, p, false, 2, t, nullptr, &D);
+    if (rc != SFGPU_OK) return rc;
+    cudaStream_t st = c->stream;
+    const size_t P = g.plane();
+    SF_CUDA(cudaMemsetAsync(D, 0xff, 2 * P * sizeof(float), st)); // NaN pattern: the kernel writes the W x H pixels only
+    k_occ_costs<<<grid2d(g.W, g.H), dim3(32, 8), 0, st>>>(g, occ_args(t.L), D, D + P, nullptr, p->graphcut_int_terms != 0 ? 1 : 0);
+    SF_CUDA(cudaMemcpyAsync(d0->data, D, P * sizeof(float), cudaMemcpyDeviceToHost, st));
+    SF_CUDA(cudaMemcpyAsync(d1->data, D + P, P * sizeof(float), cudaMemcpyDeviceToHost, st));
+    SF_CUDA(cudaStreamSynchronize(st));
+    SF_CUDA(cudaGetLastError());
     return SFGPU_OK;
 }
 

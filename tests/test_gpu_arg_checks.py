@@ -139,6 +139,15 @@ ENTRIES = [
           lambda L, h, I, X: L.sfgpu_variational_mt(h, I["wx"], I["wy"], arr(CP, [I["im[%d]" % f] for f in range(3)]), X["params"],
                                                     I["channel_w"], I["occlusions_out"], X["avg"]),
           extras=lambda: dict(params=mt_helpers.clone_params(MT), avg=(C.c_float * 2)(7.0, 7.0))),
+    Entry("sfgpu_mt_system", images("wx:i wy:i du:i dv:i occ:i channel_w:c " + seq("im", 3, "c") + " a11:i a12:i a22:i b1:i b2:i psi_h:i psi_v:i"),
+          lambda L, h, I, X: L.sfgpu_mt_system(h, *[I[a] for a in ("a11", "a12", "a22", "b1", "b2", "psi_h", "psi_v")],
+                                               arr(CP, [I["im[%d]" % f] for f in range(3)]), I["wx"], I["wy"], I["du"], I["dv"], I["occ"],
+                                               I["channel_w"], X["params"]),
+          extras=lambda: dict(params=mt_helpers.clone_params(MT))),
+    Entry("sfgpu_mt_occ_costs", images("wx:i wy:i " + seq("im", 3, "c") + " d0:i d1:i"),
+          lambda L, h, I, X: L.sfgpu_mt_occ_costs(h, I["d0"], I["d1"], arr(CP, [I["im[%d]" % f] for f in range(3)]), I["wx"], I["wy"],
+                                                  X["params"]),
+          extras=lambda: dict(params=mt_helpers.clone_params(MT))),
     Entry("sfgpu_normalize", images(seq("seq", 3, "c")),
           lambda L, h, I, X: L.sfgpu_normalize(h, arr(CP, [I["seq[%d]" % f] for f in range(3)]), 3, X["params"]),
           extras=lambda: dict(params=mt_helpers.clone_params(MT))),

@@ -298,6 +298,20 @@ def test_mt_channel_weights_parity(ctx, mt_checker):
     check(g, r, "channel weights")
 
 
+def test_mt_channel_weights_on_a_coarser_level(ctx, mt_checker):
+    """layers = 2 with channel weights: the coarser level reads the level-0 weight planes with its own stride, like the
+    reference does (it never rescales the weights, SURVEY Q14)."""
+    w, h = 253, 131
+    ims, wx, wy = mh.window(w, h, 3)
+    rng = np.random.default_rng(12)
+    chw = ColorImage.from_array(rng.uniform(0.5, 1.5, size=(3, h, w)).astype(np.float32))
+    p = mh.params(3, layers=2, niter_alter=2, niter_outer=3, robust_color=4, robust_color_eps=0.5)
+    r = mh.run_cpu(*mt_checker, ims, wx, wy, p, SOR_REDBLACK, chw)
+    g = mh.run_gpu(ctx, ims, wx, wy, p, chw)
+    assert g["stats"].levels == 2
+    check(g, r, "channel weights, 2 layers")
+
+
 @pytest.mark.parametrize("w,h", [(17, 13), (33, 9), (66, 31), (127, 40)])
 def test_mt_tiny_and_ragged_windows(monkeypatch, w, h):
     """Ragged widths around the 64-column tile of the packed all-terms pass and the 56-column strips of the marching

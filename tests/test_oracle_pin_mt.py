@@ -34,6 +34,36 @@ def test_mt_restatement_matches_golden(oracle, name):
     assert np.array_equal(np.array([r["params"].img_norm_std[k] for k in range(3)], np.float32), g["norm_std"])
 
 
+@pytest.mark.parametrize("S,kw", [
+    (3, dict()),
+    (2, dict(robust_color=4, robust_color_eps=0.5, dataterm=0, occlusion_reasoning=0)),
+    (4, dict(one_direction=1, rho=[1, 1, 1], omega=[0, 2, 1], smoothing=0, robust_grad=2, robust_grad_eps=0.5)),
+])
+def test_mt_operator_entries_compose_to_one_iteration(oracle, S, kw):
+    """sfo_mt_system -> sfo_sor_coupled -> wx + du is exactly sfo_variational_mt with one alternation, one outer and one inner
+    iteration: the operator entries are the functions the pinned driver is made of."""
+    from slowflow_b200 import ColorImage, Image
+    w, h = 61, 45
+    ims, wx, wy = mh.window(w, h, S)
+    p = mh.params(S, niter_alter=1, niter_outer=1, niter_inner=1, **kw)
+    rng = np.random.default_rng(3)
+    chw = ColorImage.from_array(rng.uniform(0.5, 1.5, size=(3, h, w)).astype(np.float32))
+    full = mh.run_cpu(oracle.lib, "sfo_", ims, wx, wy, p, 1, chw)
+    frames = [f.copy() for f in ims]
+    q = mh.clone_params(p)
+    oracle.lib.sfo_normalize(mh.frame_array(frames), len(frames), C.byref(q))
+    occ = Image(w, h)
+    occ.buf[:] = -1.0 if (p.occlusion_reasoning or p.one_direction) else 0.0
+    A = [Image(w, h) for _ in range(7)]
+    assert oracle.lib.sfo_mt_system(*[a.ptr() for a in A], mh.frame_array(frames), wx.ptr(), wy.ptr(), None, None, occ.ptr(),
+                                    chw.ptr(), C.byref(q)) == 0
+    du, dv = Image(w, h), Image(w, h)
+    oracle.lib.sfo_sor_coupled(du.ptr(), dv.ptr(), *[a.ptr() for a in A], q.niter_solver, q.sor_omega, 1)
+    assert np.array_equal(wx.array + du.array, full["wx"].array)
+    assert np.array_equal(wy.array + dv.array, full["wy"].array)
+    assert np.abs(du.array).max() > 1e-3
+
+
 @pytest.mark.parametrize("size,S,kw", [
     ((131, 77), 3, dict(niter_alter=2, niter_outer=2, robust_color=4, robust_color_eps=0.5)),
     ((96, 64), 3, dict(niter_alter=1, niter_outer=1, robust_color=3, robust_color_truncation=5.0, dataterm=0)),
