@@ -185,7 +185,36 @@ int sfgpu_mt_frame_cache(sfgpu_ctx *ctx, int max_frames);
 /* normalize() of variational_mt.cpp:17-85: in place on F host frames; fills params->img_norm_* */
 int sfgpu_normalize(sfgpu_ctx *ctx, color_image_t *const *seq, int F, sf_mt_params_t *params);
 
-/* iteration statistics of the last sfgpu_variational_mt call on this context */
+/* The jet loop of slow_flow.cpp:706-1030 (deep_matching = 0) over ONE sequence of integer frames, on the device.
+ * frames[0 .. n_frames-1]: the loaded sequence as cv::Mat fields (sf_frame_int_t, like sfgpu_variational_sequence_u8/u16),
+ * bits = 8 or 16, all of one width x height.  scale != 1: every frame is pre-scaled first, exactly as sfgpu_prescale
+ * does (slow_flow.cpp:538-542).  The sequence is then normalised as ONE sequence over all n_frames (normalize(),
+ * variational_mt.cpp:17-85); params->img_norm_avg / img_norm_std receive the values normalize() publishes (6 significant
+ * digits), and those published values are the ones the windows use.
+ * With steps = params->S - 1, jet j in [first_jet, first_jet + n_jets) writes, at index k = j - first_jet:
+ *   fwd_x[k], fwd_y[k]   forward window frames[j*steps .. j*steps + 2*steps]: zero initial flow, channel_w
+ *                        (NULL: all ones), one_direction = params->one_direction; result x steps (:865-911)
+ *   back_x[k], back_y[k] backward window, the reversed frames j*steps + 3*steps down to j*steps + steps:
+ *                        no channel weights (Q10), one_direction = params->one_direction || backward_one_direction;
+ *                        result x steps (:1018-1030)
+ *   occlusions[k]        (the array may be NULL) the forward window's -1/0/+1 labels (Variational_MT::getOcclusions)
+ * Every output, bit for bit and on whole planes, equals this sequence of calls:
+ *   unpack the frame to float (exact) -> sfgpu_prescale -> sfgpu_normalize over all n_frames
+ *   -> sfgpu_variational_mt per window -> multiply by steps in fp32.
+ * Output planes (and channel_w) have the (scaled) frame geometry.  n_frames >= 1 + (first_jet + n_jets + 2) * steps: a
+ * multi-GPU caller shards the jets with first_jet / n_jets, and every shard normalises over the whole sequence.
+ * Each jet's new frames are uploaded while the previous jet solves, and with page-locked memory every window's results
+ * are downloaded while the next window computes (pageable memory is staged as in sfgpu_variational_sequence).
+ * sfgpu_get_mt_stats afterwards sums the windows of the call; its setup_ms is the time of the statistics pass and
+ * total_ms that of the call.  Every argument check runs before anything is written.  SFGPU_ERR_UNSUPPORTED for
+ * smoothing >= 2, like sfgpu_variational_mt.  Uses the context's io area, so a following sfgpu_variational_sequence_u8/u16
+ * cannot use continue_from_previous. */
+int sfgpu_slow_flow_jets(sfgpu_ctx *ctx, int n_frames, const sf_frame_int_t *frames, int bits, float scale,
+                         int first_jet, int n_jets, sf_mt_params_t *params, int backward_one_direction,
+                         const color_image_t *channel_w, image_t *const *fwd_x, image_t *const *fwd_y,
+                         image_t *const *back_x, image_t *const *back_y, image_t *const *occlusions);
+
+/* iteration statistics of the last sfgpu_variational_mt (or sfgpu_slow_flow_jets) call on this context */
 typedef struct sfgpu_mt_stats_s {
     int levels;            /* pyramid levels actually run */
     int outer_iterations;  /* total outer iterations executed over all levels / alternations */

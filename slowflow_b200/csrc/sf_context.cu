@@ -308,6 +308,17 @@ bool arg_geom(const std::string &at, const std::string &name, const color_image_
 bool arg_is(const std::string &at, const std::string &name, const image_t *a, Geom g) { return check_image(at, name, a, g, false); }
 bool arg_is(const std::string &at, const std::string &name, const color_image_t *a, Geom g) { return check_image(at, name, a, g, false); }
 
+bool arg_frame_int(const std::string &at, const std::string &name, const sf_frame_int_t &q, Geom g, int bits) {
+    const size_t sample = bits / 8;
+    if (!q.data || q.width != g.W || q.height != g.H || (q.channels != 1 && q.channels != 3) ||
+        q.step < (size_t)q.width * q.channels * sample || (q.step % sample) != 0) {
+        set_error(at + name + ": integer frames must match the call's geometry (" + std::to_string(g.W) + "x" + std::to_string(g.H) +
+                  "), have 1 or 3 channels and step >= width*channels*bytes");
+        return false;
+    }
+    return true;
+}
+
 } // namespace sf
 
 // ------------------------------------------------------------------------------------------ ABI: basics

@@ -138,6 +138,33 @@ bool arg_geom(const std::string &at, const std::string &name, const color_image_
 bool arg_is(const std::string &at, const std::string &name, const image_t *a, Geom g);
 bool arg_is(const std::string &at, const std::string &name, const color_image_t *a, Geom g);
 
+// arg_frame_int: an integer frame (sf_frame_int_t) of `bits` 8 or 16 with non-null data, width x height of g, 1 or 3
+// channels and a row step of at least width * channels samples that is a multiple of the sample size
+bool arg_frame_int(const std::string &at, const std::string &name, const sf_frame_int_t &q, Geom g, int bits);
+
+// One window of Variational_MT::variational (variational_mt.cpp:526-784) on device planes (sf_mt.cu), in three steps:
+//   mt_window_layout  pyramid geometry and the planes of the context's multi-frame workspace.  own_frames0: the level-0
+//                     frames are workspace planes too (else the caller sets frames[0][f] to its own device frames);
+//                     chw_plane: 3 planes for channel weights (chw points at them; the caller may point it elsewhere).
+//                     levels == 0: the reference computes nothing and nothing else may be called.
+//   mt_window_build   after the caller has filled frames[0], wx, wy (and chw): the coarser levels' frames, the initial
+//                     flow on the coarsest level, the level workspace
+//   mt_window_solve   coarse-to-fine; the flow of level 0 is left in wx, wy, the occlusion labels in occ.  Synchronises the
+//                     context's stream once per level.
+struct MtWindow {
+    int levels = 0, ref = 0;
+    float sigma = 0.f;
+    std::vector<Geom> geoms;                  // per level
+    std::vector<std::vector<float *>> frames; // [level][frame], 3 planes each
+    std::vector<float *> warped, masks, derivs;
+    float *wx = nullptr, *wy = nullptr, *wxb = nullptr, *wyb = nullptr, *uu = nullptr, *vv = nullptr, *odu = nullptr,
+          *odv = nullptr, *dpsis = nullptr, *occ = nullptr, *d0 = nullptr, *d1 = nullptr, *blur_tmp = nullptr, *chw_plane = nullptr;
+    const float *chw = nullptr;
+};
+int mt_window_layout(sfgpu_ctx *c, const sf_mt_params_t *p, Geom g0, bool own_frames0, bool chw_plane, MtWindow &w);
+int mt_window_build(sfgpu_ctx *c, MtWindow &w);
+int mt_window_solve(sfgpu_ctx *c, const sf_mt_params_t *p, bool one_direction, MtWindow &w, float avg_change[2]);
+
 // exact binary Potts min-cut on the device (sf_mincut.cu); results in occ / device_cut_labels(), status after a stream sync
 int device_grid_mincut(sfgpu_ctx *c, DeviceCut *&cut, int W, int H, long long *tr_dev, long long pair_cap, float *occ, int S);
 const int *device_cut_status(const DeviceCut *cut);       // {0 = converged, phases, grid-wide passes}

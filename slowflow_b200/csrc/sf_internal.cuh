@@ -178,6 +178,28 @@ void launch_add(cudaStream_t st, Geom g, float *dst, const float *a, const float
 void launch_fill(cudaStream_t st, float *dst, size_t n, float v);
 
 // ---------------------------------------------------------------------------------------------
+// input side of the multi-frame path: what slow_flow.cpp does to every frame before the solver sees it
+// packed 8-/16-bit frame (cv::Mat rows of `step` bytes, 1 or 3 interleaved channels) -> planar fp32 of g, exact, stride
+// padding zeroed (mat2colorImg / colorMat2colorImg, utils/utils.h:122-160; sf_sequence.cu)
+void launch_unpack_frame(cudaStream_t st, Geom g, const unsigned char *raw, size_t step, int channels, int bits, float *dst);
+// separable Gaussian of cv::GaussianBlur (replicate border) and its taps (cv::getGaussianKernel) (sf_mt.cu)
+struct BlurTaps { int r; float k[17]; }; // k[0] centre, k[i] at distance i
+BlurTaps make_taps(double sigma);
+void launch_blur(cudaStream_t st, Geom g, const float *src, float *tmp, float *dst, const BlurTaps &t, int planes);
+// the pre-scaling of slow_flow.cpp:538-542 from src (gs) into dst (gd = sfgpu_prescale_size); tmp, blur: 3 planes of gs
+void launch_prescale(cudaStream_t st, Geom gs, const float *src, float *tmp, float *blur, Geom gd, float *dst, float scale);
+// normalize() (variational_mt.cpp:17-85) in four steps: per frame the block partials of the channel sums (norm_blocks(g) x 6
+// doubles), from a planar fp32 frame or from the packed integer frame that unpacks to it (same partials); the statistics
+// of F frames from their partials, in a fixed order on the host; the in-place normalisation of a frame (a channel with
+// std <= 0 is left as it is); the values the reference publishes (6 significant digits) into p->img_norm_*.
+int norm_blocks(Geom g);
+void launch_norm_sums(cudaStream_t st, Geom g, const float *im, double *sums);
+void launch_norm_sums_packed(cudaStream_t st, Geom g, const unsigned char *raw, size_t step, int channels, int bits, double *sums);
+void norm_statistics(const double *partials, int F, Geom g, double avg[3], double sd[3]);
+void launch_norm_apply(cudaStream_t st, Geom g, float *im, const double avg[3], const double sd[3]);
+void norm_publish(const double avg[3], const double sd[3], sf_mt_params_t *p);
+
+// ---------------------------------------------------------------------------------------------
 // K4: red-black SOR on the coupled 2x2-block 5-point system (solver.c:63, re-ordered).
 // The SOR arena is 11 consecutive planes: a11' a12' a22' b1 b2 psi_h psi_v duA dvA duB dvB.
 enum SorPlane { SP_A11 = 0, SP_A12, SP_A22, SP_B1, SP_B2, SP_PH, SP_PV, SP_DUA, SP_DVA, SP_DUB, SP_DVB, SP_COUNT };

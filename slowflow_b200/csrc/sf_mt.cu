@@ -181,7 +181,6 @@ __global__ void __launch_bounds__(256) k_occ_labels(Geom g, const unsigned char 
 
 // separable Gaussian (replicate border), symmetric-sum evaluation like cv::GaussianBlur's float path.  Both passes handle
 // 4 consecutive pixels per thread with float4 loads / stores (rows are 16-byte aligned: stride = ceil4(width)).
-struct BlurTaps { int r; float k[17]; }; // k[0] centre, k[i] at distance i
 constexpr int BLUR_SEG = 128 * 4; // columns per block of the horizontal pass (128 threads x 4)
 // horizontal pass: the block stages its row segment + r columns on either side (clamped to the row) in shared memory
 __global__ void __launch_bounds__(128) k_blur_h4(Geom g, const float *__restrict__ src, float *__restrict__ dst, BlurTaps t, int planes) {
@@ -234,7 +233,7 @@ __global__ void __launch_bounds__(256) k_blur_v4(Geom g, const float *__restrict
         *reinterpret_cast<float4 *>(dst + c * P + (size_t)y * g.S + x) = acc;
     }
 }
-static void launch_blur(cudaStream_t st, Geom g, const float *src, float *tmp, float *dst, const BlurTaps &t, int planes) {
+void launch_blur(cudaStream_t st, Geom g, const float *src, float *tmp, float *dst, const BlurTaps &t, int planes) {
     k_blur_h4<<<dim3((g.S + BLUR_SEG - 1) / BLUR_SEG, g.H), 128, 0, st>>>(g, src, tmp, t, planes);
     k_blur_v4<<<dim3((g.S / 4 + 31) / 32, (g.H + 7) / 8), dim3(32, 8), 0, st>>>(g, tmp, dst, t, planes);
 }
@@ -287,6 +286,14 @@ __global__ void __launch_bounds__(256) k_resize(Geom gs, const float *__restrict
 }
 static dim3 resize_grid(Geom gd) { return dim3((gd.S / 4 + 31) / 32, (gd.H + 7) / 8); }
 
+// GaussianBlur(src, sigma = 1/sqrt(2 scale), BORDER_REPLICATE) then resize(fx = fy = scale, INTER_LINEAR) (slow_flow.cpp:539-542);
+// the mapping of a resize by factor uses 1/fx, not the ratio of the rounded sizes
+void launch_prescale(cudaStream_t st, Geom gs, const float *src, float *tmp, float *blur, Geom gd, float *dst, float scale) {
+    const BlurTaps taps = make_taps(1.0 / sqrt((double)(2.0f * scale)));
+    launch_blur(st, gs, src, tmp, blur, taps, 3);
+    k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(gs, blur, gd, dst, 1.0 / (double)scale, 1.0 / (double)scale, 1.0f, 3);
+}
+
 // rawWeighting (utils/utils.cpp:1336-1374): per-pixel channel weights of a Bayer mosaic whose red site is at
 // (red_x, red_y) mod 2 -- the measured channel gets `weight`, the two interpolated ones 0.5*(3 - weight)
 __global__ void __launch_bounds__(256) k_raw_weights(Geom g, float *__restrict__ w3, int red_x, int red_y, float weight) {
@@ -310,13 +317,30 @@ __global__ void __launch_bounds__(256) k_raw_weights(Geom g, float *__restrict__
 
 // normalize(): per-channel sums in double (variational_mt.cpp:27-46), then (I - avg) / std (:61-69).  Every block writes
 // its six partial sums to sums[block*6 + k]; the host adds them in block order (deterministic: no atomics on the path).
-__global__ void __launch_bounds__(256) k_norm_sums(Geom g, const float *__restrict__ im, double *__restrict__ sums /*gridDim.x * 6*/) {
+// The samples come from a planar fp32 frame or, with the same rows, columns, channel order and tree, straight from the
+// packed 8-/16-bit frame that converts to it exactly (k_unpack_frame, sf_sequence.cu): both give the same partials.
+struct PlanarSamples {
+    const float *im;
+    size_t P;
+    __device__ __forceinline__ double operator()(int c, int j, int i, size_t S) const { return im[c * P + (size_t)j * S + i]; }
+};
+template <typename T>
+struct PackedSamples {
+    const unsigned char *raw;
+    size_t step;
+    int channels;
+    __device__ __forceinline__ double operator()(int c, int j, int i, size_t) const {
+        const T *row = reinterpret_cast<const T *>(raw + (size_t)j * step);
+        return (double)(float)row[channels == 1 ? i : 3 * i + c];
+    }
+};
+template <typename Samples>
+__global__ void __launch_bounds__(256) k_norm_sums(Geom g, Samples src, double *__restrict__ sums /*gridDim.x * 6*/) {
     double s[6] = {0, 0, 0, 0, 0, 0};
-    const size_t P = g.plane();
     for (int j = blockIdx.x; j < g.H; j += gridDim.x)
         for (int i = threadIdx.x; i < g.W; i += blockDim.x)
             for (int c = 0; c < 3; c++) {
-                const double v = im[c * P + (size_t)j * g.S + i];
+                const double v = src(c, j, i, g.S);
                 s[c] += v;
                 s[3 + c] += v * v;
             }
@@ -341,14 +365,51 @@ __global__ void __launch_bounds__(256) k_norm_apply(Geom g, float *__restrict__ 
     if (s2 > 0) im[o + 2 * P] = (float)(((double)im[o + 2 * P] - a2) / s2);
 }
 
+int norm_blocks(Geom g) { return std::min(g.H, 592); }
+void launch_norm_sums(cudaStream_t st, Geom g, const float *im, double *sums) {
+    k_norm_sums<<<norm_blocks(g), 256, 0, st>>>(g, PlanarSamples{im, g.plane()}, sums);
+}
+void launch_norm_sums_packed(cudaStream_t st, Geom g, const unsigned char *raw, size_t step, int channels, int bits, double *sums) {
+    if (bits == 8)
+        k_norm_sums<<<norm_blocks(g), 256, 0, st>>>(g, PackedSamples<unsigned char>{raw, step, channels}, sums);
+    else
+        k_norm_sums<<<norm_blocks(g), 256, 0, st>>>(g, PackedSamples<unsigned short>{raw, step, channels}, sums);
+}
+
+// the host side of normalize(): frame f's block partials (norm_blocks(g) x 6 at partials + f * norm_blocks(g) * 6) added in
+// block order, the per-frame means averaged over the F frames, std = sqrt(E[I^2] - avg^2) / 255 (:27-51)
+void norm_statistics(const double *partials, int F, Geom g, double avg[3], double sd[3]) {
+    const int nblk = norm_blocks(g);
+    const double n = (double)g.H * g.W;
+    for (int k = 0; k < 3; k++) avg[k] = sd[k] = 0.0;
+    for (int f = 0; f < F; f++) {
+        double fs[6] = {0, 0, 0, 0, 0, 0};
+        for (int blk = 0; blk < nblk; blk++)
+            for (int k = 0; k < 6; k++) fs[k] += partials[((size_t)f * nblk + blk) * 6 + k];
+        for (int k = 0; k < 3; k++) { avg[k] += fs[k] / n; sd[k] += fs[3 + k] / n; }
+    }
+    for (int k = 0; k < 3; k++) {
+        avg[k] /= F;
+        sd[k] = sqrt((sd[k] / F) - avg[k] * avg[k]) / 255.0f; // :48-51
+    }
+}
+void launch_norm_apply(cudaStream_t st, Geom g, float *im, const double avg[3], const double sd[3]) {
+    k_norm_apply<<<dim3((g.W + 31) / 32, (g.H + 7) / 8), dim3(32, 8), 0, st>>>(g, im, avg[0], avg[1], avg[2], sd[0], sd[1], sd[2]);
+}
+// the reference publishes the values through a stringstream with 6 significant digits (:72-84)
+void norm_publish(const double avg[3], const double sd[3], sf_mt_params_t *p) {
+    for (int k = 0; k < 3; k++) {
+        char buf[64];
+        snprintf(buf, sizeof(buf), "%.6g", avg[k]);
+        p->img_norm_avg[k] = (float)atof(buf);
+        snprintf(buf, sizeof(buf), "%.6g", sd[k]);
+        p->img_norm_std[k] = (float)atof(buf);
+    }
+}
+
 static dim3 grid2d(int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8); }
 
 // ------------------------------------------------------------------------------------------ level state
-struct MtLevel {
-    Geom g;
-    std::vector<float *> frames; // F colour images (3 planes each)
-};
-
 // Per-context multi-frame workspace; kept between calls (buffers only grow).
 struct MtWork {
     float *pool = nullptr;
@@ -409,7 +470,7 @@ struct MtWork {
 };
 void mt_work_free(MtWork *w) { delete w; }
 
-static BlurTaps make_taps(double sigma) {
+BlurTaps make_taps(double sigma) {
     // cv::getGaussianKernel: n = cvRound(8 sigma + 1) | 1 for CV_32F, exp(-x^2 / 2 sigma^2) normalised
     BlurTaps t;
     int n = ((int)lrint(sigma * 8 + 1)) | 1;
@@ -806,6 +867,141 @@ static int compute_one_level(LevelCtx &L, float avg_change[2]) { // variational_
     return SFGPU_OK;
 }
 
+
+// ------------------------------------------------------------------------------------------ one window
+int mt_window_layout(sfgpu_ctx *c, const sf_mt_params_t *p, Geom g0, bool own_frames0, bool chw_plane, MtWindow &w) {
+    const int ref = p->S - 1, F = 2 * ref + 1;
+    // ---- pyramid geometry (variational_mt.cpp:583-652): floor((float)w * p_scale); a level is dropped when
+    // the NEXT one would be <= order+1 = floor(3 sigma)+2 pixels (:647-651)
+    w.sigma = 1.0f / sqrtf(2.0f * p->p_scale);
+    const int order = (int)floorf(3.0f * w.sigma) + 1;
+    std::vector<Geom> &geoms = w.geoms;
+    geoms.clear();
+    int L = p->layers;
+    for (int l = 0; l < L; l++) {
+        if (l == 0) geoms.push_back(g0);
+        else geoms.push_back(make_geom((int)floorf((float)geoms[l - 1].W * p->p_scale), (int)floorf((float)geoms[l - 1].H * p->p_scale)));
+        if (floorf((float)geoms[l].W * p->p_scale) <= order + 1 || floorf((float)geoms[l].H * p->p_scale) <= order + 1) {
+            L = l;
+            break;
+        }
+    }
+    w.levels = L;
+    if (L == 0) return SFGPU_OK;
+    geoms.resize(L);
+    c->mt_stats.levels += L;
+    w.ref = ref;
+
+    // ---- device memory: frames of all levels + per-level work planes sized for level 0
+    const size_t P0 = g0.plane();
+    size_t frame_floats = 0;
+    for (int l = own_frames0 ? 0 : 1; l < L; l++) frame_floats += (size_t)F * 3 * geoms[l].plane();
+    const size_t work_planes = (size_t)(F - 1) * 3 + (F - 1) + 2 /*wx wy*/ + 2 /*wx,wy of next level*/ + 2 /*uu vv*/ + 2 /*odu odv*/ + 1 /*dpsis*/ +
+                               1 /*occ*/ + 2 /*d0 d1*/ + 3 /*blur tmp*/ + (chw_plane ? 3 : 0) +
+                               (c->mt_data_variant == 0 ? (size_t)F * 15 /*per-frame derivative planes*/ : 0);
+    if (!c->mtw) c->mtw = new MtWork();
+    MtWork &work = *c->mtw;
+    {
+        const int rcw = work.reserve(frame_floats + work_planes * P0, (size_t)((g0.W + 31) / 32) * 64 * 4, (size_t)g0.W * g0.H);
+        if (rcw != SFGPU_OK) return rcw;
+    }
+    float *ptr = work.pool;
+    w.frames.assign(L, std::vector<float *>(F, nullptr));
+    for (int l = own_frames0 ? 0 : 1; l < L; l++)
+        for (int f = 0; f < F; f++) { w.frames[l][f] = ptr; ptr += 3 * geoms[l].plane(); }
+    auto take = [&](size_t planes) { float *r = ptr; ptr += planes * P0; return r; };
+    w.warped.assign(F, nullptr);
+    w.masks.assign(F, nullptr);
+    for (int f = 0; f < F; f++)
+        if (f != ref) { w.warped[f] = take(3); w.masks[f] = take(1); }
+    w.wx = take(1); w.wy = take(1); w.wxb = take(1); w.wyb = take(1);
+    w.uu = take(1); w.vv = take(1); w.odu = take(1); w.odv = take(1); w.dpsis = take(1); w.occ = take(1); w.d0 = take(1); w.d1 = take(1);
+    w.blur_tmp = take(3);
+    w.chw_plane = chw_plane ? take(3) : nullptr;
+    w.chw = w.chw_plane;
+    w.derivs.assign(F, nullptr);
+    if (c->mt_data_variant == 0)
+        for (int f = 0; f < F; f++) w.derivs[f] = take(15);
+    return SFGPU_OK;
+}
+
+int mt_window_build(sfgpu_ctx *c, MtWindow &w) {
+    cudaStream_t st = c->stream;
+    const int L = w.levels, F = 2 * w.ref + 1;
+    const std::vector<Geom> &geoms = w.geoms;
+    const Geom g0 = geoms[0];
+    // ---- pyramid: GaussianBlur(sigma) + resize per frame and level (:604-614)
+    if (L > 1) {
+        const BlurTaps taps = make_taps((double)w.sigma);
+        for (int l = 1; l < L; l++) {
+            const Geom gs = geoms[l - 1], gd = geoms[l];
+            for (int f = 0; f < F; f++) {
+                // vertical pass writes into the (not yet used) warp scratch of frame slot 0/1
+                float *tmp2 = w.warped[w.ref == 0 ? 1 : 0];
+                launch_blur(st, gs, w.frames[l - 1][f], w.blur_tmp, tmp2, taps, 3);
+                k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(gs, tmp2, gd, w.frames[l][f], (double)gs.W / gd.W,
+                                                                  (double)gs.H / gd.H, 1.0f, 3);
+                c->prof_acc.kernel_launches += 3;
+            }
+        }
+    }
+    // ---- coarse-to-fine (:662-762): the initial flow goes to the coarsest level
+    if (L > 1) {
+        const Geom gd = geoms[L - 1];
+        const float fx = (1.0f * gd.W) / g0.W, fy = (1.0f * gd.H) / g0.H;
+        k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(g0, w.wx, gd, w.wxb, (double)g0.W / gd.W, (double)g0.H / gd.H, fx, 1);
+        k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(g0, w.wy, gd, w.wyb, (double)g0.W / gd.W, (double)g0.H / gd.H, fy, 1);
+        std::swap(w.wx, w.wxb);
+        std::swap(w.wy, w.wyb);
+        c->prof_acc.kernel_launches += 2;
+    }
+    return c->ensure_workspace(g0); // size the level workspace once for the finest level
+}
+
+int mt_window_solve(sfgpu_ctx *c, const sf_mt_params_t *p, bool one_direction, MtWindow &w, float avg_change[2]) {
+    cudaStream_t st = c->stream;
+    const int L = w.levels, ref = w.ref;
+    const std::vector<Geom> &geoms = w.geoms;
+    Geom cur_g = geoms[L - 1];
+    avg_change[0] = avg_change[1] = 0.f;
+    int rc = SFGPU_OK;
+    for (int l = L - 1; l >= 0 && rc == SFGPU_OK; l--) {
+        const Geom g = geoms[l];
+        if (l < L - 1) { // up-sample the flow of level l+1 and scale the vectors (:687-722)
+            const float fx = (1.0f * g.W) / cur_g.W, fy = (1.0f * g.H) / cur_g.H;
+            k_resize<<<resize_grid(g), dim3(32, 8), 0, st>>>(cur_g, w.wx, g, w.wxb, (double)cur_g.W / g.W, (double)cur_g.H / g.H, fx, 1);
+            k_resize<<<resize_grid(g), dim3(32, 8), 0, st>>>(cur_g, w.wy, g, w.wyb, (double)cur_g.W / g.W, (double)cur_g.H / g.H, fy, 1);
+            std::swap(w.wx, w.wxb);
+            std::swap(w.wy, w.wyb);
+            cur_g = g;
+            c->prof_acc.kernel_launches += 2;
+        }
+        rc = c->ensure_workspace(g);
+        if (rc != SFGPU_OK) break;
+        LevelCtx Lc;
+        Lc.c = c; Lc.p = p; Lc.g = g; Lc.ref = ref;
+        Lc.one_direction = one_direction;
+        Lc.alpha = p->alpha;
+        Lc.gamma_over3 = p->gamma / 3.0f;
+        Lc.delta_over3 = p->delta / 3.0f;
+        Lc.pc = make_penalty(p->robust_color, p->robust_color_eps, p->robust_color_truncation);
+        Lc.pg = (p->robust_grad >= 0) ? make_penalty(p->robust_grad, p->robust_grad_eps, p->robust_grad_truncation) : Lc.pc; // Q8
+        Lc.preg = make_penalty(p->robust_reg, p->robust_reg_eps, p->robust_reg_truncation);
+        Lc.frames = w.frames[l];
+        Lc.warped = w.warped;
+        Lc.warped[ref] = w.frames[l][ref];
+        Lc.masks = w.masks;
+        Lc.derivs = w.derivs;
+        Lc.fused_terms = c->mt_data_variant == 0;
+        Lc.wx = w.wx; Lc.wy = w.wy; Lc.uu = w.uu; Lc.vv = w.vv; Lc.odu = w.odu; Lc.odv = w.odv;
+        Lc.dpsis = w.dpsis; Lc.occ = w.occ; Lc.d0 = w.d0; Lc.d1 = w.d1;
+        Lc.chw = w.chw; Lc.chw_pstride = geoms[0].plane();
+        Lc.work = c->mtw;
+        rc = compute_one_level(Lc, avg_change);
+    }
+    return rc;
+}
+
 } // namespace sf
 
 // ------------------------------------------------------------------------------------------ ABI
@@ -898,7 +1094,7 @@ int sfgpu_normalize(sfgpu_ctx *c, color_image_t *const *seq, int F, sf_mt_params
     if (const char *e = getenv("SLOWFLOW_GPU_NORMALIZE_RESIDENT_BYTES")) resident_limit = (size_t)strtoull(e, nullptr, 10); // tests
     const bool resident = (size_t)F * 3 * P * sizeof(float) <= resident_limit;
     const size_t fstride = resident ? 3 * P : 0;
-    const int nblk = std::min(g.H, 592);
+    const int nblk = norm_blocks(g);
     struct Bufs { // freed on every path
         float *dev = nullptr;
         double *dsum = nullptr;
@@ -910,39 +1106,22 @@ int sfgpu_normalize(sfgpu_ctx *c, color_image_t *const *seq, int F, sf_mt_params
     double *dsum = b.dsum;
     for (int f = 0; f < F; f++) {
         SF_CUDA(cudaMemcpyAsync(dev + (size_t)f * fstride, seq[f]->c1, 3 * P * sizeof(float), cudaMemcpyHostToDevice, st));
-        k_norm_sums<<<nblk, 256, 0, st>>>(g, dev + (size_t)f * fstride, dsum + (size_t)f * nblk * 6);
+        launch_norm_sums(st, g, dev + (size_t)f * fstride, dsum + (size_t)f * nblk * 6);
     }
     SF_CUDA(cudaGetLastError());
     std::vector<double> hs((size_t)F * nblk * 6);
     SF_CUDA(cudaMemcpyAsync(hs.data(), dsum, hs.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaStreamSynchronize(st));
-    double avg[3] = {0, 0, 0}, sd[3] = {0, 0, 0};
-    const double n = (double)g.H * g.W;
-    for (int f = 0; f < F; f++) {
-        double fs[6] = {0, 0, 0, 0, 0, 0};
-        for (int blk = 0; blk < nblk; blk++)
-            for (int k = 0; k < 6; k++) fs[k] += hs[((size_t)f * nblk + blk) * 6 + k];
-        for (int k = 0; k < 3; k++) { avg[k] += fs[k] / n; sd[k] += fs[3 + k] / n; }
-    }
-    for (int k = 0; k < 3; k++) {
-        avg[k] /= F;
-        sd[k] = sqrt((sd[k] / F) - avg[k] * avg[k]) / 255.0f; // :48-51
-    }
+    double avg[3], sd[3];
+    norm_statistics(hs.data(), F, g, avg, sd);
     for (int f = 0; f < F; f++) {
         if (!resident) SF_CUDA(cudaMemcpyAsync(dev, seq[f]->c1, 3 * P * sizeof(float), cudaMemcpyHostToDevice, st));
-        k_norm_apply<<<grid2d(g.W, g.H), dim3(32, 8), 0, st>>>(g, dev + (size_t)f * fstride, avg[0], avg[1], avg[2], sd[0], sd[1], sd[2]);
+        launch_norm_apply(st, g, dev + (size_t)f * fstride, avg, sd);
         SF_CUDA(cudaMemcpyAsync(seq[f]->c1, dev + (size_t)f * fstride, 3 * P * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
     SF_CUDA(cudaGetLastError());
     SF_CUDA(cudaStreamSynchronize(st));
-    for (int k = 0; k < 3; k++) {
-        // the reference publishes the values through a stringstream with 6 significant digits (:72-84)
-        char buf[64];
-        snprintf(buf, sizeof(buf), "%.6g", avg[k]);
-        params->img_norm_avg[k] = (float)atof(buf);
-        snprintf(buf, sizeof(buf), "%.6g", sd[k]);
-        params->img_norm_std[k] = (float)atof(buf);
-    }
+    norm_publish(avg, sd, params);
     c->prof_acc.kernel_launches += 2 * F;
     return SFGPU_OK;
 }
@@ -982,12 +1161,7 @@ int sfgpu_prescale(sfgpu_ctx *c, color_image_t *dst, const color_image_t *src, f
     if (rc != SFGPU_OK) return rc;
     float *d_src = c->io, *d_tmp = c->io + 3 * Ps, *d_blur = c->io + 6 * Ps, *d_dst = c->io + 9 * Ps;
     SF_CUDA(cudaMemcpyAsync(d_src, src->c1, 3 * Ps * sizeof(float), cudaMemcpyHostToDevice, st));
-    // GaussianBlur(img, img, Size(), 1/sqrt(2*scale), ..., BORDER_REPLICATE) then resize(..., scale, scale, INTER_LINEAR)
-    // (slow_flow.cpp:539-542); the mapping of a resize by factor uses 1/fx, not the ratio of the rounded sizes
-    const double sigma = 1.0 / sqrt((double)(2.0f * scale));
-    const BlurTaps taps = make_taps(sigma);
-    launch_blur(st, gs, d_src, d_tmp, d_blur, taps, 3);
-    k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(gs, d_blur, gd, d_dst, 1.0 / (double)scale, 1.0 / (double)scale, 1.0f, 3);
+    launch_prescale(st, gs, d_src, d_tmp, d_blur, gd, d_dst, scale);
     c->prof_acc.kernel_launches += 3;
     SF_CUDA(cudaMemcpyAsync(dst->c1, d_dst, 3 * Pd * sizeof(float), cudaMemcpyDeviceToHost, st));
     SF_CUDA(cudaStreamSynchronize(st));
@@ -1195,179 +1369,70 @@ int sfgpu_variational_mt(sfgpu_ctx *c, image_t *wx, image_t *wy, const color_ima
     const double t_call = now_ms();
     if (avg_change_out) avg_change_out[0] = avg_change_out[1] = 0.f;
 
-    // ---- pyramid geometry (variational_mt.cpp:583-652): floor((float)w * p_scale); a level is dropped when
-    // the NEXT one would be <= order+1 = floor(3 sigma)+2 pixels (:647-651)
-    const float sigma = 1.0f / sqrtf(2.0f * p->p_scale);
-    const int order = (int)floorf(3.0f * sigma) + 1;
-    std::vector<Geom> geoms;
-    int L = p->layers;
-    for (int l = 0; l < L; l++) {
-        if (l == 0) geoms.push_back(flow_g);
-        else geoms.push_back(make_geom((int)floorf((float)geoms[l - 1].W * p->p_scale), (int)floorf((float)geoms[l - 1].H * p->p_scale)));
-        if (floorf((float)geoms[l].W * p->p_scale) <= order + 1 || floorf((float)geoms[l].H * p->p_scale) <= order + 1) {
-            L = l;
-            break;
-        }
-    }
-    if (L == 0) return SFGPU_OK; // the reference computes nothing in this case
-    geoms.resize(L);
-    c->mt_stats.levels = L;
-
-    // ---- device memory: frames of all levels + per-level work planes sized for level 0
-    const Geom g0 = geoms[0];
-    const size_t P0 = g0.plane();
     // with the frame cache (sfgpu_mt_frame_cache) the level-0 frames live in the cache's own device buffers
     const bool cached = !c->mt_cache.empty() && (int)c->mt_cache.size() >= F;
-    size_t frame_floats = 0;
-    for (int l = cached ? 1 : 0; l < L; l++) frame_floats += (size_t)F * 3 * geoms[l].plane();
-    const size_t work_planes = (size_t)(F - 1) * 3 + (F - 1) + 2 /*wx wy*/ + 2 /*wx,wy of next level*/ + 2 /*uu vv*/ + 2 /*odu odv*/ + 1 /*dpsis*/ +
-                               1 /*occ*/ + 2 /*d0 d1*/ + 3 /*blur tmp*/ + (channel_w ? 3 : 0) +
-                               (c->mt_data_variant == 0 ? (size_t)F * 15 /*per-frame derivative planes*/ : 0);
-    if (!c->mtw) c->mtw = new MtWork();
-    MtWork &work = *c->mtw;
-    {
-        const int rcw = work.reserve(frame_floats + work_planes * P0, (size_t)((g0.W + 31) / 32) * 64 * 4, (size_t)g0.W * g0.H);
-        if (rcw != SFGPU_OK) return rcw;
-    }
-    float *ptr = work.pool;
-    std::vector<MtLevel> levels(L);
+    MtWindow w;
+    int rc = mt_window_layout(c, p, flow_g, !cached, channel_w != nullptr, w);
+    if (rc != SFGPU_OK || w.levels == 0) return rc; // levels == 0: the reference computes nothing
+    const size_t P0 = flow_g.plane();
     std::vector<bool> frame_resident(F, false); // level-0 frame already on the device (cache hit)
-    for (int l = 0; l < L; l++) {
-        levels[l].g = geoms[l];
-        if (l == 0 && cached) {
-            // slot per frame: the one that holds this host buffer, else the least recently used slot no frame of this call has
-            const unsigned long long now = ++c->mt_cache_clock;
-            const size_t want = 3 * P0;
-            if (c->mt_cache_slot_floats != want) { // first use, or another geometry: one pool for all slots
-                SF_CUDA(cudaStreamSynchronize(st));
-                if (c->mt_cache_pool) cudaFree(c->mt_cache_pool);
-                c->mt_cache_pool = nullptr;
-                c->mt_cache_slot_floats = 0;
-                SF_CUDA(cudaMalloc(&c->mt_cache_pool, c->mt_cache.size() * want * sizeof(float)));
-                c->mt_cache_slot_floats = want;
-                for (size_t k = 0; k < c->mt_cache.size(); k++) {
-                    c->mt_cache[k] = sfgpu_ctx::MtFrameSlot();
-                    c->mt_cache[k].dev = c->mt_cache_pool + k * want;
-                    c->mt_cache[k].floats = want;
-                }
+    if (cached) {
+        // slot per frame: the one that holds this host buffer, else the least recently used slot no frame of this call has
+        const unsigned long long now = ++c->mt_cache_clock;
+        const size_t want = 3 * P0;
+        if (c->mt_cache_slot_floats != want) { // first use, or another geometry: one pool for all slots
+            SF_CUDA(cudaStreamSynchronize(st));
+            if (c->mt_cache_pool) cudaFree(c->mt_cache_pool);
+            c->mt_cache_pool = nullptr;
+            c->mt_cache_slot_floats = 0;
+            SF_CUDA(cudaMalloc(&c->mt_cache_pool, c->mt_cache.size() * want * sizeof(float)));
+            c->mt_cache_slot_floats = want;
+            for (size_t k = 0; k < c->mt_cache.size(); k++) {
+                c->mt_cache[k] = sfgpu_ctx::MtFrameSlot();
+                c->mt_cache[k].dev = c->mt_cache_pool + k * want;
+                c->mt_cache[k].floats = want;
             }
-            for (int f = 0; f < F; f++) {
-                sfgpu_ctx::MtFrameSlot *slot = nullptr;
-                for (auto &e : c->mt_cache)
-                    if (e.host == (const void *)im[f]->c1 && e.floats == want && e.stamp != now) { slot = &e; frame_resident[f] = true; break; }
-                if (!slot) {
-                    for (auto &e : c->mt_cache)
-                        if (e.stamp != now && (!slot || e.stamp < slot->stamp)) slot = &e;
-                    slot->host = im[f]->c1;
-                    c->mt_cache_misses++;
-                } else {
-                    c->mt_cache_hits++;
-                }
-                slot->stamp = now;
-                levels[0].frames.push_back(slot->dev);
-            }
-            continue;
         }
-        for (int f = 0; f < F; f++) { levels[l].frames.push_back(ptr); ptr += 3 * geoms[l].plane(); }
+        for (int f = 0; f < F; f++) {
+            sfgpu_ctx::MtFrameSlot *slot = nullptr;
+            for (auto &e : c->mt_cache)
+                if (e.host == (const void *)im[f]->c1 && e.floats == want && e.stamp != now) { slot = &e; frame_resident[f] = true; break; }
+            if (!slot) {
+                for (auto &e : c->mt_cache)
+                    if (e.stamp != now && (!slot || e.stamp < slot->stamp)) slot = &e;
+                slot->host = im[f]->c1;
+                c->mt_cache_misses++;
+            } else {
+                c->mt_cache_hits++;
+            }
+            slot->stamp = now;
+            w.frames[0][f] = slot->dev;
+        }
     }
-    auto take = [&](size_t planes) { float *r = ptr; ptr += planes * P0; return r; };
-    std::vector<float *> warped(F, nullptr), masks(F, nullptr);
-    for (int f = 0; f < F; f++)
-        if (f != ref) { warped[f] = take(3); masks[f] = take(1); }
-    float *wxa = take(1), *wya = take(1), *wxb = take(1), *wyb = take(1);
-    float *uu = take(1), *vv = take(1), *odu = take(1), *odv = take(1), *dpsis = take(1), *occ = take(1), *d0 = take(1), *d1 = take(1);
-    float *blur_tmp = take(3);
-    float *chw = channel_w ? take(3) : nullptr;
-    std::vector<float *> derivs(F, nullptr);
-    if (c->mt_data_variant == 0)
-        for (int f = 0; f < F; f++) derivs[f] = take(15);
 
     // ---- upload
     {
         std::vector<HostCopy> up;
         for (int f = 0; f < F; f++)
-            if (!frame_resident[f]) up.push_back(HostCopy{levels[0].frames[f], im[f]->c1, 3 * P0 * sizeof(float)});
-        up.push_back(HostCopy{wxa, wx->data, P0 * sizeof(float)});
-        up.push_back(HostCopy{wya, wy->data, P0 * sizeof(float)});
-        if (chw) up.push_back(HostCopy{chw, channel_w->c1, 3 * P0 * sizeof(float)});
+            if (!frame_resident[f]) up.push_back(HostCopy{w.frames[0][f], im[f]->c1, 3 * P0 * sizeof(float)});
+        up.push_back(HostCopy{w.wx, wx->data, P0 * sizeof(float)});
+        up.push_back(HostCopy{w.wy, wy->data, P0 * sizeof(float)});
+        if (channel_w) up.push_back(HostCopy{w.chw_plane, channel_w->c1, 3 * P0 * sizeof(float)});
         const int rcu = host_copies(c, up, true); // pageable caller frames: multi-threaded staging (sf_hostcopy.cu)
         if (rcu != SFGPU_OK) return rcu;
     }
-
-    // ---- pyramid: GaussianBlur(sigma) + resize per frame and level (:604-614)
-    if (L > 1) {
-        const BlurTaps taps = make_taps((double)sigma);
-        for (int l = 1; l < L; l++) {
-            const Geom gs = geoms[l - 1], gd = geoms[l];
-            for (int f = 0; f < F; f++) {
-                // vertical pass writes into the (not yet used) warp scratch of frame slot 0/1
-                float *tmp2 = warped[ref == 0 ? 1 : 0];
-                launch_blur(st, gs, levels[l - 1].frames[f], blur_tmp, tmp2, taps, 3);
-                k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(gs, tmp2, gd, levels[l].frames[f], (double)gs.W / gd.W,
-                                                                  (double)gs.H / gd.H, 1.0f, 3);
-                c->prof_acc.kernel_launches += 3;
-            }
-        }
-    }
-
-    // ---- coarse-to-fine (:662-762)
-    float *cur_x = wxa, *cur_y = wya, *oth_x = wxb, *oth_y = wyb;
-    Geom cur_g = g0;
-    if (L > 1) {
-        const Geom gd = geoms[L - 1];
-        const float fx = (1.0f * gd.W) / g0.W, fy = (1.0f * gd.H) / g0.H;
-        k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(g0, cur_x, gd, oth_x, (double)g0.W / gd.W, (double)g0.H / gd.H, fx, 1);
-        k_resize<<<resize_grid(gd), dim3(32, 8), 0, st>>>(g0, cur_y, gd, oth_y, (double)g0.W / gd.W, (double)g0.H / gd.H, fy, 1);
-        std::swap(cur_x, oth_x);
-        std::swap(cur_y, oth_y);
-        cur_g = gd;
-        c->prof_acc.kernel_launches += 2;
-    }
-    float avg_change[2] = {0.f, 0.f};
-    int rc = c->ensure_workspace(g0); // size the level workspace once for the finest level
+    rc = mt_window_build(c, w);
     if (cudaStreamSynchronize(st) == cudaSuccess) c->mt_stats.setup_ms = now_ms() - t_call;
-    for (int l = L - 1; l >= 0 && rc == SFGPU_OK; l--) {
-        const Geom g = geoms[l];
-        if (l < L - 1) { // up-sample the flow of level l+1 and scale the vectors (:687-722)
-            const float fx = (1.0f * g.W) / cur_g.W, fy = (1.0f * g.H) / cur_g.H;
-            k_resize<<<resize_grid(g), dim3(32, 8), 0, st>>>(cur_g, cur_x, g, oth_x, (double)cur_g.W / g.W, (double)cur_g.H / g.H, fx, 1);
-            k_resize<<<resize_grid(g), dim3(32, 8), 0, st>>>(cur_g, cur_y, g, oth_y, (double)cur_g.W / g.W, (double)cur_g.H / g.H, fy, 1);
-            std::swap(cur_x, oth_x);
-            std::swap(cur_y, oth_y);
-            cur_g = g;
-            c->prof_acc.kernel_launches += 2;
-        }
-        rc = c->ensure_workspace(g);
-        if (rc != SFGPU_OK) break;
-        LevelCtx Lc;
-        Lc.c = c; Lc.p = p; Lc.g = g; Lc.ref = ref;
-        Lc.one_direction = p->one_direction != 0;
-        Lc.alpha = p->alpha;
-        Lc.gamma_over3 = p->gamma / 3.0f;
-        Lc.delta_over3 = p->delta / 3.0f;
-        Lc.pc = make_penalty(p->robust_color, p->robust_color_eps, p->robust_color_truncation);
-        Lc.pg = (p->robust_grad >= 0) ? make_penalty(p->robust_grad, p->robust_grad_eps, p->robust_grad_truncation) : Lc.pc; // Q8
-        Lc.preg = make_penalty(p->robust_reg, p->robust_reg_eps, p->robust_reg_truncation);
-        Lc.frames = levels[l].frames;
-        Lc.warped = warped;
-        Lc.warped[ref] = levels[l].frames[ref];
-        Lc.masks = masks;
-        Lc.derivs = derivs;
-        Lc.fused_terms = c->mt_data_variant == 0;
-        Lc.wx = cur_x; Lc.wy = cur_y; Lc.uu = uu; Lc.vv = vv; Lc.odu = odu; Lc.odv = odv;
-        Lc.dpsis = dpsis; Lc.occ = occ; Lc.d0 = d0; Lc.d1 = d1;
-        Lc.chw = chw; Lc.chw_pstride = P0;
-        Lc.work = &work;
-        rc = compute_one_level(Lc, avg_change);
-    }
+    float avg_change[2] = {0.f, 0.f};
+    if (rc == SFGPU_OK) rc = mt_window_solve(c, p, p->one_direction != 0, w, avg_change);
     if (rc != SFGPU_OK) return rc;
 
     {
         std::vector<HostCopy> down;
-        down.push_back(HostCopy{cur_x, wx->data, P0 * sizeof(float)});
-        down.push_back(HostCopy{cur_y, wy->data, P0 * sizeof(float)});
+        down.push_back(HostCopy{w.wx, wx->data, P0 * sizeof(float)});
+        down.push_back(HostCopy{w.wy, wy->data, P0 * sizeof(float)});
         if (occlusions_out && occlusions_out->data)
-            down.push_back(HostCopy{occ, occlusions_out->data, P0 * sizeof(float)});
+            down.push_back(HostCopy{w.occ, occlusions_out->data, P0 * sizeof(float)});
         const int rcd = host_copies(c, down, false);
         if (rcd != SFGPU_OK) return rcd;
     }

@@ -53,12 +53,16 @@ struct SeqFrames { // where the frames of a call come from
     const void *host(int f) const { return ints ? ints[f].data : (const void *)f32[f]->c1; }
 };
 
-static void launch_unpack(sfgpu_ctx *c, Geom g, const SeqFrames &src, int f, const unsigned char *raw, float *dst) {
+void launch_unpack_frame(cudaStream_t st, Geom g, const unsigned char *raw, size_t step, int channels, int bits, float *dst) {
     const dim3 grid((g.S / 4 + 255) / 256, g.H);
-    if (src.depth == 8)
-        launch_pdl(k_unpack_frame<unsigned char>, grid, dim3(256), 0, c->stream, g, raw, (size_t)src.ints[f].step, src.ints[f].channels, dst);
+    if (bits == 8)
+        launch_pdl(k_unpack_frame<unsigned char>, grid, dim3(256), 0, st, g, raw, step, channels, dst);
     else
-        launch_pdl(k_unpack_frame<unsigned short>, grid, dim3(256), 0, c->stream, g, raw, (size_t)src.ints[f].step, src.ints[f].channels, dst);
+        launch_pdl(k_unpack_frame<unsigned short>, grid, dim3(256), 0, st, g, raw, step, channels, dst);
+}
+
+static void launch_unpack(sfgpu_ctx *c, Geom g, const SeqFrames &src, int f, const unsigned char *raw, float *dst) {
+    launch_unpack_frame(c->stream, g, raw, (size_t)src.ints[f].step, src.ints[f].channels, src.depth, dst);
     c->prof_acc.kernel_launches++;
 }
 
@@ -155,19 +159,9 @@ static int sequence(sfgpu_ctx *c, const char *fn, int n_pairs, const SeqFrames &
     if (!arg_geom(who.at(0), "wx", wx[0], g)) return SFGPU_ERR_ARG;
     for (int j = 0; j < n_pairs; j++)
         if (!arg_is(who.at(j), "wx", wx[j], g) || !arg_is(who.at(j), "wy", wy[j], g)) return SFGPU_ERR_ARG;
-    const size_t sample = src.depth / 8;
     for (int f = 0; f <= n_pairs; f++) {
         const std::string at = who.at(std::max(f - 1, 0)), name = "frames[" + std::to_string(f) + "]";
-        if (src.f32) {
-            if (!arg_is(at, name, src.f32[f], g)) return SFGPU_ERR_ARG;
-            continue;
-        }
-        const sf_frame_int_t &q = src.ints[f];
-        if (!q.data || q.width != g.W || q.height != g.H || (q.channels != 1 && q.channels != 3) ||
-            q.step < (size_t)q.width * q.channels * sample || (q.step % sample) != 0) {
-            set_error(at + name + ": integer frames must match the flow geometry, have 1 or 3 channels and step >= width*channels*bytes");
-            return SFGPU_ERR_ARG;
-        }
+        if (src.f32 ? !arg_is(at, name, src.f32[f], g) : !arg_frame_int(at, name, src.ints[f], g, src.depth)) return SFGPU_ERR_ARG;
     }
     return run_sequence(c, n_pairs, src, g, wx, wy, params, continue_from_previous != 0);
 }
