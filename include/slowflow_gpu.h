@@ -208,7 +208,8 @@ int sfgpu_normalize(sfgpu_ctx *ctx, color_image_t *const *seq, int F, sf_mt_para
  * sfgpu_get_mt_stats afterwards sums the windows of the call; its setup_ms is the time of the statistics pass and
  * total_ms that of the call.  Every argument check runs before anything is written.  SFGPU_ERR_UNSUPPORTED for
  * smoothing >= 2, like sfgpu_variational_mt.  Uses the context's io area, so a following sfgpu_variational_sequence_u8/u16
- * cannot use continue_from_previous. */
+ * cannot use continue_from_previous.  sfgpu_slow_flow_jets_epic (with the EPIC entries below) is the same loop with EPIC
+ * initial flows. */
 int sfgpu_slow_flow_jets(sfgpu_ctx *ctx, int n_frames, const sf_frame_int_t *frames, int bits, float scale,
                          int first_jet, int n_jets, sf_mt_params_t *params, int backward_one_direction,
                          const color_image_t *channel_w, image_t *const *fwd_x, image_t *const *fwd_y,
@@ -406,6 +407,43 @@ int sfgpu_rgb_to_lab(sfgpu_ctx *ctx, color_image_t *dst, const color_image_t *sr
 int sfgpu_epicflow_sequence(sfgpu_ctx *ctx, int n_pairs, const color_image_t *const *frames, const float_image *const *matches,
                             float_image *const *edges, const epic_params_t *epic_params, const variational_params_t *flow_params,
                             image_t *const *wx, image_t *const *wy, sfgpu_epic_stats_t *stats);
+/* The jet loop of slow_flow.cpp:706-1030 in its other mode (deep_matching != 0): every window starts from an EPIC
+ * interpolation of sparse matches (forward window slow_flow.cpp:801-843, backward window :979) instead of a zero flow.
+ * Frames, bits, scale, first_jet / n_jets, params (img_norm_* published), backward_one_direction, channel_w (forward
+ * windows only), the outputs (x S-1), occlusions and SFGPU_ERR_UNSUPPORTED for smoothing >= 2 are as in
+ * sfgpu_slow_flow_jets.  With s = S-1, nf[f] = frame f after unpack, sfgpu_prescale (scale != 1) and sfgpu_normalize over
+ * all n_frames (what sfgpu_slow_flow_jets computes), and r = j*s + s the reference frame of jet j's forward window, the
+ * outputs at k = j - first_jet are, bit for bit and on whole planes:
+ *   forward:  lab = sfgpu_rgb_to_lab(nf[r])                       (only when saliency_th != 0)
+ *             sfgpu_epic(fx, fy, lab, fwd_matches[k], edges[k], epic_params, &epic_stats[2k])
+ *             fx, fy *= 1.0f / s                                  (fp32)
+ *             sfgpu_variational_mt(fx, fy, nf[j*s .. j*s + 2s], params, channel_w, occlusions[k])
+ *             fwd_x[k], fwd_y[k] = fx, fy * s
+ *   backward: the same with Lab from nf[r + s], back_matches[k], edges[k + 1], &epic_stats[2k + 1], the frames
+ *             nf[j*s + 3s - i] for i = 0 .. 2s, no channel weights, and one_direction = params->one_direction ||
+ *             backward_one_direction.
+ * Matches and edge maps are in the window geometry (after pre-scaling); edges[m] (n_jets + 1 distinct arrays) belongs to
+ * reference frame (first_jet + m)*s + s and serves jet m - 1's backward and jet m's forward window.  euc is added once to
+ * every edges[m] in the caller's array, as epic() adds it; since the reference reads the edge file afresh per window, both
+ * windows see edges + euc, as here.  Lab is converted from the window's own normalised reference frame: normalize() runs
+ * in place on the sequence (slow_flow.cpp:673) before the loop (:706) reads im = &seq[j*steps] (:721-724) and calls
+ * rgb_to_lab (:814), which also puts 8- and 16-bit sequences on one scale for the saliency filter.  epic_params is required;
+ * epic_stats: 2 * n_jets entries (forward, backward per jet) or NULL.
+ * Jets run in chunks of 4 (8 EPIC items in one batch); with page-locked memory the next chunk's frames and edge maps go up
+ * while this chunk's windows solve, and every window's results go down while the next one computes.  Device memory is
+ * bounded by the chunk, not by n_jets.
+ * Errors: every argument check (those of sfgpu_slow_flow_jets and of sfgpu_epic: match columns >= 4, method, edge
+ * geometry; and distinct edge arrays) runs before anything is written.  A window left with no match after the filters
+ * stops the call: the chunks before its chunk are complete (flows, occlusions, stats, edges), the later outputs are not
+ * written, the later chunks' edge maps are untouched, and the message names the jet and the direction. */
+int sfgpu_slow_flow_jets_epic(sfgpu_ctx *ctx, int n_frames, const sf_frame_int_t *frames, int bits, float scale,
+                              int first_jet, int n_jets, sf_mt_params_t *params, int backward_one_direction,
+                              const color_image_t *channel_w, const float_image *const *fwd_matches,
+                              const float_image *const *back_matches, float_image *const *edges,
+                              const epic_params_t *epic_params, image_t *const *fwd_x, image_t *const *fwd_y,
+                              image_t *const *back_x, image_t *const *back_y, image_t *const *occlusions,
+                              sfgpu_epic_stats_t *epic_stats);
+
 /* operator twin of dist_trf_nnfield_subset (epic_aux.cpp:350-401) with the seeds as the query points: the label map
  * (w*h), and per seed the nn nearest seeds over the geodesic neighbourhood graph with their distances */
 int sfgpu_epic_nnfield(sfgpu_ctx *ctx, int *best, float *dist, int *labels, const int *seeds, int ns, int nn,

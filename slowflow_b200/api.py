@@ -61,7 +61,7 @@ ABI_SYMBOLS = [
     "sfgpu_last_error", "sfgpu_device_count", "sfgpu_synchronize", "sfgpu_set_sor_variant", "sfgpu_set_sor_fuse",
     "sfgpu_variational", "sfgpu_variational_dev", "sfgpu_variational_sequence", "sfgpu_variational_sequence_u8",
     "sfgpu_variational_sequence_u16", "sfgpu_host_register",
-    "sfgpu_host_unregister", "sfgpu_variational_mt", "sfgpu_mt_frame_cache", "sfgpu_normalize", "sfgpu_slow_flow_jets", "sfgpu_get_mt_stats", "sfgpu_profile_enable",
+    "sfgpu_host_unregister", "sfgpu_variational_mt", "sfgpu_mt_frame_cache", "sfgpu_normalize", "sfgpu_slow_flow_jets", "sfgpu_slow_flow_jets_epic", "sfgpu_get_mt_stats", "sfgpu_profile_enable",
     "sfgpu_profile_reset", "sfgpu_profile_get", "sfgpu_image_warp", "sfgpu_warp_frame_derivs", "sfgpu_compute_dpsis_weight",
     "sfgpu_compute_smoothness", "sfgpu_compute_data_and_match", "sfgpu_prep_two_frame", "sfgpu_mt_system", "sfgpu_mt_occ_costs", "sfgpu_sub_laplacian", "sfgpu_sor_coupled",
     "sfgpu_epic", "sfgpu_epic_batch", "sfgpu_epic_nnfield", "sfgpu_rgb_to_lab", "sfgpu_epicflow_sequence", "epic_params_default", "sfgpu_version", "sfgpu_grid_mincut", "sfgpu_grid_mincut_dev", "sfgpu_prescale_size", "sfgpu_prescale", "sfgpu_raw_weighting",
@@ -110,6 +110,10 @@ def load_library(path=None):
     lib.sfgpu_get_mt_stats.argtypes = [C.c_void_p, C.POINTER(MTStats)]
     lib.sfgpu_slow_flow_jets.argtypes = [C.c_void_p, C.c_int, C.POINTER(FrameInt), C.c_int, C.c_float, C.c_int, C.c_int,
                                          C.POINTER(MTParams), C.c_int, CP] + [C.POINTER(IP)] * 5
+    FIPP = C.POINTER(C.POINTER(FloatImage))
+    lib.sfgpu_slow_flow_jets_epic.argtypes = ([C.c_void_p, C.c_int, C.POINTER(FrameInt), C.c_int, C.c_float, C.c_int, C.c_int,
+                                               C.POINTER(MTParams), C.c_int, CP, FIPP, FIPP, FIPP, C.POINTER(EpicParams)] +
+                                              [C.POINTER(IP)] * 5 + [C.POINTER(EpicStats)])
     lib.sfgpu_profile_enable.argtypes = [C.c_void_p, C.c_int]
     lib.sfgpu_profile_reset.argtypes = [C.c_void_p]
     lib.sfgpu_profile_get.argtypes = [C.c_void_p, C.POINTER(Profile)]
@@ -361,6 +365,28 @@ class Context:
                "sfgpu_variational_mt")
         return float(out[0]), float(out[1])
 
+    @staticmethod
+    def _frame_ints(frames):
+        """(sf_frame_int_t array, bits) of numpy uint8 / uint16 frames (H, W) or (H, W, 3) in cv::Mat layout."""
+        bits = frames[0].dtype.itemsize * 8
+        assert bits in (8, 16) and all(f.dtype == frames[0].dtype for f in frames)
+        fa = (FrameInt * len(frames))()
+        for k, f in enumerate(frames):
+            ch = 1 if f.ndim == 2 else f.shape[2]
+            assert f.strides[1] == ch * f.dtype.itemsize and (f.ndim == 2 or f.strides[2] == f.dtype.itemsize)
+            fa[k] = FrameInt(f.shape[1], f.shape[0], ch, f.strides[0], f.ctypes.data)
+        return fa, bits
+
+    def _jet_planes(self, frames, scale, n_jets, occlusions):
+        """The output planes of the jet entries in the scaled geometry, and their image_t* arrays."""
+        w, h = C.c_int(), C.c_int()
+        _check(self.lib, self.lib.sfgpu_prescale_size(frames[0].shape[1], frames[0].shape[0], scale, C.byref(w), C.byref(h)),
+               "sfgpu_prescale_size")
+        planes = [[Image(w.value, h.value) for _ in range(n_jets)] for _ in range(5 if occlusions else 4)]
+        IP = C.POINTER(image_t)
+        arrays = [(IP * n_jets)(*[C.pointer(p.c) for p in ps]) for ps in planes]
+        return planes, arrays[:4] + [arrays[4] if occlusions else None]
+
     def slow_flow_jets(self, frames, params, n_jets, first_jet=0, scale=1.0, backward_one_direction=False, channel_w=None,
                        occlusions=False):
         """The jet loop of slow_flow.cpp:706-1030 on the device (sfgpu_slow_flow_jets).  frames: the whole sequence as numpy
@@ -369,26 +395,47 @@ class Context:
         frames j*(S-1) .. j*(S-1) + 3*(S-1).  Returns (forward flows, backward flows, occlusions): lists of n_jets
         (x, y) Image pairs in the scaled geometry, already multiplied by S-1, and n_jets occlusion Images (None unless
         `occlusions`)."""
-        n = len(frames)
-        bits = frames[0].dtype.itemsize * 8
-        assert bits in (8, 16) and all(f.dtype == frames[0].dtype for f in frames)
-        fa = (FrameInt * n)()
-        for k, f in enumerate(frames):
-            ch = 1 if f.ndim == 2 else f.shape[2]
-            assert f.strides[1] == ch * f.dtype.itemsize and (f.ndim == 2 or f.strides[2] == f.dtype.itemsize)
-            fa[k] = FrameInt(f.shape[1], f.shape[0], ch, f.strides[0], f.ctypes.data)
-        w, h = C.c_int(), C.c_int()
-        _check(self.lib, self.lib.sfgpu_prescale_size(frames[0].shape[1], frames[0].shape[0], scale, C.byref(w), C.byref(h)),
-               "sfgpu_prescale_size")
-        planes = [[Image(w.value, h.value) for _ in range(n_jets)] for _ in range(5 if occlusions else 4)]
-        IP = C.POINTER(image_t)
-        arrays = [(IP * n_jets)(*[C.pointer(p.c) for p in ps]) for ps in planes]
-        _check(self.lib, self.lib.sfgpu_slow_flow_jets(self.h, n, fa, bits, scale, int(first_jet), int(n_jets), C.byref(params),
-                                                       1 if backward_one_direction else 0, _ip(channel_w), *arrays[:4],
-                                                       arrays[4] if occlusions else None), "sfgpu_slow_flow_jets")
+        fa, bits = self._frame_ints(frames)
+        planes, arrays = self._jet_planes(frames, scale, n_jets, occlusions)
+        _check(self.lib, self.lib.sfgpu_slow_flow_jets(self.h, len(frames), fa, bits, scale, int(first_jet), int(n_jets), C.byref(params),
+                                                       1 if backward_one_direction else 0, _ip(channel_w), *arrays),
+               "sfgpu_slow_flow_jets")
         fwd = list(zip(planes[0], planes[1]))
         back = list(zip(planes[2], planes[3]))
         return fwd, back, planes[4] if occlusions else None
+
+    def slow_flow_jets_epic(self, frames, params, n_jets, fwd_matches, back_matches, edges, epic_params=None, first_jet=0,
+                            scale=1.0, backward_one_direction=False, channel_w=None, occlusions=False):
+        """The jet loop with EPIC initial flows (sfgpu_slow_flow_jets_epic, the deep-matching mode of slow_flow.cpp:801-843,
+        979): as ``slow_flow_jets``, but jet k's forward / backward window starts from EPIC of fwd_matches[k] /
+        back_matches[k] (float32 (n, >= 4) arrays x1 y1 x2 y2) with the edge map of its reference frame, x 1/(S-1).
+        edges: n_jets + 1 float32 (H, W) cost maps in the scaled geometry, edges[m] that of reference frame
+        (first_jet + m)*(S-1) + S-1; epic_params.euc is added to each IN PLACE, once.  Returns (forward flows, backward
+        flows, occlusions, EPIC stats) with 2 * n_jets EpicStats: forward, backward per jet."""
+        import numpy as np
+        assert len(fwd_matches) == n_jets and len(back_matches) == n_jets and len(edges) == n_jets + 1
+        for m in list(fwd_matches) + list(back_matches):
+            assert m.dtype == np.float32 and m.flags.c_contiguous and m.ndim == 2
+        for e in edges:
+            assert e.dtype == np.float32 and e.flags.c_contiguous and e.ndim == 2
+        if epic_params is None:
+            epic_params = epic_params_default()
+        fa, bits = self._frame_ints(frames)
+        planes, arrays = self._jet_planes(frames, scale, n_jets, occlusions)
+        FP, FIP = C.POINTER(C.c_float), C.POINTER(FloatImage)
+
+        def fis(arrs):
+            keep = [FloatImage(a.ctypes.data_as(FP), a.shape[1], a.shape[0]) for a in arrs]
+            return keep, (FIP * len(keep))(*[C.pointer(x) for x in keep])
+        fm, bm, ed = fis(fwd_matches), fis(back_matches), fis(edges)
+        st = (EpicStats * (2 * n_jets))()
+        _check(self.lib, self.lib.sfgpu_slow_flow_jets_epic(self.h, len(frames), fa, bits, scale, int(first_jet), int(n_jets),
+                                                            C.byref(params), 1 if backward_one_direction else 0, _ip(channel_w),
+                                                            fm[1], bm[1], ed[1], C.byref(epic_params), *arrays, st),
+               "sfgpu_slow_flow_jets_epic")
+        fwd = list(zip(planes[0], planes[1]))
+        back = list(zip(planes[2], planes[3]))
+        return fwd, back, planes[4] if occlusions else None, list(st)
 
     def mt_frame_cache(self, max_frames):
         """Device-side cache of level-0 frames keyed by their host buffers (sfgpu_mt_frame_cache): for callers that solve

@@ -268,7 +268,8 @@ int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d
 
 // ------------------------------------------------------------------------------------------ argument checks
 std::string Caller::at(int k) const {
-    return item ? std::string(fn) + ": " + item + " " + std::to_string(first + k) + ": " : std::string(fn) + ": ";
+    if (!item) return std::string(fn) + ": ";
+    return std::string(fn) + ": " + item + " " + std::to_string(first + k / per) + (part ? std::string(" ") + part[k % per] : "") + ": ";
 }
 
 static float *data_of(const image_t *a) { return a->data; }

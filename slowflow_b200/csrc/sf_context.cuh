@@ -121,11 +121,14 @@ int run_two_frame(sfgpu_ctx *c, Geom g, float *d_wx, float *d_wy, const float *d
 // ---- image arguments of the host-buffer entries (the container contract of slowflow_gpu.h:30-44).  An entry copies whole
 // planes of P = stride * height floats (3 P from a colour image's c1), with P from the call's one geometry.
 // Names the entry point in error messages, and in a batch or sequence the item ("item" / "pair" numbered from `first`;
-// null: none): at(k) is "<fn>: " or "<fn>: <item> <first + k>: ".
+// null: none): at(k) is "<fn>: " or "<fn>: <item> <first + k>: ".  With per > 1, per consecutive k share an item and
+// part names them: "<fn>: <item> <first + k / per> <part[k % per]>: " (the two windows of a jet).
 struct Caller {
     const char *fn;
     const char *item;
     int first;
+    int per = 1;
+    const char *const *part = nullptr;
     std::string at(int k) const;
 };
 // A failed check sets "<at><name>: <what>" and returns false; the entry then returns SFGPU_ERR_ARG before it touches the
@@ -188,4 +191,6 @@ void epic_add_euc(int n, float_image *const *edges, float euc);
 // entries.  The last kernels are left queued on the context's stream; on an error d_flow is not fully written.
 int epic_device(sfgpu_ctx *c, int n, Geom g, const float *d_cost, const float *d_lab, const float_image *const *input_matches,
                 const epic_params_t *params, float *d_flow, sfgpu_epic_stats_t *stats, const Caller &who);
+// rgb_to_lab (image.c:694) of the 3 planes of P floats at src into dst on the context's stream (sf_epicflow.cu)
+void launch_rgb_to_lab(sfgpu_ctx *c, size_t P, const float *src, float *dst);
 } // namespace sf

@@ -40,7 +40,7 @@ __global__ void __launch_bounds__(256) k_rgb_to_lab(size_t P, const float *__res
     dst[i + 2 * P] = __fmul_rn(B, corr);
 }
 
-static void launch_rgb_to_lab(sfgpu_ctx *c, size_t P, const float *src, float *dst) {
+void launch_rgb_to_lab(sfgpu_ctx *c, size_t P, const float *src, float *dst) {
     k_rgb_to_lab<<<(unsigned)((P + 255) / 256), 256, 0, c->stream>>>(P, src, dst);
     c->prof_acc.kernel_launches++;
 }
